@@ -2,9 +2,13 @@
 """Benchmark of the MindTheEdge depth-edge hot path on B200 (the driver's contract).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl mte|reference]
-                    [--workload loss|auc|dee|ddad|train]
+                    [--workload loss|auc|dee|ddad|train] [--dump-outputs DIR]
 
-One JSON line on stdout (rank 0).  Workloads = BASELINE.json configs:
+One JSON line on stdout (rank 0).  K is the number of timed steps of the workload's headline number.  With
+--dump-outputs, rank 0 writes what the timed path computed in its last timed step as DIR/<name>.npy (see
+dump_outputs); the inputs are seeded, so two builds run with the same arguments can be compared output for output.
+The library must have been built before (__graft_entry__.build()): the bench compiles nothing.
+Workloads = BASELINE.json configs:
 
 loss   (headline; configs 1/3 loss shape) per GPU a batch of 8 images x the 4-scale pyramid (384x1280 ... 48x160,
        fp32, DEE normals, no mask, inv2depth fused) -> 5.22 Mpixel per step; a step is one forward + one backward
@@ -51,6 +55,29 @@ KITTI_N, KITTI_T = 102, 12
 KITTI_CROP = [44, 1197, 153, 371]
 DDAD_H, DDAD_W, DDAD_N = 1216, 1936, 8
 DEE_FRAMES = 148   # one frame per SM for the one-CTA-per-frame hysteresis
+DUMP_BYTES = 60 * 10**6   # --dump-outputs budget: stays under 64 MB with the .npy headers
+
+
+def dump_outputs(out_dir, arrays):
+    """Write every array as <out_dir>/<name>.npy: float64 for float64 data and integers wider than 16 bits, float32
+    (exact) otherwise.  When the set exceeds DUMP_BYTES, every array keeps the same share of its elements at flat
+    positions drawn by np.random.default_rng(0) (sorted), so that arrays of one size are sampled at the same positions
+    in every run."""
+    conv = {}
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        wide = a.dtype == np.float64 or (np.issubdtype(a.dtype, np.integer) and a.dtype.itemsize > 2)
+        conv[name] = a.astype(np.float64 if wide else np.float32)
+    total = sum(a.nbytes for a in conv.values())
+    share = min(1.0, DUMP_BYTES / total) if total else 1.0
+    picks = {}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in conv.items():
+        if share < 1.0:
+            if a.size not in picks:
+                picks[a.size] = np.sort(np.random.default_rng(0).choice(a.size, int(a.size * share), replace=False))
+            a = a.reshape(-1)[picks[a.size]]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def measured_peak_gbs():
@@ -308,7 +335,7 @@ def dee_frames(n, seed0):
 # ---------------------------------------------------------------------------
 # edge loss (headline)
 # ---------------------------------------------------------------------------
-def bench_loss(args, rank, world, device):
+def bench_loss(args, rank, world, device, outputs=None):
     import ctypes as C
     from mindtheedge_b200 import _lib
     from mindtheedge_b200.losses import _attrs, _scales_struct, multiscale_edge_loss
@@ -391,6 +418,12 @@ def bench_loss(args, rank, world, device):
                 graphs[i].replay()
         ms, _ = time_region(timed, world, device, stream)
         clocks = sampler.stop() if rank == 0 else None
+    if outputs is not None:   # the last timed step ran on set (steps - 1) % n_sets; the kernel split below rewrites it
+        _f, _b, gmap, gpred, losses = keep[(args.steps - 1) % n_sets][:5]
+        outputs["loss"] = losses.cpu().numpy()   # weighted total, then each scale's loss
+        for s in range(SCALES):
+            outputs[f"grad_map_s{s}"] = gmap[s].cpu().numpy()
+            outputs[f"grad_pred_s{s}"] = gpred[s].cpu().numpy()
     ms_per_step = ms / args.steps
     value = world * px_per_step / (ms_per_step * 1e-3) / 1e6
     loss_value = float(keep[0][4][0].item())
@@ -727,7 +760,7 @@ def bench_auc(args, rank, world, device, steps=None, warmup=None, ddad=False):
 # ---------------------------------------------------------------------------
 # DEE annotation post-process (config 4)
 # ---------------------------------------------------------------------------
-def bench_dee(args, rank, world, device):
+def bench_dee(args, rank, world, device, outputs=None):
     from mindtheedge_b200.tools import dee_postprocess
     n = DEE_FRAMES
     frames = dee_frames(n, 100 + 1000 * rank)      # frame i of the job -> rank i mod R: every rank has its own frames
@@ -744,10 +777,15 @@ def bench_dee(args, rank, world, device):
         sampler.start()
         sampler.settle(step)
     def timed():
-        for _ in range(args.steps):   # outputs are dropped at once: the allocator reuses the same blocks every step
+        for _ in range(args.steps - 1):   # outputs are dropped at once: the allocator reuses the same blocks every step
             step()
-    ms, _ = time_region(timed, world, device)
+        return step()
+    ms, (nrm_last, edges_last) = time_region(timed, world, device)
     clocks = sampler.stop() if rank == 0 else None
+    if outputs is not None:
+        outputs["normals"] = nrm_last.cpu().numpy()
+        outputs["edges"] = edges_last.cpu().numpy()
+    del nrm_last, edges_last
     ms /= args.steps
     value = world * px / (ms * 1e-3) / 1e6
     parts = {}
@@ -850,7 +888,7 @@ def make_trunk():
     return Trunk()
 
 
-def bench_train(args, rank, world, device):
+def bench_train(args, rank, world, device, outputs=None):
     """models/SemiSupEdgeModel.py:98-162 in miniature: trunk -> 4 inverse-depth scales -> edge loss over all scales
     (compute_edge_loss_with_all_scales :164-198: inv2depth, GradLoss per scale, sum, / 4) -> backward -> optimizer
     step (trainers/common_trainer.py:111-143); DDP all-reduces the trunk's gradient buckets over NCCL."""
@@ -906,7 +944,7 @@ def bench_train(args, rank, world, device):
     for name, fn in (("mte", loss_mte), ("eager", loss_eager)):
         for _ in range(max(3, args.warmup)):
             step(fn)
-        steps = max(3, min(args.steps, 20))
+        steps = args.steps if name == "mte" else max(3, min(args.steps, 20))   # the eager arm is a side number
         sampler = ClockSampler(torch.cuda.current_device())
         if rank == 0 and name == "mte":
             sampler.start()
@@ -914,6 +952,9 @@ def bench_train(args, rank, world, device):
         ms, last = time_region(lambda: [step(fn, ev[i]) for i in range(steps)][-1], world, device)
         if rank == 0 and name == "mte":
             res["clocks"] = sampler.stop()
+        if outputs is not None and name == "mte":
+            outputs["loss"] = last.detach().cpu().numpy().reshape(1)
+            outputs["trunk_params"] = torch.cat([p.detach().reshape(-1) for p in trunk.parameters()]).cpu().numpy()
         res[name] = {"ms_per_step": round(ms / steps, 3), "steps": steps,
                      "loss_fwd_ms": round(float(np.median([a.elapsed_time(b) for a, b in ev])), 4),
                      "loss": float(last.item())}
@@ -1154,7 +1195,13 @@ def main():
     ap.add_argument("--impl", default="mte", choices=["mte", "reference"])
     ap.add_argument("--workload", default="loss", choices=["loss", "auc", "dee", "ddad", "train"])
     ap.add_argument("--no-secondary", action="store_true", help="skip the second workload and the CPU baselines")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32/float64, <= 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl mte)")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         run_reference(args)
@@ -1165,10 +1212,8 @@ def main():
     torch.cuda.set_device(local)
     device = torch.device("cuda", local)
     host_cores = bind_to_gpu_cores(local, world)
-    from mindtheedge_b200 import build
-    if rank == 0:
-        build.build()
-    barrier(world)
+    from mindtheedge_b200 import _lib  # noqa: F401  (fails at once when libmte.so has not been built)
+    outputs = {} if args.dump_outputs and rank == 0 else None
 
     def finish_auc(a):
         return {"metric": a["metric"], "value": a["value"], "unit": a["unit"], "n_gpus": world, "steps": args.steps,
@@ -1180,25 +1225,23 @@ def main():
                 **({"uncropped": a["uncropped"]} if "uncropped" in a else {})}
 
     if args.workload == "loss":
-        line = bench_loss(args, rank, world, device)
+        line = bench_loss(args, rank, world, device, outputs)
         if not args.no_secondary:
             a = bench_auc(args, rank, world, device, steps=max(2, min(args.steps, 5)), warmup=3)
             a.pop("clocks", None)
             line["auc_eval"] = a
-    elif args.workload == "auc":
-        if args.steps > 200:
-            args.steps = 200
-        line = finish_auc(bench_auc(args, rank, world, device))
-    elif args.workload == "ddad":
-        if args.steps > 100:
-            args.steps = 100
-        line = finish_auc(bench_auc(args, rank, world, device, ddad=True))
+            if outputs is not None:
+                outputs["auc_eval_counts"] = np.array(a["counts"])
+    elif args.workload in ("auc", "ddad"):
+        line = finish_auc(bench_auc(args, rank, world, device, ddad=args.workload == "ddad"))
+        if outputs is not None:
+            outputs["counts"] = np.array(line["counts"])
     elif args.workload == "dee":
-        if args.steps > 200:
-            args.steps = 200
-        line = bench_dee(args, rank, world, device)
+        line = bench_dee(args, rank, world, device, outputs)
     else:
-        line = bench_train(args, rank, world, device)
+        line = bench_train(args, rank, world, device, outputs)
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     line["host_cores_bound"] = host_cores
     if rank == 0 and not args.no_secondary:
         line["cpu_baseline"] = cpu_baseline_subprocess(args.workload)

@@ -177,6 +177,25 @@ def test_reference_arm_prints_one_contract_line():
     assert d["e2e"]["h2d_bytes_per_step"] == 0 and d["e2e"]["d2h_bytes_per_step"] == 0 and d["e2e"]["value"] == d["value"]
 
 
+def test_bench_dump_outputs_types_and_budget(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: float64 for float64 / int64 data and float32 for u8 / fp32, whole arrays while the set
+    fits the budget; over it, every array of one size is sampled at the same seeded positions in every run."""
+    import bench
+    small = {"counts": np.arange(12, dtype=np.int64).reshape(3, 4), "edges": np.arange(6, dtype=np.uint8).reshape(2, 3)}
+    bench.dump_outputs(str(tmp_path / "small"), small)
+    c, e = np.load(tmp_path / "small" / "counts.npy"), np.load(tmp_path / "small" / "edges.npy")
+    assert c.dtype == np.float64 and np.array_equal(c, small["counts"])
+    assert e.dtype == np.float32 and np.array_equal(e, small["edges"])
+    monkeypatch.setattr(bench, "DUMP_BYTES", 6000)
+    big = {"a": np.arange(1000, dtype=np.float32).reshape(10, 100), "b": np.arange(1000, dtype=np.float64) * 2}
+    for run in ("r1", "r2"):
+        bench.dump_outputs(str(tmp_path / run), big)
+    a, b = np.load(tmp_path / "r1" / "a.npy"), np.load(tmp_path / "r1" / "b.npy")
+    assert a.nbytes + b.nbytes <= 6000 and a.size == b.size == 500
+    assert (np.diff(a) > 0).all() and np.array_equal(b, 2 * a.astype(np.float64))
+    assert np.array_equal(a, np.load(tmp_path / "r2" / "a.npy"))
+
+
 def test_atan2_candidate_error_bound():
     """dee_front_tma_kernel (csrc/dee.cu: atan2_candidate) lets an fp32 angle candidate decide the u8 normal level and
     the NMS bin ALONE when it is >= 1e-3 levels / 5e-5 bin units away from every boundary.  That needs a hard bound
