@@ -187,12 +187,22 @@ int mte_dee_postprocess(const void *prob, int in_dtype, int n_images, int H, int
  * thinner replaces py-bsds500 thin.binary_thin (:45, :125).
  * ------------------------------------------------------------------------ */
 size_t mte_pr_workspace_bytes(int n_images, int H, int W, int n_thresholds, double max_dist);
+/* workspace of mte_pr_counts with apply_thinning = 1: the above plus a slab of
+ * thinned bit planes (about 64 MB at most, less for small batches) */
+size_t mte_pr_thin_workspace_bytes(int n_images, int H, int W, int n_thresholds, double max_dist);
 /* pred: [N,H,W] of pred_dtype:
  *   MTE_F32/MTE_F64 strength map, thresholded as pred >= thresholds[t] (in fp64)
  *   MTE_U8          level plane from mte_canny_from_depth: edge at t iff level <= t
  * gt: [N,H,W] u8, non-zero = boundary.  crop = {x0,x1,y0,y1} (python slices
  * [y0:y1, x0:x1], clipped) or NULL.  counts: device int64[T,4] in the order
- * count_r,sum_r,count_p,sum_p, ACCUMULATED into (zero it first). */
+ * count_r,sum_r,count_p,sum_p, ACCUMULATED into (zero it first).
+ * apply_thinning: 0 = match the binarised window as it is; 1 = thin it first
+ * (evaluate_boundaries' default, eval_depth_edges.py:125): the window is cut
+ * out of the plane BEFORE it is thinned, so thinning zero-pads at the crop
+ * border, not at the plane border, and runs to convergence; sum_p is then the
+ * size of the thinned set.  Thresholds may come in any order and repeat (row t
+ * of counts belongs to thresholds[t]); the workspace must hold
+ * mte_pr_thin_workspace_bytes.  Any other value is MTE_ERR_ARG. */
 int mte_pr_counts(const void *pred, int pred_dtype, const uint8_t *gt, int n_images, int H, int W,
                   const int32_t *crop_host, const double *thresholds_host, int n_thresholds, double max_dist,
                   int apply_thinning, int64_t *counts, void *workspace, size_t workspace_bytes,

@@ -12,6 +12,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("MTE_LIB", os.path.join(_HERE, "libmte.so"))  # MTE_LIB: A/B builds while tuning
 
 MTE_MAX_SCALES = 4
+MTE_MAX_THRESHOLDS = 254
 MTE_WS_HEADER_BYTES = 65536
 MTE_F32, MTE_F64, MTE_U8 = 0, 1, 2
 MTE_LOSS_CE, MTE_LOSS_ATTENTION, MTE_LOSS_SPATIAL, MTE_LOSS_DICE = 1, 2, 4, 8
@@ -55,6 +56,7 @@ _SIGNATURES = {
     "mte_dee_workspace_bytes": (_sz, [_i, _i, _i]),
     "mte_dee_postprocess": (_i, [_vp, _i, _i, _i, _i, _i, _i, _d, _d, _vp, _vp, _i, _vp, _sz, _vp]),
     "mte_pr_workspace_bytes": (_sz, [_i, _i, _i, _i, _d]),
+    "mte_pr_thin_workspace_bytes": (_sz, [_i, _i, _i, _i, _d]),
     "mte_pr_counts": (_i, [_vp, _i, _vp, _i, _i, _i, C.POINTER(C.c_int32), C.POINTER(C.c_double), _i, _d, _i,
                            _vp, _vp, _sz, _vp]),
     "mte_match_workspace_bytes": (_sz, [_i, _i, _i, _d]),

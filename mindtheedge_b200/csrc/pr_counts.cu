@@ -16,11 +16,16 @@
 //   vertex-disjoint augmenting path per tree, claimed with CAS }
 //   until an (exhaustive) phase finds no free GT pixel => no augmenting path exists => maximum.
 // Per-pixel state is 16-bit offset codes in an L2-resident per-CTA arena; nothing is allocated.
+// With apply_thinning = 1 every problem's window is thinned first (thin_window_kernel below) and the per-problem
+// matchers read the thinned bit planes.
 #include <math.h>
 #include <stdlib.h>
 #include <string.h>
 
+#include <algorithm>
+
 #include "common.cuh"
+#include "thin.cuh"
 
 namespace mte {
 namespace pr {
@@ -32,10 +37,14 @@ constexpr unsigned short kDead = 0xFFFE;  // predicted pixel without any GT pixe
 constexpr int kMaxOffsets = 0xFFF0;
 constexpr int kCtasPerSm = 2;
 
-enum { IN_LEVELS = 0, IN_BINARY = 1, IN_F32 = 2, IN_F64 = 3 };
+enum { IN_LEVELS = 0, IN_BINARY = 1, IN_F32 = 2, IN_F64 = 3, IN_BITS = 4 };
 
 struct MatchP {
     const void *pred;          // [N,H,W] levels u8 / binary u8 / f32 / f64   (binary mode: [nProblems,H,W])
+    const unsigned *bits;      // bits mode: one thinned bit plane of the window per problem of the chunk
+    size_t bitsPlane;          // stride of the bit planes in words (h rows of bitsNw words, rounded up)
+    int bitsNw;
+    int probBase;              // global index of the chunk's first problem (image = g / T, threshold = g % T)
     const unsigned char *gt;   // [N,H,W]   (binary mode: [nProblems,H,W])
     int inMode;
     int N, H, W, T;
@@ -101,13 +110,26 @@ __device__ __forceinline__ unsigned short cas16(unsigned short *addr, unsigned s
     return atomicCAS(addr, expected, val);
 }
 
+// the binarisation rule of a threshold sweep: level plane -> level <= t, strength map -> pred >= thr[t] in fp64
+// (NaN is never set).  o indexes the [N,H,W] plane.
+__device__ __forceinline__ bool sweep_pred(const void *pred, int inMode, size_t o, int t, const double *thr) {
+    switch (inMode) {
+        case IN_LEVELS: return ((const unsigned char *)pred)[o] <= t;
+        case IN_F32: return (double)((const float *)pred)[o] >= thr[t];
+        default: return ((const double *)pred)[o] >= thr[t];
+    }
+}
+
+// prob: the problem's index within the launch (bits and binary modes index their planes with it)
 __device__ __forceinline__ bool is_pred(const MatchP &P, int img, int t, int prob, int gy, int gx) {
     const size_t o = (size_t)gy * P.W + gx;
     switch (P.inMode) {
-        case IN_LEVELS: return ((const unsigned char *)P.pred)[(size_t)img * P.H * P.W + o] <= t;
         case IN_BINARY: return ((const unsigned char *)P.pred)[(size_t)prob * P.H * P.W + o] != 0;
-        case IN_F32: return (double)((const float *)P.pred)[(size_t)img * P.H * P.W + o] >= P.thr[t];
-        default: return ((const double *)P.pred)[(size_t)img * P.H * P.W + o] >= P.thr[t];
+        case IN_BITS: {
+            const int y = gy - P.y0, x = gx - P.x0;
+            return (P.bits[(size_t)prob * P.bitsPlane + (size_t)y * P.bitsNw + (x >> 5)] >> (x & 31)) & 1u;
+        }
+        default: return sweep_pred(P.pred, P.inMode, (size_t)img * P.H * P.W + o, t, P.thr);
     }
 }
 
@@ -142,8 +164,9 @@ __global__ void __launch_bounds__(kThreads) match_kernel(const __grid_constant__
         const int prob = sProblem;
         if (prob >= P.nProblems) break;
         // problems are ordered image-major so consecutive CTAs share the GT plane in L2
-        const int img = (P.inMode == IN_BINARY) ? prob : prob / P.T;
-        const int t = (P.inMode == IN_BINARY) ? 0 : prob - img * P.T;
+        const int g = P.probBase + prob;
+        const int img = (P.inMode == IN_BINARY) ? prob : g / P.T;
+        const int t = (P.inMode == IN_BINARY) ? 0 : g - img * P.T;
         const unsigned char *gt = P.gt + (size_t)img * P.H * P.W;
         if (threadIdx.x == 0) { sNP = 0; sNQ = 0; sMatched = 0; }
         __syncthreads();
@@ -407,8 +430,9 @@ __global__ void __launch_bounds__(kSmThreads, 1) match_smem_kernel(const __grid_
         __syncthreads();
         const int prob = sProblem;
         if (prob >= P.nProblems) break;
-        const int img = (P.inMode == IN_BINARY) ? prob : prob / P.T;
-        const int t = (P.inMode == IN_BINARY) ? 0 : prob - img * P.T;
+        const int g = P.probBase + prob;
+        const int img = (P.inMode == IN_BINARY) ? prob : g / P.T;
+        const int t = (P.inMode == IN_BINARY) ? 0 : g - img * P.T;
         const unsigned char *gt = P.gt + (size_t)img * P.H * P.W;
         if (threadIdx.x == 0) { sNP = 0; sNQ = 0; sMatched = 0; }
         __syncthreads();
@@ -1335,6 +1359,50 @@ __global__ void __launch_bounds__(kSwThreads, 1) match_sweep_kernel(const __grid
 }
 
 // ---------------------------------------------------------------------------
+// Thinned sweep (apply_thinning = 1): one CTA per (image, threshold) problem of a chunk binarises its window with
+// the sweep rule, thins it to convergence with the bit-parallel routine of thin.cuh (zero padding at the WINDOW
+// border: the reference crops before it thins) and writes the thinned bit plane to the problem's slot of the slab.
+// The per-problem matchers then read the slab in IN_BITS mode.  The two bit planes live in dynamic shared memory when
+// they fit (KITTI crop 218 x 1153: 2 x 32.3 KB), else the slab slot and a scratch slot of the workspace are used.
+// ---------------------------------------------------------------------------
+struct ThinP {
+    const void *pred;   // [N,H,W] levels u8 / f32 / f64
+    int inMode, H, W, T;
+    int x0, y0, w, h, nw;
+    size_t plane;       // stride of the bit planes in words: h * nw rounded up to 64 (the words past h * nw are unused)
+    unsigned *slab;     // [chunk][plane] thinned planes (out)
+    unsigned *scratch;  // [chunk][plane] second plane of the global-memory path
+    int probBase;
+};
+struct ThrTable {
+    double v[MTE_MAX_THRESHOLDS];
+};
+
+__global__ void __launch_bounds__(thin::kThreads) thin_window_kernel(const __grid_constant__ ThinP Q,
+                                                                     const __grid_constant__ ThrTable thr, int inSmem) {
+    extern __shared__ __align__(16) unsigned char dyn[];
+    const int g = Q.probBase + (int)blockIdx.x;
+    const int img = g / Q.T, t = g - img * Q.T;
+    unsigned *slab = Q.slab + blockIdx.x * Q.plane;
+    unsigned *a = inSmem ? reinterpret_cast<unsigned *>(dyn) : slab;
+    unsigned *b = inSmem ? a + Q.plane : Q.scratch + blockIdx.x * Q.plane;
+    const size_t imgBase = (size_t)img * Q.H * Q.W;
+    const size_t n = (size_t)Q.h * Q.nw;  // the window's words: row y < h only, never the stride's padding
+    // binarise: one warp per word, one lane per pixel (bits past w stay zero)
+    const int lane = threadIdx.x & 31;
+    for (size_t i = threadIdx.x >> 5; i < n; i += thin::kThreads / 32) {
+        const int y = (int)(i / Q.nw), x = (int)(i - (size_t)y * Q.nw) * 32 + lane;
+        const bool set = x < Q.w && sweep_pred(Q.pred, Q.inMode, imgBase + (size_t)(Q.y0 + y) * Q.W + Q.x0 + x, t, thr.v);
+        const unsigned m = __ballot_sync(MTE_FULL_MASK, set);
+        if (lane == 0) a[i] = m;
+    }
+    __syncthreads();
+    const unsigned *r = thin::thin_plane(a, b, Q.h, Q.nw, -1);
+    if (r != slab)
+        for (size_t i = threadIdx.x; i < n; i += thin::kThreads) slab[i] = r[i];
+}
+
+// ---------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------
 struct OffsetTable {
@@ -1507,8 +1575,9 @@ static int launch(MatchP &P, const Layout &L, char *ws, double max_dist, const d
     const bool useSmem = SL.capP > 0 && tb.n <= kSmemTableOff && !debug_knob("MTE_MATCH_DENSE");
     // threshold sweeps (level planes; strength maps with ascending thresholds): one CTA per image solves all T nested
     // problems incrementally; what does not fit falls through to the per-problem kernels via the overflow list
-    bool sweep = useSmem && P.counts && !P.matchA && !P.matchB && P.inMode != IN_BINARY && P.T > 1 &&
-                 !debug_knob("MTE_MATCH_NO_SWEEP");
+    // (thinned sets are not nested: the bits mode never sweeps)
+    bool sweep = useSmem && P.counts && !P.matchA && !P.matchB && P.inMode != IN_BINARY && P.inMode != IN_BITS &&
+                 P.T > 1 && !debug_knob("MTE_MATCH_NO_SWEEP");
     if (sweep && P.inMode != IN_LEVELS)
         for (int t = 1; t < P.T; t++)
             if (!(thr_host[t] > thr_host[t - 1])) sweep = false;
@@ -1586,6 +1655,66 @@ extern "C" size_t mte_pr_workspace_bytes(int n_images, int H, int W, int T, doub
     return layout(n_images * T, H, W, T).total;
 }
 
+// The thinned sweep's slab (plus the scratch planes of the global-memory thinning path) follows the matcher's
+// workspace.  It is sized for chunks of the uncropped plane with both planes in global memory and kept to about
+// kThinSlabBudget, so the thinned planes of a chunk stay in L2 between the thinning and the matching launch; a call
+// with a crop or with shared-memory thinning fits more problems into the same bytes.
+constexpr size_t kThinSlabBudget = (size_t)64 << 20;
+
+static size_t thin_plane_bytes(int h, int w) { return align_up((size_t)h * thin::words_per_row(w) * 4, 256); }
+
+static size_t thin_region_bytes(int nProblems, int H, int W) {
+    const size_t per = 2 * thin_plane_bytes(H, W);
+    size_t chunk = kThinSlabBudget / per;
+    if (chunk < 1) chunk = 1;
+    if (chunk > (size_t)nProblems) chunk = (size_t)nProblems;
+    return chunk * per;
+}
+
+extern "C" size_t mte_pr_thin_workspace_bytes(int n_images, int H, int W, int T, double max_dist) {
+    if (n_images < 1 || H < 1 || W < 1 || T < 1) return 0;
+    (void)max_dist;
+    return layout(n_images * T, H, W, T).total + thin_region_bytes(n_images * T, H, W);
+}
+
+static int pr_counts_thinned(MatchP &P, const Layout &L, char *ws, double max_dist, const double *thr_host,
+                             cudaStream_t st) {
+    ThinP Q;
+    memset(&Q, 0, sizeof(Q));
+    Q.pred = P.pred; Q.inMode = P.inMode; Q.H = P.H; Q.W = P.W; Q.T = P.T;
+    Q.x0 = P.x0; Q.y0 = P.y0; Q.w = P.w; Q.h = P.h; Q.nw = thin::words_per_row(P.w);
+    Q.plane = thin_plane_bytes(P.h, P.w) / 4;
+    ThrTable tt;
+    memset(&tt, 0, sizeof(tt));
+    if (thr_host) memcpy(tt.v, thr_host, sizeof(double) * P.T);
+    const size_t smem = 2 * Q.plane * 4;
+    bool inSmem = smem <= (size_t)dev_info().smemOptin;
+    if (inSmem && opt_in_smem((const void *)thin_window_kernel, (int)smem) != cudaSuccess) {
+        cudaGetLastError();
+        inSmem = false;
+    }
+    const size_t region = thin_region_bytes(P.nProblems, P.H, P.W);
+    int chunk = (int)std::min(region / ((inSmem ? 1 : 2) * Q.plane * 4), (size_t)P.nProblems);
+    Q.slab = reinterpret_cast<unsigned *>(ws + L.total);
+    Q.scratch = Q.slab + (size_t)chunk * Q.plane;
+    P.inMode = IN_BITS;
+    P.bits = Q.slab;
+    P.bitsPlane = Q.plane;
+    P.bitsNw = Q.nw;
+    const int nAll = P.nProblems;
+    for (int base = 0; base < nAll; base += chunk) {
+        const int n = std::min(chunk, nAll - base);
+        Q.probBase = base;
+        thin_window_kernel<<<n, thin::kThreads, inSmem ? smem : 0, st>>>(Q, tt, inSmem ? 1 : 0);
+        MTE_RETURN_IF_CUDA_ERROR();
+        P.probBase = base;
+        P.nProblems = n;
+        const int rc = launch(P, L, ws, max_dist, nullptr, st);
+        if (rc) return rc;
+    }
+    return MTE_OK;
+}
+
 extern "C" int mte_pr_counts(const void *pred, int pred_dtype, const uint8_t *gt, int N, int H, int W,
                              const int32_t *crop, const double *thresholds, int T, double max_dist,
                              int apply_thinning, int64_t *counts, void *workspace, size_t ws_bytes,
@@ -1594,10 +1723,11 @@ extern "C" int mte_pr_counts(const void *pred, int pred_dtype, const uint8_t *gt
     if (N < 1 || H < 1 || W < 1) return MTE_ERR_SHAPE;
     if (T < 1 || T > MTE_MAX_THRESHOLDS) return MTE_ERR_ARG;
     if (!(max_dist >= 0.0)) return MTE_ERR_ARG;
-    if (apply_thinning) return MTE_ERR_ARG;  // thinning runs as mte_binary_thin + mte_correspond_pixels (host layer)
+    if (apply_thinning != 0 && apply_thinning != 1) return MTE_ERR_ARG;
     if (pred_dtype != MTE_U8 && !thresholds) return MTE_ERR_NULL;
     const Layout L = layout(N * T, H, W, T);
-    if (ws_bytes < L.total) return MTE_ERR_WORKSPACE;
+    const size_t need = apply_thinning ? mte_pr_thin_workspace_bytes(N, H, W, T, max_dist) : L.total;
+    if (ws_bytes < need) return MTE_ERR_WORKSPACE;
     MatchP P;
     memset(&P, 0, sizeof(P));
     P.pred = pred; P.gt = gt;
@@ -1607,5 +1737,8 @@ extern "C" int mte_pr_counts(const void *pred, int pred_dtype, const uint8_t *gt
     P.nProblems = N * T;
     P.counts = reinterpret_cast<unsigned long long *>(counts);
     if (P.w == 0 || P.h == 0) return MTE_OK;  // empty window: nothing to count
+    if (apply_thinning)
+        return pr_counts_thinned(P, L, static_cast<char *>(workspace), max_dist, thresholds,
+                                 reinterpret_cast<cudaStream_t>(stream));
     return launch(P, L, static_cast<char *>(workspace), max_dist, thresholds, reinterpret_cast<cudaStream_t>(stream));
 }

@@ -5,96 +5,51 @@
 // neighbourhood satisfies G1 & G2 & G3 (first) or G1 & G2 & G3' (second) of Lam, Lee & Suen, until a
 // sub-iteration deletes nothing.  PARITY UNPINNED (restated from the published algorithm, see oracle/thin.py).
 //
-// One CTA per image: the plane ping-pongs between the output buffer and a workspace plane (both L2 resident
-// for the crop sizes of the metric), a 256-entry deletion LUT per sub-iteration sits in shared memory.
-#include "common.cuh"
+// One CTA per image: the byte plane is packed into a bit plane, thinned by the bit-parallel routine of thin.cuh and
+// unpacked again.  The two bit planes live in dynamic shared memory when they fit (384 x 1280: 2 x 61.4 KB), else in
+// the CTA's slice of the workspace.
+#include "thin.cuh"
 
 namespace mte {
 namespace thin {
 
-constexpr int kThreads = 1024;
-
-struct Luts {
-    unsigned int bits[2][8];  // 256-bit deletion tables
-};
-
-// neighbour numbering x1..x8 starts east and runs counter-clockwise; bit k-1 of the code is x_k
-static Luts build_luts() {
-    Luts L;
-    for (int s = 0; s < 2; s++)
-        for (int i = 0; i < 8; i++) L.bits[s][i] = 0;
-    for (int c = 0; c < 256; c++) {
-        int x[10];
-        x[0] = 0;
-        for (int k = 1; k <= 8; k++) x[k] = (c >> (k - 1)) & 1;
-        x[9] = x[1];
-        int b = 0, n1 = 0, n2 = 0;
-        for (int i = 1; i <= 4; i++) {
-            if (x[2 * i - 1] == 0 && (x[2 * i] || x[2 * i + 1])) b++;
-            if (x[2 * i - 1] || x[2 * i]) n1++;
-            if (x[2 * i] || x[2 * i + 1]) n2++;
-        }
-        const int mn = n1 < n2 ? n1 : n2;
-        const bool g1 = b == 1, g2 = mn >= 2 && mn <= 3;
-        const bool g3 = ((x[2] || x[3] || !x[8]) && x[1]) == 0;
-        const bool g3p = ((x[6] || x[7] || !x[4]) && x[5]) == 0;
-        if (g1 && g2 && g3) L.bits[0][c >> 5] |= 1u << (c & 31);
-        if (g1 && g2 && g3p) L.bits[1][c >> 5] |= 1u << (c & 31);
-    }
-    return L;
-}
-
-__device__ __forceinline__ int px(const unsigned char *p, int y, int x, int H, int W) {
-    return (y >= 0 && y < H && x >= 0 && x < W) ? (p[(size_t)y * W + x] != 0) : 0;
-}
-
-__global__ void __launch_bounds__(kThreads) thin_kernel(const unsigned char *__restrict__ in,
-                                                        unsigned char *__restrict__ out,
-                                                        unsigned char *__restrict__ tmp, int H, int W, int max_iter,
-                                                        const __grid_constant__ Luts L) {
-    __shared__ unsigned int lut[2][8];
-    if (threadIdx.x < 16) lut[threadIdx.x >> 3][threadIdx.x & 7] = L.bits[threadIdx.x >> 3][threadIdx.x & 7];
+__global__ void __launch_bounds__(kThreads) binary_thin_kernel(const unsigned char *__restrict__ in,
+                                                               unsigned char *__restrict__ out, unsigned *planes,
+                                                               int H, int W, int max_iter, int inSmem) {
+    extern __shared__ __align__(16) unsigned dyn[];
+    const int nw = words_per_row(W);
+    const size_t pw = (size_t)H * nw;
+    unsigned *a = inSmem ? dyn : planes + blockIdx.x * 2 * pw;
+    unsigned *b = a + pw;
     const size_t plane = (size_t)H * W;
-    const unsigned char *src0 = in + blockIdx.x * plane;
-    unsigned char *a = out + blockIdx.x * plane, *b = tmp + blockIdx.x * plane;
-    for (size_t i = threadIdx.x; i < plane; i += kThreads) a[i] = src0[i] != 0;
-    __syncthreads();
-    // a always holds the current image; b receives the result of a sub-iteration, then they swap
-    for (int it = 0; max_iter < 0 || it < max_iter; it++) {
-        bool stop = false;
-        for (int s = 0; s < 2; s++) {
-            int killed = 0;
-            for (size_t i = threadIdx.x; i < plane; i += kThreads) {
-                const int y = (int)(i / W), x = (int)(i - (size_t)y * W);
-                unsigned char v = a[i];
-                if (v) {
-                    const int code = px(a, y, x + 1, H, W) | (px(a, y - 1, x + 1, H, W) << 1) |
-                                     (px(a, y - 1, x, H, W) << 2) | (px(a, y - 1, x - 1, H, W) << 3) |
-                                     (px(a, y, x - 1, H, W) << 4) | (px(a, y + 1, x - 1, H, W) << 5) |
-                                     (px(a, y + 1, x, H, W) << 6) | (px(a, y + 1, x + 1, H, W) << 7);
-                    if ((lut[s][code >> 5] >> (code & 31)) & 1u) { v = 0; killed = 1; }
-                }
-                b[i] = v;
-            }
-            if (!__syncthreads_or(killed)) { stop = true; break; }  // nothing deleted: a is the result
-            unsigned char *t = a; a = b; b = t;
-        }
-        if (stop) break;
+    const unsigned char *src = in + blockIdx.x * plane;
+    // pack: one warp per word, one lane per pixel (bits past W stay zero)
+    const int lane = threadIdx.x & 31;
+    for (size_t i = threadIdx.x >> 5; i < pw; i += kThreads / 32) {
+        const int y = (int)(i / nw), x = (int)(i - (size_t)y * nw) * 32 + lane;
+        const unsigned m = __ballot_sync(MTE_FULL_MASK, x < W && src[(size_t)y * W + x] != 0);
+        if (lane == 0) a[i] = m;
     }
     __syncthreads();
+    const unsigned *r = thin_plane(a, b, H, nw, max_iter);
     unsigned char *dst = out + blockIdx.x * plane;
-    if (a != dst)
-        for (size_t i = threadIdx.x; i < plane; i += kThreads) dst[i] = a[i];
+    for (size_t i = threadIdx.x; i < plane; i += kThreads) {
+        const int y = (int)(i / W), x = (int)(i - (size_t)y * W);
+        dst[i] = (unsigned char)((r[(size_t)y * nw + (x >> 5)] >> (x & 31)) & 1u);
+    }
 }
+
+static size_t planes_bytes(int H, int W) { return (size_t)2 * H * words_per_row(W) * sizeof(unsigned); }
 
 }  // namespace thin
 }  // namespace mte
 
 using namespace mte;
 
+// covers the global-memory bit planes of every image (the shared-memory path needs none of it)
 extern "C" size_t mte_thin_workspace_bytes(int N, int H, int W) {
     if (N < 1 || H < 1 || W < 1) return 0;
-    return MTE_WS_HEADER_BYTES + align_up((size_t)N * H * W, 256);
+    return MTE_WS_HEADER_BYTES + align_up((size_t)N * thin::planes_bytes(H, W), 256);
 }
 
 extern "C" int mte_binary_thin(const uint8_t *in, uint8_t *out, int N, int H, int W, int max_iter, void *workspace,
@@ -102,9 +57,15 @@ extern "C" int mte_binary_thin(const uint8_t *in, uint8_t *out, int N, int H, in
     if (!in || !out || !workspace) return MTE_ERR_NULL;
     if (N < 1 || H < 1 || W < 1) return MTE_ERR_SHAPE;
     if (ws_bytes < mte_thin_workspace_bytes(N, H, W)) return MTE_ERR_WORKSPACE;
-    static const thin::Luts L = thin::build_luts();
-    unsigned char *tmp = static_cast<unsigned char *>(workspace) + MTE_WS_HEADER_BYTES;
-    thin::thin_kernel<<<N, thin::kThreads, 0, reinterpret_cast<cudaStream_t>(stream)>>>(in, out, tmp, H, W, max_iter, L);
+    const size_t smem = thin::planes_bytes(H, W);
+    bool inSmem = smem <= (size_t)dev_info().smemOptin;
+    if (inSmem && opt_in_smem((const void *)thin::binary_thin_kernel, (int)smem) != cudaSuccess) {
+        cudaGetLastError();
+        inSmem = false;
+    }
+    unsigned *planes = reinterpret_cast<unsigned *>(static_cast<char *>(workspace) + MTE_WS_HEADER_BYTES);
+    thin::binary_thin_kernel<<<N, thin::kThreads, inSmem ? smem : 0, reinterpret_cast<cudaStream_t>(stream)>>>(
+        in, out, planes, H, W, max_iter, inSmem ? 1 : 0);
     MTE_RETURN_IF_CUDA_ERROR();
     return MTE_OK;
 }

@@ -45,7 +45,7 @@ _DT = {torch.float32: _lib.MTE_F32, torch.float64: _lib.MTE_F64, torch.uint8: _l
 # ---------------------------------------------------------------------------
 # tensor-level ops
 # ---------------------------------------------------------------------------
-def _pr_counts_cuda(pred, gt, thresholds, n_levels, max_dist, crop):
+def _pr_counts_cuda(pred, gt, thresholds, n_levels, max_dist, crop, apply_thinning=False):
     """CUDA implementation of ``mte::pr_counts`` -> int64 [T,4] (count_r, sum_r, count_p, sum_p)."""
     with runtime.on_device(pred, gt) as dev:
         pred, gt = pred.contiguous(), gt.contiguous()
@@ -58,9 +58,11 @@ def _pr_counts_cuda(pred, gt, thresholds, n_levels, max_dist, crop):
             thr = t.ctypes.data_as(C.POINTER(C.c_double))
         out = torch.zeros((T, 4), dtype=torch.int64, device=dev)
         cr = None if len(crop) == 0 else (C.c_int32 * 4)(*[int(v) for v in crop])
-        ws = runtime.workspace(dev, _lib.lib.mte_pr_workspace_bytes(N, H, W, T, float(max_dist)))
+        query = _lib.lib.mte_pr_thin_workspace_bytes if apply_thinning else _lib.lib.mte_pr_workspace_bytes
+        ws = runtime.workspace(dev, query(N, H, W, T, float(max_dist)))
         runtime.call("mte_pr_counts", dev, pred.data_ptr(), _DT[pred.dtype], gt.data_ptr(), N, H, W, cr, thr, T,
-                     float(max_dist), 0, out.data_ptr(), ws.data_ptr(), ws.numel(), runtime.current_stream_ptr(dev))
+                     float(max_dist), int(bool(apply_thinning)), out.data_ptr(), ws.data_ptr(), ws.numel(),
+                     runtime.current_stream_ptr(dev))
     return out
 
 
@@ -78,15 +80,15 @@ def _correspond_pixels_cuda(a, b, max_dist, want_maps):
     return ma, mb, cnt
 
 
-runtime.define_op("pr_counts(Tensor pred, Tensor gt, float[] thresholds, int n_levels, float max_dist, int[] crop) "
-                  "-> Tensor", _pr_counts_cuda)
+runtime.define_op("pr_counts(Tensor pred, Tensor gt, float[] thresholds, int n_levels, float max_dist, int[] crop, "
+                  "bool apply_thinning=False) -> Tensor", _pr_counts_cuda)
 runtime.define_op("correspond_pixels(Tensor a, Tensor b, float max_dist, bool want_maps) -> (Tensor, Tensor, Tensor)",
                   _correspond_pixels_cuda)
 
 
 def pr_counts(pred: torch.Tensor, gt: torch.Tensor, thresholds=None, *, n_levels: Optional[int] = None,
               max_dist: float = 0.0075, crop: Optional[Sequence[int]] = None,
-              out: Optional[torch.Tensor] = None) -> torch.Tensor:
+              out: Optional[torch.Tensor] = None, apply_thinning: bool = False) -> torch.Tensor:
     """Counts for a batch of images, one GT map each (torch custom op ``mte::pr_counts``).
 
     pred  [N,H,W] CUDA: float32/float64 strength map (``pred >= thresholds[t]``) or uint8 level
@@ -94,6 +96,9 @@ def pr_counts(pred: torch.Tensor, gt: torch.Tensor, thresholds=None, *, n_levels
           ``n_levels``).
     gt    [N,H,W] uint8, non-zero = boundary.
     crop  ``[x0, x1, y0, y1]`` as the reference's ``gt_crop`` (python slices ``[y0:y1, x0:x1]``).
+    apply_thinning  thin every binarised window before matching (``evaluate_boundaries``' default): the crop is
+          applied first, so thinning zero-pads at the crop border; ``sum_p`` counts the thinned pixels.  Thresholds
+          may then come in any order and repeat.
     ->    int64 [T,4] on the device, columns count_r, sum_r, count_p, sum_p, summed over the
           batch and ACCUMULATED into ``out`` when given."""
     runtime.require_cuda(pred, "pred")
@@ -113,7 +118,7 @@ def pr_counts(pred: torch.Tensor, gt: torch.Tensor, thresholds=None, *, n_levels
     else:
         thr = [float(v) for v in np.asarray(thresholds, dtype=np.float64)]
     c = torch.ops.mte.pr_counts(pred, gt, thr, int(n_levels or 0), float(max_dist),
-                                [] if crop is None else [int(v) for v in crop])
+                                [] if crop is None else [int(v) for v in crop], bool(apply_thinning))
     if out is None:
         return c
     out += c
@@ -155,15 +160,17 @@ def evaluate_boundaries(predicted_boundaries, gt_boundaries, thresholds=99, max_
     count_p = np.zeros(T)
     sum_p = np.zeros(T)
     d_pred = torch.from_numpy(pred).cuda()
-    if not apply_thinning and len(gt_boundaries) == 1:
+    if len(gt_boundaries) == 1 and (not apply_thinning or T <= _lib.MTE_MAX_THRESHOLDS):
         g_np = np.asarray(gt_boundaries[0])
         gt = torch.from_numpy(np.ascontiguousarray(g_np != 0).astype(np.uint8)).cuda()
-        c = pr_counts(d_pred[None], gt[None], thresholds, max_dist=max_dist).cpu().numpy()
+        c = pr_counts(d_pred[None], gt[None], thresholds, max_dist=max_dist,
+                      apply_thinning=bool(apply_thinning)).cpu().numpy()
         # the matcher sees "non-zero = boundary", but sum_r is gt.sum() (eval_depth_edges.py:138): for maps that are
         # not 0/1 (255-valued, soft, or multiplied by a fractional mask image) the two differ
         sum_r[:] = float(g_np.sum())
         return (c[:, 0].astype(np.float64), sum_r, c[:, 2].astype(np.float64), c[:, 3].astype(np.float64), thresholds)
-    # general path (thinning and/or several GT maps): binarise per threshold, thin, match against every GT
+    # general path (several GT maps, or more thresholds than one thinned sweep takes): binarise per threshold, thin,
+    # match against every GT
     from .bsds import thin as _thin
     thr_dev = torch.from_numpy(np.asarray(thresholds, dtype=np.float64)).cuda()
     bins = (d_pred.double()[None] >= thr_dev[:, None, None]).to(torch.uint8)  # [T,h,w]
