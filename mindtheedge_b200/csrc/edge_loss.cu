@@ -47,8 +47,10 @@ __global__ void __launch_bounds__(kThreads) edge_loss_bwd_pointwise_kernel(const
 // Bilinear resize (F.interpolate(mode='bilinear', align_corners=False),
 // grad_loss.py:127) -- only used when the prediction and target sizes differ.
 // ---------------------------------------------------------------------------
+// fp32 source coordinate, rounded once (fused multiply-add): this is what the reference's fp32 interpolation yields
+// (oracle bilinear_matrix restates it); at non-dyadic scales a second rounding moves the weights by up to 1e-4.
 __device__ __forceinline__ void src_index(int o, float scale, int n, int &i0, int &i1, float &f) {
-    float s = scale * ((float)o + 0.5f) - 0.5f;
+    float s = fmaf(scale, (float)o + 0.5f, -0.5f);
     s = s < 0.f ? 0.f : s;
     i0 = min((int)s, n - 1);
     i1 = min(i0 + 1, n - 1);
@@ -87,7 +89,9 @@ __global__ void resize_bwd_kernel(const float *__restrict__ gout, float *__restr
         if (x == w - 1) X1 = W - 1;
         Y0 = max(Y0, 0); X0 = max(X0, 0); Y1 = min(Y1, H - 1); X1 = min(X1, W - 1);
         const float *g = gout + (size_t)b * H * W;
-        float acc = 0.f;
+        // fp64 sum: a large upsampling gathers thousands of terms of both signs into one source pixel (1x1 -> 96x97:
+        // 9312), where an fp32 running sum drifts by ~5e-5 of the result
+        double acc = 0.0;
         for (int Y = Y0; Y <= Y1; Y++) {
             int a0, a1; float fy;
             src_index(Y, sy, h, a0, a1, fy);
@@ -101,10 +105,10 @@ __global__ void resize_bwd_kernel(const float *__restrict__ gout, float *__restr
                 float wx = 0.f;
                 if (b0 == x) wx += 1.f - fx;
                 if (b1 == x) wx += fx;
-                if (wx != 0.f) acc += wy * wx * g[(size_t)Y * W + X];
+                if (wx != 0.f) acc += (double)(wy * wx) * (double)g[(size_t)Y * W + X];
             }
         }
-        gin[i] = acc;
+        gin[i] = (float)acc;
     }
 }
 

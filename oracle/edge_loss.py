@@ -188,11 +188,19 @@ def responses_np(x: np.ndarray) -> np.ndarray:
 
 
 def bilinear_matrix(n_in: int, n_out: int) -> np.ndarray:
-    """1-D weights of F.interpolate(mode='bilinear', align_corners=False)."""
+    """1-D weights of F.interpolate(mode='bilinear', align_corners=False).
+
+    The reference computes the source coordinate in fp32 (area_pixel_compute_scale / _source_index with the float
+    opmath type): scale = float(n_in) / float(n_out), src = scale * (o + 0.5) - 0.5 rounded once
+    (torch's CPU kernel agrees with that to 1e-7 where two roundings are 1e-5 off).  For a
+    scale that is not dyadic (1242 -> 1280) that coordinate is off the exact one by up to ~1e-4 px, which moves the
+    interpolated value by up to 7e-5 of the depth range, so the weights are built from the same fp32 coordinate (the
+    interpolation itself stays fp64).  For dyadic scales the coordinate is exact either way."""
     M = np.zeros((n_out, n_in))
-    scale = n_in / n_out
+    scale = np.float32(n_in) / np.float32(n_out)
     for o in range(n_out):
-        src = max((o + 0.5) * scale - 0.5, 0.0)
+        src = float(np.float32(float(scale) * (o + 0.5) - 0.5))   # fp64 product + sum is exact: one fp32 rounding
+        src = max(src, 0.0)
         i0 = min(int(math.floor(src)), n_in - 1)
         i1 = min(i0 + 1, n_in - 1)
         f = src - i0
@@ -215,7 +223,7 @@ def edge_loss_np64(
         x = out
     else:
         Mr, Mc = bilinear_matrix(h, H), bilinear_matrix(w, W)
-        x = np.einsum("ij,bjk,lk->bil", Mr, out, Mc)
+        x = Mr @ out @ Mc.T          # matmul: a plain 3-operand einsum contracts in one O(h*w*H*W) loop
     m = np.ones_like(e) if gt_mask is None else np.asarray(gt_mask, dtype=np.float64)[:, 0]
 
     if is_grad:
@@ -268,5 +276,5 @@ def edge_loss_np64(
     else:
         dx = dl_dg
     if not same:
-        dx = np.einsum("ij,bil,lk->bjk", Mr, dx, Mc)
+        dx = Mr.T @ dx @ Mc
     return loss, g[:, None], dx[:, None]
