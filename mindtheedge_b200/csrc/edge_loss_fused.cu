@@ -53,27 +53,46 @@ __device__ __forceinline__ unsigned ld_acquire_u32(const unsigned *p) {
     asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
     return v;
 }
+__device__ __forceinline__ unsigned ld_relaxed_u32(const unsigned *p) {
+    unsigned v;
+    asm volatile("ld.relaxed.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
+    return v;
+}
+__device__ __forceinline__ unsigned atom_add_acq_rel_u32(unsigned *p, unsigned v) {
+    unsigned old;
+    asm volatile("atom.acq_rel.gpu.global.add.u32 %0, [%1], %2;" : "=r"(old) : "l"(p), "r"(v) : "memory");
+    return old;
+}
 
-// All CTAs of the (cooperative, co-resident) grid meet here once per launch.  The counter is reset by the last CTA
-// of the launch (every CTA has left the barrier before it takes its final ticket).
-__device__ __forceinline__ void grid_barrier(unsigned *ctr, unsigned nCtas) {
+// The grid barrier (all CTAs of the cooperative, co-resident grid, once per launch) in two halves, so that the first
+// segment's opening loads go out between them.  Memory model: what every CTA must see after the barrier is what the
+// CTAs wrote in phase 1, the fixed-point atomics into `accum` (phase 2 reads them with __ldcg) and the plain zero
+// stores of the seam rows (other CTAs red.add onto them later).  __syncthreads() orders every thread's phase-1
+// writes before thread 0's arrival, and a release is cumulative, so the release add publishes all of them: its
+// fence (MEMBAR.ALL.GPU, not the sequentially consistent MEMBAR.SC.GPU of __threadfence) waits until they have been
+// performed.  The waiter polls with relaxed loads (no L1 invalidate per poll), and one acquire load after it has seen
+// the full count synchronises with every arrival (they form one release sequence on the counter); __syncthreads()
+// passes that on to the CTA.  The counter is reset by the last CTA of the launch (every CTA has left the barrier
+// before it takes its final ticket).
+__device__ __forceinline__ void grid_arrive(unsigned *ctr) {
     __syncthreads();
+    if (threadIdx.x == 0) asm volatile("red.release.gpu.global.add.u32 [%0], 1;" ::"l"(ctr) : "memory");
+}
+__device__ __forceinline__ void grid_wait(const unsigned *ctr, unsigned nCtas) {
     if (threadIdx.x == 0) {
-        __threadfence();
-        atomicAdd(ctr, 1u);
 #ifdef MTE_FUSED_NOSLEEP
-        while (ld_acquire_u32(ctr) < nCtas) {}
+        while (ld_relaxed_u32(ctr) < nCtas) {}
 #else
-        while (ld_acquire_u32(ctr) < nCtas) __nanosleep(20);
+        while (ld_relaxed_u32(ctr) < nCtas) __nanosleep(20);
 #endif
-        __threadfence();
+        (void)ld_acquire_u32(ctr);
     }
     __syncthreads();
 }
 
 #ifdef MTE_FUSED_TRACE
-// timing build only (scripts/trace_fused.py): per-phase time stamps folded over all CTAs into eight u64 slots at byte
-// 1024 of the workspace header (min via max of the complement).  Breaks the zero-header invariant: never in a release.
+// timing build only (scripts/trace_fused.py): per-phase time stamps folded over all CTAs into ten u64 slots at byte
+// 1032 of the workspace header (min via max of the complement).  Breaks the zero-header invariant: never in a release.
 __device__ __forceinline__ unsigned long long gtime() {
     unsigned long long t;
     asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
@@ -444,16 +463,18 @@ __global__ void __maxnreg__(MTE_FUSED_REGS) edge_loss_fused_kernel(const __grid_
             }
         }
     }
-    // the first segment's opening loads go out before the barrier
+    MTE_TRACE(2, true);    // first CTA done with phase 1
+    MTE_TRACE(3, false);   // last CTA done with phase 1 (the last arrival follows)
+    grid_arrive(F.barrier);
+    // the first segment's opening loads go out while the other CTAs arrive
     int u0 = uBeg;
     Seg sg;
     bool have = false;
     while (u0 < uEnd && !have) have = next_segment(P, u0, uEnd, sg);
     float2 xa[2], xc[2];
     if (have) fused_prologue(P.s[sg.si], sg, lane, ring, xa, xc);
-    MTE_TRACE(2, true);    // first CTA done with phase 1
-    MTE_TRACE(3, false);   // last CTA done with phase 1
-    grid_barrier(F.barrier, gridDim.x);
+    grid_wait(F.barrier, gridDim.x);
+    MTE_TRACE(8, true);    // first CTA out of the barrier
     MTE_TRACE(4, false);   // last CTA out of the barrier
 #else
     __syncthreads();
@@ -504,15 +525,15 @@ __global__ void __maxnreg__(MTE_FUSED_REGS) edge_loss_fused_kernel(const __grid_
     }
     MTE_TRACE(5, true);    // first CTA done with phase 2
     MTE_TRACE(6, false);   // last CTA done with phase 2
-    // ---- the last CTA to leave folds alpha, the normalisers and the loss (same code as the two-kernel forward)
+    // ---- the last CTA to leave folds alpha, the normalisers and the loss (same code as the two-kernel forward).  The
+    // election needs only the accumulator atomics of every CTA ordered before its ticket; __syncthreads() + the
+    // release half of thread 0's acq_rel add publish them (MEMBAR.ALL.GPU, no sequentially consistent fence), and the
+    // acquire half lets the last CTA read the sums.  The grad_pred / grad_map stores are published by the kernel's end.
     __syncthreads();
-    if (threadIdx.x == 0) {
-        __threadfence();
-        sLast = atomicAdd(P.ticket + 1, 1u) == gridDim.x - 1u;
-        __threadfence();
-    }
+    if (threadIdx.x == 0) sLast = atom_add_acq_rel_u32(P.ticket + 1, 1u) == gridDim.x - 1u;
     __syncthreads();
     if (sLast) {
+        MTE_TRACE(9, false);   // the last CTA is elected
         finalize_loss<false>(P, sLoss);
         __syncthreads();
         if (threadIdx.x == 0) {
@@ -535,8 +556,12 @@ __global__ void __maxnreg__(MTE_FUSED_REGS) edge_loss_fused_kernel(const __grid_
 
 // d loss / d pred was produced for the expected upstream gradient; bring it to the actual one.  Exits at once when
 // they agree (the common case: loss.backward() with the expectation 1, or a steady training loop).
-__global__ void __launch_bounds__(128) edge_loss_rescale_kernel(const __grid_constant__ LossP P, const float *gradLoss,
-                                                                float *ctx, float *expectedOut) {
+// One wave of one CTA per SM: at <= 32 registers x 128 threads a CTA fits in the 4 K registers the fused kernel leaves
+// free, so every CTA is resident (waiting in pdl_wait) before the fused grid ends and none is scheduled after it.
+constexpr int kRescaleThreads = 128;
+constexpr int kRescaleVec = 4;   // float4 per thread in flight per iteration (the rescaling path streams grad_pred)
+__global__ void __launch_bounds__(kRescaleThreads, 65536 / (kRescaleThreads * 32))
+edge_loss_rescale_kernel(const __grid_constant__ LossP P, const float *gradLoss, float *ctx, float *expectedOut) {
     pdl_wait();   // launched as a programmatic dependent of the kernel that produces ctx and grad_pred
     float *cur = ctx + P.totalImages + 2 * MTE_MAX_SCALES;
     unsigned *done = reinterpret_cast<unsigned *>(ctx + P.totalImages + 3 * MTE_MAX_SCALES);
@@ -554,10 +579,18 @@ __global__ void __launch_bounds__(128) edge_loss_rescale_kernel(const __grid_con
         const float f = G / c;
         const size_t n4 = (size_t)S.B * S.H * S.W / 4;
         float4 *d = reinterpret_cast<float4 *>(S.dx);
-        for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (size_t)gridDim.x * blockDim.x) {
-            float4 v = d[i];
-            v.x *= f; v.y *= f; v.z *= f; v.w *= f;
-            d[i] = v;
+        const size_t step = (size_t)gridDim.x * kRescaleThreads * kRescaleVec;
+        for (size_t i0 = (size_t)blockIdx.x * kRescaleThreads * kRescaleVec + threadIdx.x; i0 < n4; i0 += step) {
+            float4 v[kRescaleVec];
+#pragma unroll
+            for (int u = 0; u < kRescaleVec; u++)
+                if (i0 + u * kRescaleThreads < n4) v[u] = d[i0 + u * kRescaleThreads];
+#pragma unroll
+            for (int u = 0; u < kRescaleVec; u++)
+                if (i0 + u * kRescaleThreads < n4) {
+                    v[u].x *= f; v[u].y *= f; v[u].z *= f; v[u].w *= f;
+                    d[i0 + u * kRescaleThreads] = v[u];
+                }
         }
     }
     // the last CTA records what grad_pred carries now (every CTA has read `cur` before taking its ticket)
@@ -689,8 +722,8 @@ extern "C" int mte_edge_loss_grad_rescale(const mte_loss_scale_t *sc, int n, con
     }
     P.nScales = n; P.totalImages = img;
     cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)num_sms() * 2u);
-    cfg.blockDim = dim3(128u);
+    cfg.gridDim = dim3((unsigned)num_sms());
+    cfg.blockDim = dim3((unsigned)kRescaleThreads);
     cfg.stream = reinterpret_cast<cudaStream_t>(stream);
     cudaLaunchAttribute at[1];
     at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
