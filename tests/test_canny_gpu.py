@@ -115,16 +115,15 @@ def test_hysteresis_fallback_when_reachable_set_exceeds_shared_memory():
     assert int((edges[2, 0] > 0).sum()) > 60000
 
 
-@pytest.mark.parametrize("force_big", [False, True])
-@pytest.mark.parametrize("shape", [(96, 1296), (64, 48), (200, 16), (384, 1280)])
-def test_hysteresis_padded_rows_and_global_bitmap_mode(shape, force_big, monkeypatch):
+@pytest.mark.parametrize("shape", [(96, 1296), (64, 48), (200, 16), (384, 1280),
+                                   (640, 1280), (600, 1296), (720, 1600), (1216, 1936)])
+def test_hysteresis_padded_rows_and_global_bitmap_mode(shape):
     """Shared-memory hysteresis on widths that are multiples of 16 but not of 32 (bitmap rows padded to whole words,
-    the DDAD width 1936 is one) and with the bitmaps forced into the image's global scratch (the mode DDAD-size planes
-    take): bit-exact with cv2.Canny for every nested pair."""
+    the DDAD width 1936 is one), and on planes whose bitmaps do not fit in shared memory, so they live in the image's
+    global scratch (BIG: more than 576 rows at W = 1280, padded rows at 600 x 1296, DDAD size): bit-exact with
+    cv2.Canny for every nested pair."""
     from mindtheedge_b200.edge import canny_from_depth
     from oracle.canny import quantise_depth
-    if force_big:
-        monkeypatch.setenv("MTE_HYST_BIG", "1")
     H, W = shape
     depths = np.stack([scene(H, W, 21 + k) for k in range(3)])
     depths[2] = np.random.default_rng(9).uniform(0, 90, (H, W)).astype(np.float32)
