@@ -207,6 +207,18 @@ int mte_pr_counts(const void *pred, int pred_dtype, const uint8_t *gt, int n_ima
                   const int32_t *crop_host, const double *thresholds_host, int n_thresholds, double max_dist,
                   int apply_thinning, int64_t *counts, void *workspace, size_t workspace_bytes,
                   mte_stream_t stream);
+/* The same counts per image, from the same single launch chain: counts is a
+ * device int64[N,T,4], row (i, t) holding image i's count_r,sum_r,count_p,sum_p
+ * for thresholds[t] (or level t), ACCUMULATED into as above.  Arguments,
+ * argument checks, workspace queries and return codes are those of
+ * mte_pr_counts; summed over i the rows equal its output bit for bit (every
+ * row has one writer per call, so they are deterministic).  An empty crop
+ * leaves the rows untouched.  These are the per-image EvalResult counts of
+ * _pred_eval (eval_depth_edges.py:179-230) before pr_evaluation sums them. */
+int mte_pr_counts_per_image(const void *pred, int pred_dtype, const uint8_t *gt, int n_images, int H, int W,
+                            const int32_t *crop_host, const double *thresholds_host, int n_thresholds,
+                            double max_dist, int apply_thinning, int64_t *counts, void *workspace,
+                            size_t workspace_bytes, mte_stream_t stream);
 
 size_t mte_match_workspace_bytes(int n_problems, int h, int w, double max_dist);
 /* a,b: [P,h,w] u8 boundary maps.  match_a/match_b: out [P,h,w] u8 (1 = matched)

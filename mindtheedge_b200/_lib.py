@@ -59,6 +59,8 @@ _SIGNATURES = {
     "mte_pr_thin_workspace_bytes": (_sz, [_i, _i, _i, _i, _d]),
     "mte_pr_counts": (_i, [_vp, _i, _vp, _i, _i, _i, C.POINTER(C.c_int32), C.POINTER(C.c_double), _i, _d, _i,
                            _vp, _vp, _sz, _vp]),
+    "mte_pr_counts_per_image": (_i, [_vp, _i, _vp, _i, _i, _i, C.POINTER(C.c_int32), C.POINTER(C.c_double), _i, _d,
+                                     _i, _vp, _vp, _sz, _vp]),
     "mte_match_workspace_bytes": (_sz, [_i, _i, _i, _d]),
     "mte_correspond_pixels": (_i, [_vp, _vp, _i, _i, _i, _d, _vp, _vp, _vp, _vp, _sz, _vp]),
     "mte_thin_workspace_bytes": (_sz, [_i, _i, _i]),

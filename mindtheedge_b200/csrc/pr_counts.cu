@@ -52,6 +52,7 @@ struct MatchP {
     int nProblems;             // N*T
     const double *thr;         // [T] device (float modes)
     int noff;
+    int countsImgStride;       // rows per image in counts: 0 = summed over the images ([T][4]), T = per image ([N][T][4])
     const short2 *off;         // [noff] (dx, dy), nearest first
     const unsigned short *neg; // [noff] index of the negated offset
     unsigned long long *counts;  // [T][4] count_r,sum_r,count_p,sum_p (accumulated)   (pr mode)
@@ -335,7 +336,7 @@ __global__ void __launch_bounds__(kThreads) match_kernel(const __grid_constant__
         const int matched = sMatched;
         if (threadIdx.x == 0) {
             if (P.counts) {
-                unsigned long long *c = P.counts + (size_t)t * 4;
+                unsigned long long *c = P.counts + (size_t)(t + img * P.countsImgStride) * 4;
                 atomicAdd(c + 0, (unsigned long long)matched);
                 atomicAdd(c + 1, (unsigned long long)nQ);
                 atomicAdd(c + 2, (unsigned long long)matched);
@@ -650,7 +651,7 @@ __global__ void __launch_bounds__(kSmThreads, 1) match_smem_kernel(const __grid_
         const int matched = sMatched;
         if (threadIdx.x == 0) {
             if (P.counts) {
-                unsigned long long *c = P.counts + (size_t)t * 4;
+                unsigned long long *c = P.counts + (size_t)(t + img * P.countsImgStride) * 4;
                 atomicAdd(c + 0, (unsigned long long)matched);
                 atomicAdd(c + 1, (unsigned long long)nQ);
                 atomicAdd(c + 2, (unsigned long long)matched);
@@ -1339,7 +1340,8 @@ __global__ void __launch_bounds__(kSwThreads, 1) match_sweep_kernel(const __grid
             if (threadIdx.x == 0) {
                 const int t = levels ? s : T - 1 - s;
                 const int matched = sMatched;
-                unsigned long long *c = P.counts + (size_t)t * 4;
+                // per-image rows: the image this CTA is sweeping (thread 0 wrote sImage)
+                unsigned long long *c = P.counts + (size_t)(t + sImage * P.countsImgStride) * 4;
                 atomicAdd(c + 0, (unsigned long long)matched);
                 atomicAdd(c + 1, (unsigned long long)nQ);
                 atomicAdd(c + 2, (unsigned long long)matched);
@@ -1715,10 +1717,11 @@ static int pr_counts_thinned(MatchP &P, const Layout &L, char *ws, double max_di
     return MTE_OK;
 }
 
-extern "C" int mte_pr_counts(const void *pred, int pred_dtype, const uint8_t *gt, int N, int H, int W,
-                             const int32_t *crop, const double *thresholds, int T, double max_dist,
-                             int apply_thinning, int64_t *counts, void *workspace, size_t ws_bytes,
-                             mte_stream_t stream) {
+// perImage = 0: counts [T][4] summed over the images; 1: counts [N][T][4], one row per (image, threshold).  Every
+// matcher CTA knows its image, so the only difference is the row it adds its four counts to.
+static int pr_counts_impl(const void *pred, int pred_dtype, const uint8_t *gt, int N, int H, int W, const int32_t *crop,
+                          const double *thresholds, int T, double max_dist, int apply_thinning, int64_t *counts,
+                          int perImage, void *workspace, size_t ws_bytes, mte_stream_t stream) {
     if (!pred || !gt || !counts || !workspace) return MTE_ERR_NULL;
     if (N < 1 || H < 1 || W < 1) return MTE_ERR_SHAPE;
     if (T < 1 || T > MTE_MAX_THRESHOLDS) return MTE_ERR_ARG;
@@ -1736,9 +1739,26 @@ extern "C" int mte_pr_counts(const void *pred, int pred_dtype, const uint8_t *gt
     clip_crop(crop, H, W, P.x0, P.y0, P.w, P.h);
     P.nProblems = N * T;
     P.counts = reinterpret_cast<unsigned long long *>(counts);
+    P.countsImgStride = perImage ? T : 0;
     if (P.w == 0 || P.h == 0) return MTE_OK;  // empty window: nothing to count
     if (apply_thinning)
         return pr_counts_thinned(P, L, static_cast<char *>(workspace), max_dist, thresholds,
                                  reinterpret_cast<cudaStream_t>(stream));
     return launch(P, L, static_cast<char *>(workspace), max_dist, thresholds, reinterpret_cast<cudaStream_t>(stream));
+}
+
+extern "C" int mte_pr_counts(const void *pred, int pred_dtype, const uint8_t *gt, int N, int H, int W,
+                             const int32_t *crop, const double *thresholds, int T, double max_dist,
+                             int apply_thinning, int64_t *counts, void *workspace, size_t ws_bytes,
+                             mte_stream_t stream) {
+    return pr_counts_impl(pred, pred_dtype, gt, N, H, W, crop, thresholds, T, max_dist, apply_thinning, counts, 0,
+                          workspace, ws_bytes, stream);
+}
+
+extern "C" int mte_pr_counts_per_image(const void *pred, int pred_dtype, const uint8_t *gt, int N, int H, int W,
+                                       const int32_t *crop, const double *thresholds, int T, double max_dist,
+                                       int apply_thinning, int64_t *counts, void *workspace, size_t ws_bytes,
+                                       mte_stream_t stream) {
+    return pr_counts_impl(pred, pred_dtype, gt, N, H, W, crop, thresholds, T, max_dist, apply_thinning, counts, 1,
+                          workspace, ws_bytes, stream);
 }

@@ -36,7 +36,7 @@ from .edge import canny_from_depth, read_depth_file
 __all__ = [
     "EvalResult", "_pred_eval", "pr_counts", "correspond_pixels_batch", "evaluate_boundaries", "evaluate_boundaries_bin",
     "compute_rec_prec_f1", "pr_evaluation", "pr_evaluation_arrays", "mean_recall_at_precision_range",
-    "shard_indices", "all_reduce_counts", "sweep_counts",
+    "shard_indices", "all_reduce_counts", "sweep_counts", "evaluate_boundaries_batch",
 ]
 
 _DT = {torch.float32: _lib.MTE_F32, torch.float64: _lib.MTE_F64, torch.uint8: _lib.MTE_U8}
@@ -45,8 +45,9 @@ _DT = {torch.float32: _lib.MTE_F32, torch.float64: _lib.MTE_F64, torch.uint8: _l
 # ---------------------------------------------------------------------------
 # tensor-level ops
 # ---------------------------------------------------------------------------
-def _pr_counts_cuda(pred, gt, thresholds, n_levels, max_dist, crop, apply_thinning=False):
-    """CUDA implementation of ``mte::pr_counts`` -> int64 [T,4] (count_r, sum_r, count_p, sum_p)."""
+def _pr_counts_cuda(pred, gt, thresholds, n_levels, max_dist, crop, apply_thinning=False, per_image=False):
+    """CUDA implementation of ``mte::pr_counts`` -> int64 [T,4] (count_r, sum_r, count_p, sum_p), or with
+    ``per_image`` int64 [N,T,4]."""
     with runtime.on_device(pred, gt) as dev:
         pred, gt = pred.contiguous(), gt.contiguous()
         N, H, W = pred.shape
@@ -56,13 +57,13 @@ def _pr_counts_cuda(pred, gt, thresholds, n_levels, max_dist, crop, apply_thinni
             t = np.ascontiguousarray(np.asarray(thresholds, dtype=np.float64))
             T = int(t.shape[0])
             thr = t.ctypes.data_as(C.POINTER(C.c_double))
-        out = torch.zeros((T, 4), dtype=torch.int64, device=dev)
+        out = torch.zeros((N, T, 4) if per_image else (T, 4), dtype=torch.int64, device=dev)
         cr = None if len(crop) == 0 else (C.c_int32 * 4)(*[int(v) for v in crop])
         query = _lib.lib.mte_pr_thin_workspace_bytes if apply_thinning else _lib.lib.mte_pr_workspace_bytes
         ws = runtime.workspace(dev, query(N, H, W, T, float(max_dist)))
-        runtime.call("mte_pr_counts", dev, pred.data_ptr(), _DT[pred.dtype], gt.data_ptr(), N, H, W, cr, thr, T,
-                     float(max_dist), int(bool(apply_thinning)), out.data_ptr(), ws.data_ptr(), ws.numel(),
-                     runtime.current_stream_ptr(dev))
+        runtime.call("mte_pr_counts_per_image" if per_image else "mte_pr_counts", dev, pred.data_ptr(),
+                     _DT[pred.dtype], gt.data_ptr(), N, H, W, cr, thr, T, float(max_dist), int(bool(apply_thinning)),
+                     out.data_ptr(), ws.data_ptr(), ws.numel(), runtime.current_stream_ptr(dev))
     return out
 
 
@@ -81,14 +82,14 @@ def _correspond_pixels_cuda(a, b, max_dist, want_maps):
 
 
 runtime.define_op("pr_counts(Tensor pred, Tensor gt, float[] thresholds, int n_levels, float max_dist, int[] crop, "
-                  "bool apply_thinning=False) -> Tensor", _pr_counts_cuda)
+                  "bool apply_thinning=False, bool per_image=False) -> Tensor", _pr_counts_cuda)
 runtime.define_op("correspond_pixels(Tensor a, Tensor b, float max_dist, bool want_maps) -> (Tensor, Tensor, Tensor)",
                   _correspond_pixels_cuda)
 
 
 def pr_counts(pred: torch.Tensor, gt: torch.Tensor, thresholds=None, *, n_levels: Optional[int] = None,
               max_dist: float = 0.0075, crop: Optional[Sequence[int]] = None,
-              out: Optional[torch.Tensor] = None, apply_thinning: bool = False) -> torch.Tensor:
+              out: Optional[torch.Tensor] = None, apply_thinning: bool = False, per_image: bool = False) -> torch.Tensor:
     """Counts for a batch of images, one GT map each (torch custom op ``mte::pr_counts``).
 
     pred  [N,H,W] CUDA: float32/float64 strength map (``pred >= thresholds[t]``) or uint8 level
@@ -99,8 +100,10 @@ def pr_counts(pred: torch.Tensor, gt: torch.Tensor, thresholds=None, *, n_levels
     apply_thinning  thin every binarised window before matching (``evaluate_boundaries``' default): the crop is
           applied first, so thinning zero-pads at the crop border; ``sum_p`` counts the thinned pixels.  Thresholds
           may then come in any order and repeat.
+    per_image  return the counts of every image instead of their sum: int64 [N,T,4], row (i, t) for image i and
+          threshold t, from the same single launch chain; summed over i it equals the default result.
     ->    int64 [T,4] on the device, columns count_r, sum_r, count_p, sum_p, summed over the
-          batch and ACCUMULATED into ``out`` when given."""
+          batch (``per_image``: [N,T,4]) and ACCUMULATED into ``out`` when given."""
     runtime.require_cuda(pred, "pred")
     runtime.require_cuda(gt, "gt")
     if pred.dim() == 2:
@@ -118,7 +121,8 @@ def pr_counts(pred: torch.Tensor, gt: torch.Tensor, thresholds=None, *, n_levels
     else:
         thr = [float(v) for v in np.asarray(thresholds, dtype=np.float64)]
     c = torch.ops.mte.pr_counts(pred, gt, thr, int(n_levels or 0), float(max_dist),
-                                [] if crop is None else [int(v) for v in crop], bool(apply_thinning))
+                                [] if crop is None else [int(v) for v in crop], bool(apply_thinning),
+                                bool(per_image))
     if out is None:
         return c
     out += c
@@ -197,6 +201,37 @@ def evaluate_boundaries_bin(predicted_boundaries_bin, gt_boundaries, max_dist=0.
     return c_r[0], s_r[0], c_p[0], s_p[0]
 
 
+def evaluate_boundaries_batch(preds, gts, thresholds=99, max_dist=0.0075, apply_thinning=True):
+    """``evaluate_boundaries`` for a list of 2-D predicted maps with one GT map each ->
+    ``[evaluate_boundaries(p, [g], thresholds, max_dist, apply_thinning) for p, g in zip(preds, gts)]``, element for
+    element.  Maps of one shape and dtype go to the device in one ``pr_counts(..., per_image=True)`` call; the cases
+    the single-GT device path does not take (thinning with more than ``MTE_MAX_THRESHOLDS`` thresholds) run image by
+    image."""
+    thr = _threshold_grid(thresholds)
+    T = thr.shape[0]
+    if apply_thinning and T > _lib.MTE_MAX_THRESHOLDS:
+        return [evaluate_boundaries(p, [g], thresholds, max_dist, apply_thinning) for p, g in zip(preds, gts)]
+    maps = []
+    for p in preds:
+        p = np.ascontiguousarray(p)
+        maps.append(p if p.dtype in (np.float32, np.float64) else p.astype(np.float64))
+    groups = {}
+    for i, p in enumerate(maps):
+        groups.setdefault((p.shape, p.dtype), []).append(i)
+    out = [None] * len(maps)
+    for idx in groups.values():
+        d_pred = torch.from_numpy(np.stack([maps[i] for i in idx])).cuda()
+        g_np = [np.asarray(gts[i]) for i in idx]
+        gt = torch.from_numpy(np.stack([(g != 0).astype(np.uint8) for g in g_np])).cuda()
+        c = pr_counts(d_pred, gt, thr, max_dist=max_dist, apply_thinning=bool(apply_thinning),
+                      per_image=True).cpu().numpy()
+        for k, i in enumerate(idx):
+            # sum_r is gt.sum() as in evaluate_boundaries (non-binary GT maps included)
+            out[i] = (c[k, :, 0].astype(np.float64), np.full(T, float(g_np[k].sum())), c[k, :, 2].astype(np.float64),
+                      c[k, :, 3].astype(np.float64), thr)
+    return out
+
+
 def compute_rec_prec_f1(count_r, sum_r, count_p, sum_p):
     """eval_depth_edges.py:147-161."""
     rec = count_r / (sum_r + (sum_r == 0))
@@ -253,8 +288,11 @@ def _pred_eval(pred_path, gt_path, crop):
         return im
 
     pred, gt_b = load(pred_path), load(gt_path)
-    count_r, sum_r, count_p, sum_p, used_thresholds = evaluate_boundaries(
-        pred, [gt_b], thresholds=1, apply_thinning=False, max_dist=0.002)
+    return _eval_result(*evaluate_boundaries(pred, [gt_b], thresholds=1, apply_thinning=False, max_dist=0.002))
+
+
+def _eval_result(count_r, sum_r, count_p, sum_p, used_thresholds):
+    """eval_depth_edges.py:212-230: the ``EvalResult`` of ``_pred_eval`` from its [T] count vectors."""
     rec, prec, f1 = compute_rec_prec_f1(count_r, sum_r, count_p, sum_p)
     best_ndx = np.argmax(f1)
     return EvalResult(count_r, sum_r, count_p, sum_p, count_r[best_ndx], sum_r[best_ndx], count_p[best_ndx],
@@ -309,16 +347,18 @@ def _side_streams(device, n):
     return _SIDE_STREAMS[key]
 
 
-def _sweep_chunk(depth, gt, pairs, gt_crop, min_depth, max_depth, max_dist):
+def _sweep_chunk(depth, gt, pairs, gt_crop, min_depth, max_depth, max_dist, per_image=False):
     levels = canny_from_depth(depth, pairs, min_depth, max_depth, want_edges=False, want_levels=True)
-    return pr_counts(levels, gt, n_levels=len(pairs), max_dist=max_dist, crop=gt_crop)
+    return pr_counts(levels, gt, n_levels=len(pairs), max_dist=max_dist, crop=gt_crop, per_image=per_image)
 
 
 def sweep_counts(depth: torch.Tensor, gt: torch.Tensor, edge_thresh_range, gt_crop, min_depth, max_depth,
-                 max_dist=0.002, out=None, pipeline_chunks: Optional[int] = None) -> torch.Tensor:
+                 max_dist=0.002, out=None, pipeline_chunks: Optional[int] = None,
+                 per_image: bool = False) -> torch.Tensor:
     """Device part of ``pr_evaluation`` for a batch: depth [N,H,W] (already at GT size), gt [N,H,W]
     uint8 -> int64[len(range),4].  Thresholds are swept strictest first internally (the level plane
-    needs nested pairs) and returned in the caller's order.
+    needs nested pairs) and returned in the caller's order.  ``per_image`` returns the counts of every image,
+    int64[N,len(range),4] (``_pred_eval``'s counts of image i at every setting in row i), from the same launches.
 
     ``pipeline_chunks`` > 1 cuts the batch into chunks on side streams (a chunk's NMS + hysteresis next to another
     chunk's matcher; counts are integer sums, the result does not depend on the chunking).  Measured on the bench set:
@@ -329,7 +369,7 @@ def sweep_counts(depth: torch.Tensor, gt: torch.Tensor, edge_thresh_range, gt_cr
     N = depth.shape[0] if depth.dim() == 3 else 1
     chunks = pipeline_chunks if pipeline_chunks is not None else 1
     if chunks <= 1 or depth.dim() != 3:
-        c = _sweep_chunk(depth, gt, pairs, gt_crop, min_depth, max_depth, max_dist)
+        c = _sweep_chunk(depth, gt, pairs, gt_crop, min_depth, max_depth, max_dist, per_image)
     else:
         main = torch.cuda.current_stream(depth.device)
         bounds = [round(k * N / chunks) for k in range(chunks + 1)]
@@ -338,14 +378,18 @@ def sweep_counts(depth: torch.Tensor, gt: torch.Tensor, edge_thresh_range, gt_cr
             st.wait_stream(main)
             with torch.cuda.stream(st):
                 parts.append(_sweep_chunk(depth[bounds[k]:bounds[k + 1]], gt[bounds[k]:bounds[k + 1]], pairs, gt_crop,
-                                          min_depth, max_depth, max_dist))
+                                          min_depth, max_depth, max_dist, per_image))
         for p, st in zip(parts, _side_streams(depth.device, chunks)):
             main.wait_stream(st)
             p.record_stream(main)
-        c = parts[0]
-        for p in parts[1:]:
-            c = c + p
-    c = c[_reorder_index(tuple(int(v) for v in np.argsort(order)), c.device)]
+        if per_image:   # every chunk's rows at its images' offsets
+            c = torch.cat(parts)
+        else:
+            c = parts[0]
+            for p in parts[1:]:
+                c = c + p
+    idx = _reorder_index(tuple(int(v) for v in np.argsort(order)), c.device)
+    c = c[:, idx] if per_image else c[idx]
     if out is not None:
         out += c
         return out
@@ -354,22 +398,29 @@ def sweep_counts(depth: torch.Tensor, gt: torch.Tensor, edge_thresh_range, gt_cr
 
 def pr_evaluation_arrays(depths: Sequence[np.ndarray], gts: Sequence[np.ndarray], edge_thresh_range=None,
                          gt_crop=(44, 1197, 153, 371), min_depth=0.0, max_depth=80.0, batch: int = 32,
-                         mask: Optional[np.ndarray] = None):
+                         mask: Optional[np.ndarray] = None, per_image: bool = False):
     """Array-level ``pr_evaluation``: predicted depth maps (any size; resized to the GT size on the
     host with cv2.INTER_LINEAR as edge.py:76-78 does) and GT edge images (uint8, >127 = edge).
     Images are sharded over ``torch.distributed`` ranks when initialised.  ``mask`` is the mask-image branch of
     ``_pred_eval`` (eval_depth_edges.py:182-186, 198-200, 209-210): a float plane in [0,1] that multiplies both maps
     instead of the crop.
     -> (precision_vec, recall_vec, counts int64[T,4]; with a mask the sum_r column is returned separately as float64,
-    see ``_masked_evaluation``)"""
+    see ``_masked_evaluation``).
+    ``per_image`` appends the counts of every image, in list order: (..., rows int64[N,T,4], sum_r float64[N]).
+    ``sum_r[i]`` is image i's ``sum_r`` as ``_pred_eval`` computes it: the GT pixels in the crop (``rows[i, :, 1]``),
+    with a mask the fractional ``(gt * mask).sum()``.  Under ``torch.distributed`` every rank fills its own rows of
+    zero arrays and ONE integer all-reduce sums them (exact: the result does not depend on the number of ranks);
+    ``counts`` is then the sum of the rows."""
     import cv2
     if edge_thresh_range is None:
         edge_thresh_range = list(range(20, 241, 20))
     if mask is not None:
-        return _masked_evaluation(depths, gts, edge_thresh_range, np.asarray(mask), min_depth, max_depth, batch)
+        return _masked_evaluation(depths, gts, edge_thresh_range, np.asarray(mask), min_depth, max_depth, batch,
+                                  per_image)
     rank, world = _dist_info()
     dev = torch.device("cuda", torch.cuda.current_device())
     counts = torch.zeros((len(edge_thresh_range), 4), dtype=torch.int64, device=dev)
+    rows = torch.zeros((len(depths), len(edge_thresh_range), 4), dtype=torch.int64, device=dev) if per_image else None
     mine = shard_indices(len(depths), rank, world)
     # group by GT shape and depth dtype so every launch is a dense batch; the quantisation runs in the
     # array's own float type (edge.py:85-87), so float32 and float64 maps must not be mixed
@@ -390,19 +441,31 @@ def pr_evaluation_arrays(depths: Sequence[np.ndarray], gts: Sequence[np.ndarray]
             # _pred_eval: value/255 > 0.5 -> edge (eval_depth_edges.py:202-205)
             g_dev = torch.from_numpy(np.stack([(np.asarray(gts[i]) > 127).astype(np.uint8) for i in chunk])).to(
                 dev, non_blocking=True)
-            sweep_counts(d_dev, g_dev, edge_thresh_range, gt_crop, min_depth, max_depth, out=counts)
-    all_reduce_counts(counts)
+            if per_image:
+                rows[torch.tensor(chunk, device=dev)] = sweep_counts(d_dev, g_dev, edge_thresh_range, gt_crop,
+                                                                     min_depth, max_depth, per_image=True)
+            else:
+                sweep_counts(d_dev, g_dev, edge_thresh_range, gt_crop, min_depth, max_depth, out=counts)
+    if per_image:
+        all_reduce_counts(rows)
+        counts = rows.sum(0)
+    else:
+        all_reduce_counts(counts)
     c = counts.cpu().numpy().astype(np.float64)
     rec, prec, _ = compute_rec_prec_f1(c[:, 0], c[:, 1], c[:, 2], c[:, 3])
+    if per_image:
+        sum_r = rows[:, 0, 1].cpu().numpy().astype(np.float64)
+        return [float(p) for p in prec], [float(r) for r in rec], counts, rows, sum_r
     return [float(p) for p in prec], [float(r) for r in rec], counts
 
 
-def _masked_evaluation(depths, gts, edge_thresh_range, mask, min_depth, max_depth, batch):
+def _masked_evaluation(depths, gts, edge_thresh_range, mask, min_depth, max_depth, batch, per_image=False):
     """``pr_evaluation`` with a mask image instead of a crop.  Per image and Canny setting the reference evaluates
     ``pred * mask`` (binarised again at ``>= 0.5`` by ``thresholds=1``) against ``gt * mask`` (boundary where non-zero)
     on the FULL plane, so: predicted pixel kept iff ``mask >= 0.5``, GT pixel kept iff ``mask != 0``, the matching
     radius is that of the uncropped plane, and ``sum_r`` is the fractional ``(gt * mask).sum()`` (float64, summed per
-    image, then over images in list order -- eval_depth_edges.py:138, 299)."""
+    image, then over images in list order -- eval_depth_edges.py:138, 299).  ``per_image`` as in
+    ``pr_evaluation_arrays``, ``sum_r[i]`` being image i's ``(gt * mask).sum()``."""
     import cv2
     rank, world = _dist_info()
     dev = torch.device("cuda", torch.cuda.current_device())
@@ -414,6 +477,8 @@ def _masked_evaluation(depths, gts, edge_thresh_range, mask, min_depth, max_dept
     pairs = [(int(edge_thresh_range[i] / 2), int(edge_thresh_range[i])) for i in order]
     mine = shard_indices(len(depths), rank, world)
     sum_r = 0.0
+    rows = torch.zeros((len(depths), T, 4), dtype=torch.int64, device=dev) if per_image else None
+    sum_r_img = torch.zeros(len(depths), dtype=torch.float64, device=dev) if per_image else None
     H, W = mask.shape
     for s0 in range(0, len(mine), batch):
         chunk = mine[s0:s0 + batch]
@@ -426,15 +491,28 @@ def _masked_evaluation(depths, gts, edge_thresh_range, mask, min_depth, max_dept
         if len({d.dtype for d in dep}) > 1:
             dep = [d.astype(np.float64) for d in dep]
         gb = [(np.asarray(gts[i]) > 127) for i in chunk]
-        for g in gb:
-            sum_r = sum_r + (g.astype(np.float64) * mask).sum()
+        for i, g in zip(chunk, gb):
+            s_i = (g.astype(np.float64) * mask).sum()
+            sum_r = sum_r + s_i
+            if per_image:
+                sum_r_img[i] = s_i
         d_dev = torch.from_numpy(np.stack(dep)).to(dev)
         g_dev = torch.from_numpy(np.stack(gb)).to(dev)
         levels = canny_from_depth(d_dev, pairs, min_depth, max_depth, want_edges=False, want_levels=True)
         levels = torch.where(keep_p[None], levels, torch.full_like(levels, 255))
-        c = pr_counts(levels, (g_dev & keep_g[None]).to(torch.uint8), n_levels=T, max_dist=0.002, crop=None)
-        counts += c[_reorder_index(tuple(int(v) for v in np.argsort(order)), c.device)]
-    all_reduce_counts(counts)
+        c = pr_counts(levels, (g_dev & keep_g[None]).to(torch.uint8), n_levels=T, max_dist=0.002, crop=None,
+                      per_image=per_image)
+        idx = _reorder_index(tuple(int(v) for v in np.argsort(order)), c.device)
+        if per_image:
+            rows[torch.tensor(chunk, device=dev)] = c[:, idx]
+        else:
+            counts += c[idx]
+    if per_image:
+        all_reduce_counts(rows)
+        counts = rows.sum(0)
+        all_reduce_counts(sum_r_img)   # one writer per entry, all others add 0.0: exact
+    else:
+        all_reduce_counts(counts)
     if world > 1:
         import torch.distributed as dist
         t = torch.tensor([sum_r], dtype=torch.float64, device=dev)
@@ -442,14 +520,19 @@ def _masked_evaluation(depths, gts, edge_thresh_range, mask, min_depth, max_dept
         sum_r = float(t.item())
     c = counts.cpu().numpy().astype(np.float64)
     rec, prec, _ = compute_rec_prec_f1(c[:, 0], np.full(T, sum_r), c[:, 2], c[:, 3])
+    if per_image:
+        return [float(p) for p in prec], [float(r) for r in rec], counts, rows, sum_r_img.cpu().numpy()
     return [float(p) for p in prec], [float(r) for r in rec], counts
 
 
 def pr_evaluation(edge_list, pred_list, edge_thresh_range=None, gt_crop=[44, 1197, 153, 371], min_depth=0.0,
-                  max_depth=80.0, save_folder="temp_output", num_workers=4):
+                  max_depth=80.0, save_folder="temp_output", num_workers=4, per_image=False):
     """Drop-in for eval_depth_edges.py:232-348 -> (precision_vec, recall_vec).
     ``save_folder`` and ``num_workers`` are accepted for signature compatibility; nothing is
-    written to disk and no process pool is forked."""
+    written to disk and no process pool is forked.
+    ``per_image=True`` -> (precision_vec, recall_vec, results): ``results[i][k]`` is the ``EvalResult`` that
+    ``_pred_eval`` gives for image i at Canny setting k (eval_depth_edges.py:296, before the sum at :298-301), from
+    the same batched device calls."""
     import cv2
     depth_pred_list, edge_gt_list = list(pred_list), list(edge_list)
     if len(edge_gt_list) > len(depth_pred_list):  # multiscale GT list: keep the first entry of each group (:255-258)
@@ -460,5 +543,13 @@ def pr_evaluation(edge_list, pred_list, edge_thresh_range=None, gt_crop=[44, 119
     # gt_crop is handed to _pred_eval as str(gt_crop) (:291-294): a path to an existing mask image selects the
     # mask branch
     crop, mask = _crop_or_mask(gt_crop if isinstance(gt_crop, str) else list(gt_crop))
-    prec, rec, _ = pr_evaluation_arrays(depths, gts, edge_thresh_range, crop, min_depth, max_depth, mask=mask)
-    return prec, rec
+    if not per_image:
+        prec, rec, _ = pr_evaluation_arrays(depths, gts, edge_thresh_range, crop, min_depth, max_depth, mask=mask)
+        return prec, rec
+    prec, rec, _, rows, sum_r = pr_evaluation_arrays(depths, gts, edge_thresh_range, crop, min_depth, max_depth,
+                                                     mask=mask, per_image=True)
+    rows = rows.cpu().numpy().astype(np.float64)
+    # _pred_eval evaluates one binarised edge image (thresholds=1): [1]-vectors, used threshold 0.5
+    results = [[_eval_result(r[0:1], np.array([s]), r[2:3], r[3:4], _threshold_grid(1)) for r in img_rows]
+               for img_rows, s in zip(rows, sum_r)]
+    return prec, rec, results
