@@ -193,8 +193,13 @@ size_t mte_pr_thin_workspace_bytes(int n_images, int H, int W, int n_thresholds,
 /* pred: [N,H,W] of pred_dtype:
  *   MTE_F32/MTE_F64 strength map, thresholded as pred >= thresholds[t] (in fp64)
  *   MTE_U8          level plane from mte_canny_from_depth: edge at t iff level <= t
- * gt: [N,H,W] u8, non-zero = boundary.  crop = {x0,x1,y0,y1} (python slices
- * [y0:y1, x0:x1], clipped) or NULL.  counts: device int64[T,4] in the order
+ * gt: [N,H,W] u8, non-zero = boundary.  crop = {x0,x1,y0,y1} or NULL: the
+ * window [y0:y1, x0:x1] with python slice semantics, as the reference crops:
+ * a negative bound counts from the end of its axis (b + dim), bounds are then
+ * clamped to [0, dim], and x1 <= x0 or y1 <= y0 is an empty window.
+ * max_dist: matching radius max_dist * sqrt(h^2 + w^2) px of the h x w window
+ * (as correspond_pixels); a radius of 32 px or more is MTE_ERR_ARG.
+ * counts: device int64[T,4] in the order
  * count_r,sum_r,count_p,sum_p, ACCUMULATED into (zero it first).
  * apply_thinning: 0 = match the binarised window as it is; 1 = thin it first
  * (evaluate_boundaries' default, eval_depth_edges.py:125): the window is cut
@@ -222,7 +227,8 @@ int mte_pr_counts_per_image(const void *pred, int pred_dtype, const uint8_t *gt,
 
 size_t mte_match_workspace_bytes(int n_problems, int h, int w, double max_dist);
 /* a,b: [P,h,w] u8 boundary maps.  match_a/match_b: out [P,h,w] u8 (1 = matched)
- * or NULL.  count: device int64[P]. */
+ * or NULL.  count: device int64[P].  max_dist as in mte_pr_counts (radius
+ * max_dist * sqrt(h^2 + w^2) px; 32 px or more is MTE_ERR_ARG). */
 int mte_correspond_pixels(const uint8_t *a, const uint8_t *b, int n_problems, int h, int w, double max_dist,
                           uint8_t *match_a, uint8_t *match_b, int64_t *count, void *workspace,
                           size_t workspace_bytes, mte_stream_t stream);

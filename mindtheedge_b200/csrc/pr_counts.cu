@@ -1509,14 +1509,20 @@ static Layout layout(int nProblems, int h, int w, int T) {
     return L;
 }
 
+// one bound of a python slice over dim entries: a negative bound counts from the end, then [0, dim] clamps
+static int slice_bound(int b, int dim) {
+    if (b < 0) b += dim;
+    return b < 0 ? 0 : (b > dim ? dim : b);
+}
+
 static void clip_crop(const int32_t *crop, int H, int W, int &x0, int &y0, int &w, int &h) {
     int cx0 = 0, cx1 = W, cy0 = 0, cy1 = H;
     if (crop) {
-        // python slice semantics of pred[c2:c3, c0:c1] for non-negative bounds
-        cx0 = crop[0] < 0 ? 0 : (crop[0] > W ? W : crop[0]);
-        cx1 = crop[1] < 0 ? 0 : (crop[1] > W ? W : crop[1]);
-        cy0 = crop[2] < 0 ? 0 : (crop[2] > H ? H : crop[2]);
-        cy1 = crop[3] < 0 ? 0 : (crop[3] > H ? H : crop[3]);
+        // python slice semantics of pred[c2:c3, c0:c1], as the reference crops (negative bounds included)
+        cx0 = slice_bound(crop[0], W);
+        cx1 = slice_bound(crop[1], W);
+        cy0 = slice_bound(crop[2], H);
+        cy1 = slice_bound(crop[3], H);
     }
     x0 = cx0; y0 = cy0;
     w = cx1 > cx0 ? cx1 - cx0 : 0;
