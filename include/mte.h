@@ -139,7 +139,8 @@ int mte_edge_loss_alt_bwd(const float *grad_map, const float *edge, const float 
  * float32 (packnet_code/packnet_sfm/datasets/gta_dataset.py:413, 421).
  * mte_edge_resize_preserve: resize_depth_preserve (datasets/augmentations.py:58-100) of u8
  * edge maps [B,h,w] to [B,H,W] (last valid source pixel in raster order wins) followed by
- * the "/255 if max > 1" rule of resize_sample (:193-199) and the float32 cast. */
+ * the "/255 if max > 1" rule of resize_sample (:193-199), on the max of each resized
+ * map, and the float32 cast. */
 int mte_decode_normals(const uint8_t *normal_u8, float *theta_out, size_t n, mte_stream_t stream);
 size_t mte_edge_resize_workspace_bytes(int B);
 int mte_edge_resize_preserve(const uint8_t *edge_u8, int B, int h, int w, float *edge_out, int H, int W,
@@ -247,6 +248,9 @@ int mte_binary_thin(const uint8_t *in, uint8_t *out, int n_images, int H, int W,
  *      #pred px, #pred px with distance < thresh, 0}.
  * cond_out: optional int8 [N,H,W]: -1 = not a pred px, 1 = closer than thresh,
  *      0 = not (the third return value of the reference), or NULL.
+ * Limits: 1 <= H <= 65,533 (column distances are u16) and 1 <= W <= 24,576
+ *      (one row of them sits in shared memory); anything else is MTE_ERR_SHAPE.
+ * An image without any GT px measures from (-1, 0), as scipy's EDT does.
  * ------------------------------------------------------------------------ */
 size_t mte_chamfer_workspace_bytes(int n_images, int H, int W);
 int mte_chamfer_counts(const uint8_t *pred, const uint8_t *gt, int n_images, int H, int W, double thresh,

@@ -166,9 +166,16 @@ extern "C" int mte_chamfer_counts(const uint8_t *pred, const uint8_t *gt, int N,
     double *partial = reinterpret_cast<double *>(w + L.offPartial);
     cudaError_t e = cudaMemsetAsync(has, 0, (size_t)N * sizeof(int), st);
     if (e != cudaSuccess) return (int)e;
+    // a row of u16 distances plus the kernel's static reduction buffers passes the 48 KB a launch gets without the
+    // opt-in from W = 24,481 on; opting in below that is harmless
+    const size_t rowSmem = (size_t)W * sizeof(unsigned short);
+    if (rowSmem > 32 * 1024) {
+        e = opt_in_smem((const void *)row_eval_kernel, (int)rowSmem);
+        if (e != cudaSuccess) return (int)e;
+    }
     col_dist_kernel<<<ceil_div(N * W, kThreads), kThreads, 0, st>>>(gt, g, has, N, H, W);
     MTE_RETURN_IF_CUDA_ERROR();
-    row_eval_kernel<<<dim3((unsigned)H, (unsigned)N), kThreads, (size_t)W * sizeof(unsigned short), st>>>(
+    row_eval_kernel<<<dim3((unsigned)H, (unsigned)N), kThreads, rowSmem, st>>>(
         pred, g, has, H, W, thresh, partial, reinterpret_cast<signed char *>(cond_out));
     MTE_RETURN_IF_CUDA_ERROR();
     finish_kernel<<<N, 32, 0, st>>>(partial, H, out);

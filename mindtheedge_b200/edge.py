@@ -198,7 +198,8 @@ def compute_edge_metrics(depth: torch.Tensor, edge: torch.Tensor, gt_crop=None, 
 
     depth  CUDA [H,W] (or [1,1,H,W]): predicted DEPTH at the GT size (``inv2depth`` + resize already applied),
            or, with ``edge_model``, the predicted edge probability map (thresholds 0.5 / 0.75 / 0.9).
-    edge   CUDA [H,W] GT edge map in [0,1] (the reference multiplies by 255 and binarises at 0.5).
+    edge   CUDA [H,W] GT edge map in [0,1] (the reference multiplies by 255 and binarises at 0.5, here in the
+           map's own floating dtype, as NumPy would; other dtypes in float32).
     ->     the 9 numbers the reference appends: for each of the three settings, chamfer precision
            (pred px within < 5 px of a GT px), recall (the converse) and their harmonic mean."""
     d = depth.reshape(depth.shape[-2], depth.shape[-1])
@@ -215,7 +216,8 @@ def compute_edge_metrics(depth: torch.Tensor, edge: torch.Tensor, gt_crop=None, 
         lv = canny_from_depth(d, [(30, 60), (20, 40), (10, 20)], float("-inf"), mx, want_edges=False,
                               want_levels=True)
         preds = torch.stack([(lv <= t).to(torch.uint8) * 255 for t in (2, 1, 0)])
-    gt = ((g.float() * 255) / 255 > 0.5).to(torch.uint8) * 255
+    g = g if g.is_floating_point() else g.float()
+    gt = ((g * 255) / 255 > 0.5).to(torch.uint8) * 255
     if gt_crop is not None and len(gt_crop) > 0:
         c = gt_crop
         gt = gt[c[2]:c[3], c[0]:c[1]]

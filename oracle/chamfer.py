@@ -23,14 +23,21 @@ def chamfer_distance(im_pred, im_gt, edge_to_edge_thresh=5):
     return c_dist, percentage, close, int(n_pred)
 
 
-def compute_edge_metrics(depth, gt_edge01, gt_crop=None):
+def compute_edge_metrics(depth, gt_edge01, gt_crop=None, edge_model=False):
     """Restates ModelWrapper.compute_edge_metrics (packnet_code/packnet_sfm/models/model_wrapper.py:376-442) for
-    a depth-predicting model: depth [H,W] float32 already at the GT size, gt_edge01 [H,W] in [0,1]."""
-    import cv2
+    a depth-predicting model: depth [H,W] float32 already at the GT size, gt_edge01 [H,W] in [0,1].
+
+    edge_model: depth is the predicted edge probability map, binarised as ``depth > t`` for t = 0.5, 0.75, 0.9 in
+    its own dtype.  This branch follows the documented rule only; unlike the depth branch it is not pinned to a
+    golden of the reference."""
     gt_edge = np.asarray(gt_edge01) * 255
     depth = np.asarray(depth)
-    vis = (depth * (255.0 / np.max(depth))).astype(np.uint8)
-    ims = [cv2.Canny(vis, 10, 20), cv2.Canny(vis, 20, 40), cv2.Canny(vis, 30, 60)]
+    if edge_model:
+        ims = [(depth > t).astype(np.uint8) * 255 for t in (0.5, 0.75, 0.9)]
+    else:
+        import cv2
+        vis = (depth * (255.0 / np.max(depth))).astype(np.uint8)
+        ims = [cv2.Canny(vis, 10, 20), cv2.Canny(vis, 20, 40), cv2.Canny(vis, 30, 60)]
     if gt_crop is not None and len(gt_crop) > 0:
         c = gt_crop
         gt_edge = gt_edge[c[2]:c[3], c[0]:c[1]]

@@ -12,7 +12,9 @@ import numpy as np
 def resize_depth_preserve(depth, shape):
     """Every valid (> 0) source pixel is dropped onto (int(y * H/h), int(x * W/w)); when several land on the same
     output pixel the one that comes last in raster order stays (NumPy's repeated-index assignment)."""
-    d = np.squeeze(np.asarray(depth))
+    d = np.asarray(depth)
+    if d.ndim > 2:          # [h,w,1] as the reference holds it; a 2-D map keeps its 1-pixel axes
+        d = np.squeeze(d)
     h, w = d.shape
     ys, xs = np.nonzero(d > 0)  # raster order
     Y = (ys * (shape[0] / h)).astype(np.int32)
