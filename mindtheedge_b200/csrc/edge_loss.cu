@@ -7,7 +7,7 @@
 //   the per-scale loop          packnet_code/packnet_sfm/models/SemiSupEdgeModel.py:164-198
 //   inv2depth (optional fuse)   packnet_code/packnet_sfm/utils/depth.py:104-121
 // and the autograd backward of that chain (SURVEY.md A.1).  The hot kernels live in
-// edge_loss_kernels.cuh and are instantiated in edge_loss_{fwd,bwd}_v{4,1}.cu.
+// edge_loss_kernels.cuh and are instantiated in edge_loss_{fwd,bwd}_v{4,1}.cu and edge_loss_bwd_{ring,stash}.cu.
 #include <stdlib.h>
 #include <string.h>
 
@@ -112,14 +112,24 @@ __global__ void resize_bwd_kernel(const float *__restrict__ gout, float *__restr
     }
 }
 
+// grid-stride resize launches: one 256-thread CTA per 256 output pixels, at most 16 per SM of a B200
+static int resize_grid(size_t npx) { return (int)((npx + 255) / 256 < 148 * 16 ? (npx + 255) / 256 : 148 * 16); }
+
+// The prediction of one scale resized to the target resolution, into the workspace plane `out`.
+static const float *resize_pred(const mte_loss_scale_t &s, void *out, cudaStream_t st) {
+    float *o = static_cast<float *>(out);
+    resize_fwd_kernel<<<resize_grid((size_t)s.B * s.H * s.W), 256, 0, st>>>(s.pred, o, s.B, s.h, s.w, s.H, s.W);
+    return o;
+}
+
 // ---------------------------------------------------------------------------
 // Host side
 // ---------------------------------------------------------------------------
-constexpr int kFwdCtaWaves = 2, kBwdCtaWaves = 16;
+constexpr int kBwdCtaWaves = 16;
 
 struct Plan {
     LossP P;
-    bool vec, hasNormal, hasMask, isGrad;
+    bool vec, hasNormal, hasMask, isGrad, stash;
     size_t offAccum, accumBytes, offResize[MTE_MAX_SCALES], offResizeDx[MTE_MAX_SCALES], total;
     int fwdGrid;
     bool resized[MTE_MAX_SCALES];
@@ -140,7 +150,6 @@ static int validate(const mte_loss_scale_t *sc, int n) {
     return MTE_OK;
 }
 
-// Lay out CTAs / workspace.  bwd == true uses the overlapped 30-lane strips.
 static bool can_use_stash(const mte_loss_scale_t *sc, int n, const mte_loss_attrs_t *at) {
     if (!at || !at->is_grad || debug_knob("MTE_LOSS_NO_STASH")) return false;
     for (int i = 0; i < n; i++) {
@@ -150,6 +159,8 @@ static bool can_use_stash(const mte_loss_scale_t *sc, int n, const mte_loss_attr
     return true;
 }
 
+// What every launch of one direction needs: VEC, the per-scale strips and units, the persistent grid of the unit
+// kernels and the workspace layout.  The work items of the other backward kernels are planned by plan_items.
 static int make_plan(Plan &pl, const mte_loss_scale_t *sc, int n, const mte_loss_attrs_t *at, bool bwd) {
     int rc = validate(sc, n);
     if (rc) return rc;
@@ -170,10 +181,9 @@ static int make_plan(Plan &pl, const mte_loss_scale_t *sc, int n, const mte_loss
         if (!rs && (!aligned16(sc[i].pred) || (bwd && !aligned16(sc[i].grad_pred)))) pl.vec = false;
     }
     const int VEC = pl.vec ? 4 : 1;
-    const int RH = bwd ? kBwdRH : kFwdRH;
-    const bool stashBwd = bwd && can_use_stash(sc, n, at);
-    const int lanesOut = !pl.isGrad ? 32 : ((bwd && !stashBwd) ? bwd_lanes(VEC) : kHaloLanes);
-    int cta = 0, img = 0;
+    pl.stash = bwd && can_use_stash(sc, n, at);
+    const int lanesOut = !pl.isGrad ? 32 : ((bwd && !pl.stash) ? bwd_lanes(VEC) : kHaloLanes);
+    int img = 0;
     long long unitBase = 0;
     for (int i = 0; i < n; i++) {
         ScaleP &S = P.s[i];
@@ -182,36 +192,14 @@ static int make_plan(Plan &pl, const mte_loss_scale_t *sc, int n, const mte_loss
         S.stash = sc[i].stash;
         S.x = sc[i].pred;
         S.strips = ceil_div(S.W, lanesOut * VEC);
-        S.rowBlocks = ceil_div(S.H, RH);
-        S.items = S.strips * S.rowBlocks;
-        S.ctasPerImage = ceil_div(S.items, kWarps);  // capped below: warps loop over several items
-        S.ctaBase = cta; S.imgBase = img;
+        S.imgBase = img;
         S.unitBase = (int)unitBase;
         unitBase += (long long)S.strips * (S.H + (bwd ? kSegCostB : kSegCost)) * S.B;
         S.scaleWeight = sc[i].scale_weight;
-        cta += S.ctasPerImage * S.B;
         img += S.B;
         pl.resized[i] = sc[i].h != sc[i].H || sc[i].w != sc[i].W;
     }
-    // Cap the grid near kCtaWaves resident waves so the per-CTA epilogue (partials, ticket) is amortised over
-    // several items per warp; every scale keeps at least one CTA per image.
-    // measured on B200 (profiles/r01_notes.md): the forward (per-CTA reduction epilogue) likes ~2 resident waves,
-    // the backward (no epilogue) only needs enough CTAs for the hardware scheduler to balance the tail
-    int waves = bwd ? kBwdCtaWaves : kFwdCtaWaves;
-    if (const char *e = debug_knob("MTE_CTA_WAVES")) waves = atoi(e) > 0 ? atoi(e) : waves;  // tuning knob
-    const int cap = num_sms() * 2 * waves;
-    if (cta > cap) {
-        const double shrink = (double)cap / (double)cta;
-        cta = 0;
-        for (int i = 0; i < n; i++) {
-            ScaleP &S = P.s[i];
-            int c = (int)(S.ctasPerImage * shrink);
-            S.ctasPerImage = c < 1 ? 1 : c;
-            S.ctaBase = cta;
-            cta += S.ctasPerImage * S.B;
-        }
-    }
-    P.nScales = n; P.totalCtas = cta; P.totalImages = img;
+    P.nScales = n; P.totalImages = img;
     if (unitBase > 0x7fffffffLL) return MTE_ERR_SHAPE;
     P.totalUnits = (int)unitBase;
     // forward: persistent CTAs (2 per SM), every warp owns an equal contiguous range of strip rows (at least a few
@@ -238,6 +226,38 @@ static int make_plan(Plan &pl, const mte_loss_scale_t *sc, int n, const mte_loss
     }
     pl.total = off;
     return MTE_OK;
+}
+
+// Work items and grid of edge_loss_bwd_kernel / edge_loss_bwd_stash_kernel: an item is kBwdRH rows of one strip of
+// one image, each image of a scale gets ctasPerImage CTAs whose warps loop over its items.
+static void plan_items(LossP &P) {
+    int cta = 0;
+    for (int i = 0; i < P.nScales; i++) {
+        ScaleP &S = P.s[i];
+        S.rowBlocks = ceil_div(S.H, kBwdRH);
+        S.items = S.strips * S.rowBlocks;
+        S.ctasPerImage = ceil_div(S.items, kWarps);  // capped below: warps loop over several items
+        S.ctaBase = cta;
+        cta += S.ctasPerImage * S.B;
+    }
+    // Cap the grid near kBwdCtaWaves resident waves (every scale keeps at least one CTA per image).  Measured on B200
+    // (profiles/r01_notes.md): these kernels have no per-CTA epilogue and only need enough CTAs for the hardware
+    // scheduler to balance the tail.
+    int waves = kBwdCtaWaves;
+    if (const char *e = debug_knob("MTE_CTA_WAVES")) waves = atoi(e) > 0 ? atoi(e) : waves;  // tuning knob
+    const int cap = num_sms() * 2 * waves;
+    if (cta > cap) {
+        const double shrink = (double)cap / (double)cta;
+        cta = 0;
+        for (int i = 0; i < P.nScales; i++) {
+            ScaleP &S = P.s[i];
+            int c = (int)(S.ctasPerImage * shrink);
+            S.ctasPerImage = c < 1 ? 1 : c;
+            S.ctaBase = cta;
+            cta += S.ctasPerImage * S.B;
+        }
+    }
+    P.totalCtas = cta;
 }
 
 }  // namespace loss
@@ -276,15 +296,8 @@ extern "C" int mte_edge_loss_fwd(const mte_loss_scale_t *sc, int n, const mte_lo
     P.totalCtas = pl.fwdGrid;
     P.lossOut = loss_out;
     P.ctx = static_cast<float *>(ctx);
-    for (int i = 0; i < n; i++) {
-        if (pl.resized[i]) {
-            float *tmp = reinterpret_cast<float *>(w + pl.offResize[i]);
-            const size_t npx = (size_t)sc[i].B * sc[i].H * sc[i].W;
-            const int grid = (int)((npx + 255) / 256 < 148 * 16 ? (npx + 255) / 256 : 148 * 16);
-            resize_fwd_kernel<<<grid, 256, 0, st>>>(sc[i].pred, tmp, sc[i].B, sc[i].h, sc[i].w, sc[i].H, sc[i].W);
-            P.s[i].x = tmp;
-        }
-    }
+    for (int i = 0; i < n; i++)
+        if (pl.resized[i]) P.s[i].x = resize_pred(sc[i], w + pl.offResize[i], st);
     const int mode = !at->is_grad ? MODE_NONE : (pl.hasNormal ? MODE_DIR : MODE_MAG);
     // a resized prediction is already a depth map in the workspace only if inv2depth is applied after the
     // resize, as the reference does not: inv2depth precedes the head (SemiSupEdgeModel.py:166,187)
@@ -311,16 +324,9 @@ extern "C" int mte_edge_loss_bwd(const mte_loss_scale_t *sc, int n, const mte_lo
     LossP &P = pl.P;
     P.ctx = const_cast<float *>(static_cast<const float *>(ctx));
     P.gradLoss = grad_loss;
-    for (int i = 0; i < n; i++) {
-        if (pl.resized[i]) {
-            // recompute the resized prediction (the workspace is not carried from the forward)
-            float *tmp = reinterpret_cast<float *>(w + pl.offResize[i]);
-            const size_t npx = (size_t)sc[i].B * sc[i].H * sc[i].W;
-            const int grid = (int)((npx + 255) / 256 < 148 * 16 ? (npx + 255) / 256 : 148 * 16);
-            resize_fwd_kernel<<<grid, 256, 0, st>>>(sc[i].pred, tmp, sc[i].B, sc[i].h, sc[i].w, sc[i].H, sc[i].W);
-            P.s[i].x = tmp;
-        }
-    }
+    // recompute the resized prediction (the workspace is not carried from the forward)
+    for (int i = 0; i < n; i++)
+        if (pl.resized[i]) P.s[i].x = resize_pred(sc[i], w + pl.offResize[i], st);
     // resized scales: the gradient is produced at target resolution, then pulled back by the resize adjoint
     for (int i = 0; i < n; i++)
         if (pl.resized[i]) P.s[i].dx = reinterpret_cast<float *>(w + pl.offResizeDx[i]);
@@ -333,22 +339,21 @@ extern "C" int mte_edge_loss_bwd(const mte_loss_scale_t *sc, int n, const mte_lo
             edge_loss_bwd_pointwise_kernel<false><<<num_sms() * 8, kThreads, 0, st>>>(P, at->is_sigmoid, at->pred_is_inverse);
     } else {
         const int mode = pl.hasNormal ? MODE_DIR : MODE_MAG;
-        if (can_use_stash(sc, n, at)) {
-            if (pl.vec && !debug_knob("MTE_LOSS_BWD_OLD")) {
-                P.totalCtas = pl.fwdGrid;  // persistent grid over the cost-balanced unit ranges
-                launch_bwd_ring_v4(P, pl.hasMask, at->pred_is_inverse != 0, at->is_sigmoid != 0, st);
-            } else if (pl.vec) launch_bwd_stash_v4(P, pl.hasMask, at->pred_is_inverse != 0, at->is_sigmoid != 0, st);
-            else launch_bwd_stash_v1(P, pl.hasMask, at->pred_is_inverse != 0, at->is_sigmoid != 0, st);
-        } else if (pl.vec) launch_bwd_v4(P, mode, pl.hasMask, at->pred_is_inverse != 0, at->is_sigmoid != 0, st);
-        else launch_bwd_v1(P, mode, pl.hasMask, at->pred_is_inverse != 0, at->is_sigmoid != 0, st);
+        if (pl.stash && pl.vec) {
+            P.totalCtas = pl.fwdGrid;  // persistent grid over the cost-balanced unit ranges
+            launch_bwd_ring(P, pl.hasMask, at->pred_is_inverse != 0, at->is_sigmoid != 0, st);
+        } else {
+            plan_items(P);
+            if (pl.stash) launch_bwd_stash(P, pl.hasMask, at->pred_is_inverse != 0, at->is_sigmoid != 0, st);
+            else if (pl.vec) launch_bwd_v4(P, mode, pl.hasMask, at->pred_is_inverse != 0, at->is_sigmoid != 0, st);
+            else launch_bwd_v1(P, mode, pl.hasMask, at->pred_is_inverse != 0, at->is_sigmoid != 0, st);
+        }
     }
     MTE_RETURN_IF_CUDA_ERROR();
     for (int i = 0; i < n; i++) {
         if (pl.resized[i]) {
-            const size_t npx = (size_t)sc[i].B * sc[i].h * sc[i].w;
-            const int grid = (int)((npx + 255) / 256 < 148 * 16 ? (npx + 255) / 256 : 148 * 16);
-            resize_bwd_kernel<<<grid, 256, 0, st>>>(P.s[i].dx, sc[i].grad_pred, sc[i].B, sc[i].h, sc[i].w, sc[i].H,
-                                                   sc[i].W);
+            resize_bwd_kernel<<<resize_grid((size_t)sc[i].B * sc[i].h * sc[i].w), 256, 0, st>>>(
+                P.s[i].dx, sc[i].grad_pred, sc[i].B, sc[i].h, sc[i].w, sc[i].H, sc[i].W);
         }
     }
     MTE_RETURN_IF_CUDA_ERROR();

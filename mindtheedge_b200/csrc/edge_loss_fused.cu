@@ -403,14 +403,7 @@ __global__ void __maxnreg__(MTE_FUSED_REGS) edge_loss_fused_kernel(const __grid_
     __shared__ double sLoss[MTE_MAX_SCALES];
     __shared__ int sLast;
     const LossP &P = F.L;
-    if (threadIdx.x < 16) {
-        const int di = threadIdx.x & 3, sgn_ = threadIdx.x >> 2;
-        const float sgn = sgn_ == 1 ? 1.f : (sgn_ == 2 ? -1.f : 0.f);
-        const float a = (di == 2 || di == 3) ? 1.f : (di == 1 ? -1.f : 0.f);  // h:0 rl:-1 v:1 lr:1
-        const float c = (di == 2) ? 0.f : 1.f;                                // h:1 rl:1 v:0 lr:1
-        const float bb = (di & 1) ? 1.f : 2.f;                                // axis stencils weigh the centre twice
-        sLut[threadIdx.x] = make_float4(sgn * a, sgn * c, sgn * a * bb, sgn * c * bb);
-    }
+    if (threadIdx.x < 16) sLut[threadIdx.x] = adjoint_entry(threadIdx.x);
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int nWarps = gridDim.x * kRWarps;
     const int gw = blockIdx.x * kRWarps + warp;

@@ -3,15 +3,20 @@
 // Design (HBM-bound stencil + reduction, no tensor cores):
 //  * one launch covers every image of up to 4 pyramid scales;
 //  * a warp owns a strip of 32 lanes x VEC px (VEC=4: 128-bit coalesced loads); the strips of the
-//    stencil kernels overlap by one lane on each side, so horizontal neighbours always come from a
-//    warp shuffle and vertical ones from registers -- no shared memory, no divergent edge loads,
-//    straight-line code so every load of a work item is in flight before the first use;
-//  * forward: 3x3 directional responses -> pick by quantised normal -> sigmoid -> soft-label BCE
-//    terms; per-thread fp32 partials -> warp shuffle -> one fp64 partial row per CTA -> the last CTA
-//    (atomic ticket) folds all partials in a fixed order, computes the per-image class balance alpha
-//    and writes the loss: single launch, no host sync, bit-reproducible run to run;
-//  * backward: recomputes the per-pixel coefficient from depth/edge/normal (16 B/px of traffic;
-//    the forward stashes only alpha) and gathers the 3x3 adjoint from registers + shuffles.
+//    stencil kernels overlap by one lane on each side (two for the VEC=1 non-stash backward), so
+//    horizontal neighbours always come from a warp shuffle and vertical ones from a rolling row window;
+//  * forward (edge_loss_fwd_kernel): persistent warps, each over an equal, cost-balanced range of strip
+//    rows fed by a cp.async shared-memory row ring: 3x3 responses -> pick by quantised normal -> sigmoid
+//    -> soft-label BCE terms; warp sums -> per-image 2^32 fixed-point integer atomics -> the last CTA
+//    (atomic ticket) computes the per-image class balance alpha and writes the loss: single launch, no
+//    host sync, bit-reproducible run to run.  It also writes the grad map and, for directional
+//    responses, a 1 B/px stash (picked direction + sign of the response);
+//  * backward from the stash (edge_loss_bwd_ring_kernel at VEC=4 on the forward's unit ranges,
+//    edge_loss_bwd_stash_kernel at VEC=1 on fixed work items): reads grad map, edge and stash, looks the
+//    3x3 adjoint up in a 16-entry table and scatters it into three rolling output rows;
+//  * backward without a stash (edge_loss_bwd_kernel, e.g. magnitude responses or a resized scale):
+//    recomputes the responses from depth / edge / normal and gathers the 3x3 adjoint from registers +
+//    shuffles.
 #pragma once
 #include <math.h>
 #include <stdlib.h>
@@ -28,14 +33,7 @@ enum { A_WP = 0, A_WN, A_SPU, A_SNU, A_SPM, A_SNM, A_SUMM, A_FLAGS };
 enum { F_HAS0 = 1u, F_HAS1 = 2u, F_OTHER = 4u, F_NONFINITE = 8u };
 enum { MODE_NONE = 0, MODE_MAG = 1, MODE_DIR = 2 };
 
-#ifndef MTE_FWD_MINB
-#define MTE_FWD_MINB 2
-#endif
-#ifndef MTE_FWD_RH
-#define MTE_FWD_RH 6
-#endif
-constexpr int kFwdRH = MTE_FWD_RH;   // output rows per forward work item
-constexpr int kBwdRH = 8;   // output rows per backward work item
+constexpr int kBwdRH = 8;   // output rows per work item of edge_loss_bwd_kernel / edge_loss_bwd_stash_kernel
 // the streaming (ring) kernels: warps per CTA, CTAs per SM, ring depths -- tuning knobs.  Measured on B200 at the
 // config-3 loss shape (bench.py, us per fwd+bwd step): 2 CTAs x 8 warps, depths 8/6: 43.4; 1 CTA x 16 warps: depths
 // 8/6 43.4, 7/5 41.7, 5/4 40.8, 4/4 39.9, 3/3 39.2, 3/2 38.5, 3/1 41.3; 24 warps 42.0.  Shallow rings win: deeper
@@ -79,9 +77,10 @@ struct ScaleP {
     float *g, *dx;
     unsigned char *stash;  // 1 B/px: bits 0-1 picked direction, bits 2-3 sign of the response (1:+ 2:- 0:zero)
     int B, H, W;
-    int strips, rowBlocks, items, ctasPerImage;
-    int ctaBase, imgBase;
-    int unitBase;  // forward: first unit (strip row) of this scale in the global unit order
+    int strips;
+    int rowBlocks, items, ctasPerImage, ctaBase;  // work items of edge_loss_bwd_kernel / edge_loss_bwd_stash_kernel only
+    int imgBase;
+    int unitBase;  // forward / ring backward: first unit (strip row) of this scale in the global unit order
     float scaleWeight;
 };
 
@@ -89,9 +88,9 @@ struct LossP {
     ScaleP s[MTE_MAX_SCALES];
     int nScales, totalCtas, totalImages;
     float T, weight, p2n;
-    int totalUnits;                // forward: strip rows over all scales and images
+    int totalUnits;                // forward / ring backward: units over all scales and images
     unsigned long long *accum;     // forward: [totalImages][kAcc] fixed-point (2^32) per-image sums, zero at launch
-    unsigned *ticket;              // forward: dynamic item counter; [1]: finished-warp counter (both self-resetting)
+    unsigned *ticket;              // forward: [1] finished-CTA counter, [0] kept zero (both self-resetting)
     float *lossOut;         // [1+nScales]
     float *ctx;             // [totalImages] alpha, then per scale {coef, maskBinary}
     const float *gradLoss;  // bwd: [1+nScales]
@@ -153,7 +152,6 @@ __device__ __forceinline__ float ex2_approx(float x) {
     asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
     return r;
 }
-__device__ __forceinline__ float sigmoid_fast(float z) { return rcp_approx(1.0f + ex2_approx(z * -1.4426950408889634f)); }
 // Backward: p(1-p)/(1-p+eps) amplifies the last bits of p where the sigmoid saturates, so p is
 // computed the way eager PyTorch does (accurate expf, correctly rounded divide): the gradient then
 // reproduces the reference's own rounding, not only the underlying math.
@@ -165,18 +163,6 @@ struct Row {
     float l, r;
     __device__ __forceinline__ float at(int v) const { return v < 0 ? l : (v >= VEC ? r : c[v]); }
 };
-
-// Unchecked flavour for work items that lie completely inside the image (the common case): no predicates.
-template <int VEC>
-__device__ __forceinline__ void load_vec_in(float (&out)[VEC], const float *img, int row, int W, int col0, bool cached) {
-    const float *p = img + (size_t)row * W + col0;
-    if (VEC == 4) {
-        const float4 v = cached ? ld_cached4(p) : ld_stream4(p);
-        out[0] = v.x; out[1 % VEC] = v.y; out[2 % VEC] = v.z; out[3 % VEC] = v.w;
-    } else {
-        out[0] = cached ? __ldg(p) : __ldcs(p);
-    }
-}
 
 template <int VEC>
 __device__ __forceinline__ void load_vec(float (&out)[VEC], const float *img, int row, int H, int W, int col0,
@@ -202,14 +188,6 @@ __device__ __forceinline__ void load_row(Row<VEC> &R, const float *img, int row,
         const bool ok = (row >= 0) && (row < H) && (col0 >= 0) && (col0 < W);
 #pragma unroll
         for (int v = 0; v < VEC; v++) R.c[v] = ok ? inv_to_depth(R.c[v]) : 0.f;
-    }
-}
-template <int VEC, bool INV>
-__device__ __forceinline__ void load_row_in(Row<VEC> &R, const float *img, int row, int W, int col0) {
-    load_vec_in<VEC>(R.c, img, row, W, col0, true);
-    if (INV) {
-#pragma unroll
-        for (int v = 0; v < VEC; v++) R.c[v] = inv_to_depth(R.c[v]);
     }
 }
 // Horizontal neighbours across the lane boundary (lanes 0 / 31 get don't-care values: they are halo lanes).
@@ -242,12 +220,11 @@ __device__ __forceinline__ float pick_response(int k, float P, float R, float Dm
 // ---------------------------------------------------------------------------
 // Forward
 // ---------------------------------------------------------------------------
-// Persistent warps pull work items (a 32-lane strip x RH rows of one image) from one global atomic queue, biggest
-// scale first, so the tail is one item long whatever the shape.  An item streams its rows through a 3-row register
-// window with a PD-row prefetch ring.  Its partial sums are reduced in the warp (fixed order) and added to
-// per-image 2^32 fixed-point int64 accumulators with integer atomics: the result does not depend on the order in
-// which items finish, so the loss is bit-reproducible without any per-CTA partial buffer or barrier.  The last warp
-// to finish (atomic counter) folds the per-image sums into alpha and the loss.
+// Persistent warps, each over one equal, cost-balanced range of strip rows (see fwd_segment), cut into segments at
+// strip ends.  A segment's partial sums are reduced in the warp (fixed order) and added to per-image 2^32
+// fixed-point int64 accumulators with integer atomics: the result does not depend on the order in which segments
+// finish, so the loss is bit-reproducible without any per-CTA partial buffer or barrier.  The last CTA to finish
+// (atomic ticket) folds the per-image sums into alpha and the loss.
 constexpr double kFix = 4294967296.0;  // 2^32
 
 // Run by the LAST CTA to finish (all of its warps): warp k folds scale k -- one image per lane, plain butterflies in
@@ -342,18 +319,6 @@ __device__ __forceinline__ void prep_row(PRow<VEC> &R, const float (&x)[VEC]) {
     }
 }
 
-// The two bits of the quantised normal direction (0:h 1:rl 2:v 3:lr) as predicates, straight from the four band
-// compares: with f_k = [u >= B_k] (nested), X = f1 ^ f5, Y = f3 ^ f7:  bit0 = X ^ Y (odd count), bit1 = Y for
-// theta >= 0 and X for theta < 0 (the mirrored table).  See dir_index for the ulp step on the negative side.
-__device__ __forceinline__ void dir_bits(float t, bool &b0, bool &b1) {
-    const bool neg = t < 0.f;
-    const float u = __int_as_float((__float_as_int(t) & 0x7fffffff) - (neg ? 1 : 0));
-    const bool X = (u >= MTE_B1) != (u >= MTE_B5);
-    const bool Y = (u >= MTE_B3) != (u >= MTE_B7);
-    b0 = X != Y;
-    b1 = (X && neg) || (Y && !neg);
-}
-
 // base + 4 * off as ONE 64-bit multiply-add (opaque to the optimiser, which otherwise re-associates the plane
 // offset into every access)
 template <typename T>
@@ -365,8 +330,8 @@ __device__ __forceinline__ T *elem_addr(T *base, unsigned off) {
 
 // Directional response + stash code of one pixel with the instruction selection pinned (the compiler's version of
 // the same logic spends ~10 more instructions per pixel on predicate spills and integer re-materialisation):
-//   band compares on the ulp-stepped |theta| (see dir_index / dir_bits) -> X = f1^f5, Y = f3^f7
-//   bit0 = X^Y, bit1 = theta<0 ? X : Y ; direction 0:h 1:rl 2:v 3:lr
+//   band compares f_k = [u >= B_k] (nested) on the ulp-stepped u = |theta| (see dir_index) -> X = f1^f5, Y = f3^f7
+//   bit0 = X^Y (odd count), bit1 = theta<0 ? X : Y (the mirrored table) ; direction 0:h 1:rl 2:v 3:lr
 //   c = (bit1 ? Pv : Rh) + (bit1 ? (bit0 ? Rh : dv) : (bit0 ? -Pv : Dm))
 //   code = direction | 4 << signbit(c)   (bits 2-3: 1 = "+", 2 = "-"; a zero response is recognised by the
 //   backward from the grad map itself, |c| == 0)
@@ -459,9 +424,9 @@ __device__ __forceinline__ void lds_vec(float (&out)[VEC], const unsigned char *
 }
 
 __host__ __device__ constexpr int fwd_planes(int mode, bool mask) { return 2 + (mode == MODE_DIR ? 1 : 0) + (mask ? 1 : 0); }
-__host__ __device__ constexpr int fwd_ring_depth(int mode, bool mask) { return MTE_FWD_D; }
+constexpr int kFwdRingDepth = MTE_FWD_D;
 __host__ __device__ constexpr int fwd_smem_bytes(int vec, int mode, bool mask) {
-    return kRWarps * fwd_ring_depth(mode, mask) * fwd_planes(mode, mask) * 32 * vec * 4;
+    return kRWarps * kFwdRingDepth * fwd_planes(mode, mask) * 32 * vec * 4;
 }
 
 // Forward work decomposition: the unit is one row of one strip (32 lanes x VEC px, LANES of them writing) of one
@@ -472,7 +437,7 @@ template <int VEC, int MODE, bool MASK, bool INV, bool SIG>
 __device__ __forceinline__ void fwd_segment(const LossP &P, const ScaleP &S, int img, int strip, int row0, int nrows,
                                             int lane, unsigned char *ring, float (&la)[kAcc - 1], unsigned &lflags,
                                             float &poison) {
-    constexpr int D = fwd_ring_depth(MODE, MASK);
+    constexpr int D = kFwdRingDepth;
     constexpr int NPL = fwd_planes(MODE, MASK);
     constexpr unsigned PLB = 32 * VEC * 4;     // bytes of one plane row in a slot
     constexpr unsigned SLB = NPL * PLB;        // bytes of a slot
@@ -649,6 +614,35 @@ __device__ __forceinline__ void fwd_segment(const LossP &P, const ScaleP &S, int
     }
 }
 
+// The next segment of a warp's unit range [u0, u1) (u0 advances past it).  A strip is H rows plus COST virtual units
+// that stand for the cost of opening a segment (window prologue + pipeline fill), so ranges that span several strips
+// are charged for it; nrows <= 0: the range held only virtual units (img and strip are left unset).
+struct UnitSeg {
+    int si, img, strip, row0, nrows;
+};
+template <int COST>
+__device__ __forceinline__ UnitSeg unit_segment(const LossP &P, int &u0, int u1) {
+    UnitSeg s;
+    s.si = 0;
+#pragma unroll
+    for (int k = 1; k < MTE_MAX_SCALES; k++)
+        if (k < P.nScales && u0 >= P.s[k].unitBase) s.si = k;
+    const ScaleP &S = P.s[s.si];
+    const int local = u0 - S.unitBase;
+    const int HV = S.H + COST;
+    const int t = local / HV;  // (image, strip)
+    const int r = local - t * HV;
+    const int take = min(HV - r, u1 - u0);
+    s.row0 = max(r - COST, 0);
+    s.nrows = max(r + take - COST, 0) - s.row0;
+    u0 += take;
+    if (s.nrows > 0) {
+        s.img = t / S.strips;
+        s.strip = t - s.img * S.strips;
+    }
+    return s;
+}
+
 template <int VEC, int MODE, bool MASK, bool INV, bool SIG>
 __global__ void __launch_bounds__(kRThreads, kRMinB) edge_loss_fwd_kernel(const __grid_constant__ LossP P) {
     extern __shared__ __align__(16) unsigned char fwdRing[];
@@ -661,33 +655,18 @@ __global__ void __launch_bounds__(kRThreads, kRMinB) edge_loss_fwd_kernel(const 
     pdl_launch_dependents();
     pdl_wait();
     while (u0 < u1) {
-        int si = 0;
-#pragma unroll
-        for (int k = 1; k < MTE_MAX_SCALES; k++)
-            if (k < P.nScales && u0 >= P.s[k].unitBase) si = k;
-        const ScaleP &S = P.s[si];
-        // a strip is H rows plus kSegCost virtual units that stand for the cost of opening a segment (window
-        // prologue + pipeline fill), so ranges that span several strips are charged for it
-        const int local = u0 - S.unitBase;
-        const int HV = S.H + kSegCost;
-        const int t = local / HV;  // (image, strip)
-        const int r = local - t * HV;
-        const int take = min(HV - r, u1 - u0);
-        const int row0 = max(r - kSegCost, 0);
-        const int nrows = max(r + take - kSegCost, 0) - row0;
-        u0 += take;
-        if (nrows <= 0) continue;
-        const int img = t / S.strips;
-        const int strip = t - img * S.strips;
+        const UnitSeg sg = unit_segment<kSegCost>(P, u0, u1);
+        if (sg.nrows <= 0) continue;
+        const ScaleP &S = P.s[sg.si];
         float la[kAcc - 1];
 #pragma unroll
         for (int k = 0; k < kAcc - 1; k++) la[k] = 0.f;
         unsigned lflags = 0;
         float poison = 0.f;
-        fwd_segment<VEC, MODE, MASK, INV, SIG>(P, S, img, strip, row0, nrows, lane, ring, la, lflags, poison);
+        fwd_segment<VEC, MODE, MASK, INV, SIG>(P, S, sg.img, sg.strip, sg.row0, sg.nrows, lane, ring, la, lflags, poison);
         bool bad = __any_sync(MTE_FULL_MASK, !(poison == 0.f));
         // order-independent accumulation: warp tree (fixed) -> 2^32 fixed point -> integer atomics
-        unsigned long long *acc = P.accum + (size_t)(S.imgBase + img) * kAcc;
+        unsigned long long *acc = P.accum + (size_t)(S.imgBase + sg.img) * kAcc;
 #pragma unroll
         for (int k = 0; k < kAcc - 1; k++) {
             if (MASK || k == A_WP || k == A_SPU || k == A_SNU) {
@@ -756,6 +735,20 @@ __device__ __forceinline__ float dloss_dg(float g, float ee, float mm, const Bwd
     return SIG ? d * p * q : d;
 }
 
+// Coefficients of image img of scale si: the upstream gradient of the total and of the scale's loss, the scale's
+// normaliser and mask flag and the image's alpha, all left in ctx by the forward.
+template <bool MASK>
+__device__ __forceinline__ BwdImg bwd_img(const LossP &P, const ScaleP &S, int si, int img) {
+    const float G = __ldg(P.gradLoss) * S.scaleWeight + __ldg(P.gradLoss + 1 + si);
+    const float coef = __ldg(P.ctx + P.totalImages + 2 * si) * G;
+    const float alpha = __ldg(P.ctx + S.imgBase + img);
+    BwdImg I;
+    I.cp = -coef * P.p2n * alpha;
+    I.cn = coef * (1.0f - alpha);
+    I.maskBinary = MASK && (__ldg(P.ctx + P.totalImages + 2 * si + 1) != 0.f);
+    return I;
+}
+
 template <int VEC, int MODE, bool MASK, bool INV, bool SIG>
 __global__ void __launch_bounds__(kThreads, 2) edge_loss_bwd_kernel(const __grid_constant__ LossP P) {
     static_assert(MODE != MODE_NONE, "pointwise backward has its own kernel");
@@ -771,16 +764,7 @@ __global__ void __launch_bounds__(kThreads, 2) edge_loss_bwd_kernel(const __grid
     const int img = local / S.ctasPerImage;
     const int item0 = (local - img * S.ctasPerImage) * kWarps + warp;
     const int H = S.H, W = S.W;
-
-    BwdImg I;
-    {
-        const float G = __ldg(P.gradLoss) * S.scaleWeight + __ldg(P.gradLoss + 1 + si);
-        const float coef = __ldg(P.ctx + P.totalImages + 2 * si) * G;
-        const float alpha = __ldg(P.ctx + S.imgBase + img);
-        I.cp = -coef * P.p2n * alpha;
-        I.cn = coef * (1.0f - alpha);
-        I.maskBinary = MASK && (__ldg(P.ctx + P.totalImages + 2 * si + 1) != 0.f);
-    }
+    const BwdImg I = bwd_img<MASK>(P, S, si, img);
 
     for (int item = item0; item < S.items; item += S.ctasPerImage * kWarps) {  // warp-uniform
     const int strip = item / S.rowBlocks;
@@ -914,21 +898,53 @@ __global__ void __launch_bounds__(kThreads, 2) edge_loss_bwd_kernel(const __grid
 // per pixel (direction + sign), so the backward needs neither the 3x3 stencil nor the normals: per pixel it
 // recomputes p = sigmoid(g - T) the reference-faithful way, d loss/d g, looks the four adjoint coefficients up
 // in a 16-entry shared-memory table and scatters them into three rolling output rows.
-// Traffic: g 4 + edge 4 + stash 1 (+ inverse depth 4 when fused) in, gradient 4 out.
+// Traffic: g 4 + edge 4 + stash 1 (+ inverse depth 4 when fused) in, gradient 4 out.  This is the VEC=1 kernel (rows
+// that are not whole float4s); at VEC=4 edge_loss_bwd_ring_kernel runs.
 // ---------------------------------------------------------------------------
-template <int VEC, bool MASK, bool INV, bool SIG>
+// Entry `code` (direction | sign << 2) of the 16-entry adjoint table: (A, C, A2, C2) for s = 1.
+__device__ __forceinline__ float4 adjoint_entry(int code) {
+    const int di = code & 3, sg = code >> 2;
+    const float sgn = sg == 1 ? 1.f : (sg == 2 ? -1.f : 0.f);
+    const float a = (di == 2 || di == 3) ? 1.f : (di == 1 ? -1.f : 0.f);  // h:0 rl:-1 v:1 lr:1
+    const float c = (di == 2) ? 0.f : 1.f;                                // h:1 rl:1 v:0 lr:1
+    const float bb = (di & 1) ? 1.f : 2.f;                                // axis stencils weigh the centre twice
+    return make_float4(sgn * a, sgn * c, sgn * a * bb, sgn * c * bb);
+}
+
+// What one row of adjoint coefficients (A, C, A2, C2 per pixel; horizontal neighbours from the adjacent lanes) adds to
+// the three output rows it touches: `up` to the row it acts as "up" for, `mid` to the one above, and `dn` (to be
+// subtracted) to the one above that, which it completes.
+template <int VEC>
+struct AdjointRows {
+    float up[VEC], mid[VEC], dn[VEC];
+};
+template <int VEC>
+__device__ __forceinline__ AdjointRows<VEC> adjoint_rows(const float (&A)[VEC], const float (&C)[VEC],
+                                                         const float (&A2)[VEC], const float (&C2)[VEC]) {
+    const float Al = __shfl_up_sync(MTE_FULL_MASK, A[VEC - 1], 1), Ar = __shfl_down_sync(MTE_FULL_MASK, A[0], 1);
+    const float Cl = __shfl_up_sync(MTE_FULL_MASK, C[VEC - 1], 1), Cr = __shfl_down_sync(MTE_FULL_MASK, C[0], 1);
+    const float C2l = __shfl_up_sync(MTE_FULL_MASK, C2[VEC - 1], 1), C2r = __shfl_down_sync(MTE_FULL_MASK, C2[0], 1);
+    AdjointRows<VEC> R;
+#pragma unroll
+    for (int v = 0; v < VEC; v++) {
+        const float a_l = v == 0 ? Al : A[(v + VEC - 1) % VEC], a_r = v == VEC - 1 ? Ar : A[(v + 1) % VEC];
+        const float c_l = v == 0 ? Cl : C[(v + VEC - 1) % VEC], c_r = v == VEC - 1 ? Cr : C[(v + 1) % VEC];
+        const float c2_l = v == 0 ? C2l : C2[(v + VEC - 1) % VEC], c2_r = v == VEC - 1 ? C2r : C2[(v + 1) % VEC];
+        const float SA = (a_l + a_r) + A2[v], DC = c_l - c_r;
+        R.up[v] = SA + DC;
+        R.mid[v] = c2_l - c2_r;
+        R.dn[v] = SA - DC;
+    }
+    return R;
+}
+
+template <bool MASK, bool INV, bool SIG>
 __global__ void __launch_bounds__(kThreads, 2) edge_loss_bwd_stash_kernel(const __grid_constant__ LossP P) {
+    constexpr int VEC = 1;
     constexpr int RH = kBwdRH;
     constexpr int PD = 3;
     __shared__ float4 sLut[16];  // per code: (A, C, A2, C2) for s = 1
-    if (threadIdx.x < 16) {
-        const int di = threadIdx.x & 3, sg = threadIdx.x >> 2;
-        const float sgn = sg == 1 ? 1.f : (sg == 2 ? -1.f : 0.f);
-        const float a = (di == 2 || di == 3) ? 1.f : (di == 1 ? -1.f : 0.f);  // h:0 rl:-1 v:1 lr:1
-        const float c = (di == 2) ? 0.f : 1.f;                                // h:1 rl:1 v:0 lr:1
-        const float bb = (di & 1) ? 1.f : 2.f;                                // axis stencils weigh the centre twice
-        sLut[threadIdx.x] = make_float4(sgn * a, sgn * c, sgn * a * bb, sgn * c * bb);
-    }
+    if (threadIdx.x < 16) sLut[threadIdx.x] = adjoint_entry(threadIdx.x);
     __syncthreads();
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     int si = 0;
@@ -940,18 +956,7 @@ __global__ void __launch_bounds__(kThreads, 2) edge_loss_bwd_stash_kernel(const 
     const int img = local / S.ctasPerImage;
     const int item0 = (local - img * S.ctasPerImage) * kWarps + warp;
     const int H = S.H, W = S.W;
-    constexpr int HALO = bwd_halo(VEC), LANES = bwd_lanes(VEC);
-    (void)HALO;
-
-    BwdImg I;
-    {
-        const float G = __ldg(P.gradLoss) * S.scaleWeight + __ldg(P.gradLoss + 1 + si);
-        const float coef = __ldg(P.ctx + P.totalImages + 2 * si) * G;
-        const float alpha = __ldg(P.ctx + S.imgBase + img);
-        I.cp = -coef * P.p2n * alpha;
-        I.cn = coef * (1.0f - alpha);
-        I.maskBinary = MASK && (__ldg(P.ctx + P.totalImages + 2 * si + 1) != 0.f);
-    }
+    const BwdImg I = bwd_img<MASK>(P, S, si, img);
     const size_t plane = (size_t)img * H * W;
 
     for (int item = item0; item < S.items; item += S.ctasPerImage * kWarps) {  // warp-uniform
@@ -971,12 +976,7 @@ __global__ void __launch_bounds__(kThreads, 2) edge_loss_bwd_stash_kernel(const 
             if (MASK) load_vec<VEC>(pfm[slot], S.m + plane, row, H, W, col0, false);
             if (INV) load_vec<VEC>(pfx[slot], S.x + plane, row, H, W, col0, false);
             const bool ok = row >= 0 && row < H && colOk;
-            unsigned c = 0;
-            if (ok) {
-                const unsigned char *sp = S.stash + plane + (size_t)row * W + col0;
-                c = (VEC == 4) ? __ldcs(reinterpret_cast<const unsigned *>(sp)) : (unsigned)__ldcs(sp);
-            }
-            pfc[slot] = c;
+            pfc[slot] = ok ? (unsigned)__ldcs(S.stash + plane + (size_t)row * W + col0) : 0u;
         };
 #pragma unroll
         for (int k = 0; k < PD; k++) fetch(k, row0 - 1 + k);
@@ -1008,18 +1008,12 @@ __global__ void __launch_bounds__(kThreads, 2) edge_loss_bwd_stash_kernel(const 
                 const float4 k = sLut[(codes >> (8 * v)) & 15u];
                 A[v] = d * k.x; C[v] = d * k.y; A2[v] = d * k.z; C2[v] = d * k.w;
             }
-            const float Al = __shfl_up_sync(MTE_FULL_MASK, A[VEC - 1], 1), Ar = __shfl_down_sync(MTE_FULL_MASK, A[0], 1);
-            const float Cl = __shfl_up_sync(MTE_FULL_MASK, C[VEC - 1], 1), Cr = __shfl_down_sync(MTE_FULL_MASK, C[0], 1);
-            const float C2l = __shfl_up_sync(MTE_FULL_MASK, C2[VEC - 1], 1), C2r = __shfl_down_sync(MTE_FULL_MASK, C2[0], 1);
+            const AdjointRows<VEC> R = adjoint_rows<VEC>(A, C, A2, C2);
 #pragma unroll
             for (int v = 0; v < VEC; v++) {
-                const float a_l = v == 0 ? Al : A[v - 1], a_r = v == VEC - 1 ? Ar : A[(v + 1) % VEC];
-                const float c_l = v == 0 ? Cl : C[v - 1], c_r = v == VEC - 1 ? Cr : C[(v + 1) % VEC];
-                const float c2_l = v == 0 ? C2l : C2[v - 1], c2_r = v == VEC - 1 ? C2r : C2[(v + 1) % VEC];
-                const float SA = (a_l + a_r) + A2[v], DC = c_l - c_r;
-                oacc[j % 3][v] = SA + DC;                           // output row j   (this row acts as "up")
-                if (j >= 1) oacc[(j + 2) % 3][v] += c2_l - c2_r;    // output row j-1 ("mid")
-                if (j >= 2) oacc[(j + 1) % 3][v] -= SA - DC;        // output row j-2 ("down"), now complete
+                oacc[j % 3][v] = R.up[v];                           // output row j   (this row acts as "up")
+                if (j >= 1) oacc[(j + 2) % 3][v] += R.mid[v];       // output row j-1 ("mid")
+                if (j >= 2) oacc[(j + 1) % 3][v] -= R.dn[v];        // output row j-2 ("down"), now complete
             }
             if (j >= 2) {
                 const int o = j - 2, orow = row0 + o;
@@ -1036,11 +1030,7 @@ __global__ void __launch_bounds__(kThreads, 2) edge_loss_bwd_stash_kernel(const 
                     }
                     out[v] = d;
                 }
-                if (writer && orow < H) {
-                    float *op = S.dx + plane + (size_t)orow * W + col0;
-                    if (VEC == 4) st_stream4(op, make_float4(out[0], out[1 % VEC], out[2 % VEC], out[3 % VEC]));
-                    else __stcs(op, out[0]);
-                }
+                if (writer && orow < H) __stcs(S.dx + plane + (size_t)orow * W + col0, out[0]);
             }
         }
     }
@@ -1053,26 +1043,19 @@ __global__ void __launch_bounds__(kThreads, 2) edge_loss_bwd_stash_kernel(const 
 // a zero stash byte selects the all-zero table entry, so padding needs no predicates in the row loop.
 // ---------------------------------------------------------------------------
 constexpr int kSegCostB = MTE_SEGCOST_B;
-__host__ __device__ constexpr int bwd_ring_depth(bool mask, bool inv) { return MTE_BWD_D; }
+constexpr int kBwdRingDepth = MTE_BWD_D;
 __host__ __device__ constexpr int bwd_slot_bytes(bool mask, bool inv) { return (2 + (mask ? 1 : 0) + (inv ? 1 : 0)) * 512 + 128; }
-__host__ __device__ constexpr int bwd_smem_bytes(bool mask, bool inv) { return kRWarps * bwd_ring_depth(mask, inv) * bwd_slot_bytes(mask, inv); }
+__host__ __device__ constexpr int bwd_smem_bytes(bool mask, bool inv) { return kRWarps * kBwdRingDepth * bwd_slot_bytes(mask, inv); }
 
 template <bool MASK, bool INV, bool SIG>
 __global__ void __launch_bounds__(kRThreads, kRMinB) edge_loss_bwd_ring_kernel(const __grid_constant__ LossP P) {
     constexpr int VEC = 4;
-    constexpr int D = bwd_ring_depth(MASK, INV);
+    constexpr int D = kBwdRingDepth;
     constexpr unsigned PLB = 512, SLB = bwd_slot_bytes(MASK, INV);
     constexpr unsigned O_G = 0, O_E = PLB, O_M = 2 * PLB, O_X = (MASK ? 3 : 2) * PLB, O_S = SLB - 128;
     extern __shared__ __align__(16) unsigned char bwdRing[];
     __shared__ float4 sLut[16];  // per code: (A, C, A2, C2) for s = 1
-    if (threadIdx.x < 16) {
-        const int di = threadIdx.x & 3, sg = threadIdx.x >> 2;
-        const float sgn = sg == 1 ? 1.f : (sg == 2 ? -1.f : 0.f);
-        const float a = (di == 2 || di == 3) ? 1.f : (di == 1 ? -1.f : 0.f);  // h:0 rl:-1 v:1 lr:1
-        const float c = (di == 2) ? 0.f : 1.f;                                // h:1 rl:1 v:0 lr:1
-        const float bb = (di & 1) ? 1.f : 2.f;                                // axis stencils weigh the centre twice
-        sLut[threadIdx.x] = make_float4(sgn * a, sgn * c, sgn * a * bb, sgn * c * bb);
-    }
+    if (threadIdx.x < 16) sLut[threadIdx.x] = adjoint_entry(threadIdx.x);
     __syncthreads();
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     unsigned char *ring = bwdRing + warp * (D * SLB);
@@ -1086,34 +1069,13 @@ __global__ void __launch_bounds__(kRThreads, kRMinB) edge_loss_bwd_ring_kernel(c
     pdl_launch_dependents();
     pdl_wait();
     while (u0 < u1) {
-        int si = 0;
-#pragma unroll
-        for (int k = 1; k < MTE_MAX_SCALES; k++)
-            if (k < P.nScales && u0 >= P.s[k].unitBase) si = k;
-        const ScaleP &S = P.s[si];
-        const int local = u0 - S.unitBase;
-        const int HV = S.H + kSegCostB;
-        const int t = local / HV;  // (image, strip)
-        const int r = local - t * HV;
-        const int take = min(HV - r, u1 - u0);
-        const int row0 = max(r - kSegCostB, 0);
-        const int nrows = max(r + take - kSegCostB, 0) - row0;
-        u0 += take;
-        if (nrows <= 0) continue;
-        const int img = t / S.strips;
-        const int strip = t - img * S.strips;
+        const UnitSeg sg = unit_segment<kSegCostB>(P, u0, u1);
+        if (sg.nrows <= 0) continue;
+        const ScaleP &S = P.s[sg.si];
+        const int img = sg.img, strip = sg.strip, row0 = sg.row0, nrows = sg.nrows;
         const int H = S.H;
         const unsigned W = (unsigned)S.W;
-
-        BwdImg I;
-        {
-            const float G = __ldg(P.gradLoss) * S.scaleWeight + __ldg(P.gradLoss + 1 + si);
-            const float coef = __ldg(P.ctx + P.totalImages + 2 * si) * G;
-            const float alpha = __ldg(P.ctx + S.imgBase + img);
-            I.cp = -coef * P.p2n * alpha;
-            I.cn = coef * (1.0f - alpha);
-            I.maskBinary = MASK && (__ldg(P.ctx + P.totalImages + 2 * si + 1) != 0.f);
-        }
+        const BwdImg I = bwd_img<MASK>(P, S, sg.si, img);
         // one halo lane per side (the coefficients are pointwise): lanes 1..30 write
         const int col0 = (strip * kHaloLanes + lane - 1) * VEC;
         const bool colOk = col0 >= 0 && col0 < (int)W;
@@ -1170,20 +1132,14 @@ __global__ void __launch_bounds__(kRThreads, kRMinB) edge_loss_bwd_ring_kernel(c
                         const float4 k = sLut[(codes >> (8 * v)) & 15u];
                         A[v] = d * k.x; C[v] = d * k.y; A2[v] = d * k.z; C2[v] = d * k.w;
                     }
-                    const float Al = __shfl_up_sync(MTE_FULL_MASK, A[VEC - 1], 1), Ar = __shfl_down_sync(MTE_FULL_MASK, A[0], 1);
-                    const float Cl = __shfl_up_sync(MTE_FULL_MASK, C[VEC - 1], 1), Cr = __shfl_down_sync(MTE_FULL_MASK, C[0], 1);
-                    const float C2l = __shfl_up_sync(MTE_FULL_MASK, C2[VEC - 1], 1), C2r = __shfl_down_sync(MTE_FULL_MASK, C2[0], 1);
                     // this coefficient row acts as "up" for output row j (image row row0 - 1 + j ... stored as
                     // segment output o = j), as "mid" for o = j - 1 and as "down" for o = j - 2, which it completes
+                    const AdjointRows<VEC> R = adjoint_rows<VEC>(A, C, A2, C2);
 #pragma unroll
                     for (int v = 0; v < VEC; v++) {
-                        const float a_l = v == 0 ? Al : A[(v + VEC - 1) % VEC], a_r = v == VEC - 1 ? Ar : A[(v + 1) % VEC];
-                        const float c_l = v == 0 ? Cl : C[(v + VEC - 1) % VEC], c_r = v == VEC - 1 ? Cr : C[(v + 1) % VEC];
-                        const float c2_l = v == 0 ? C2l : C2[(v + VEC - 1) % VEC], c2_r = v == VEC - 1 ? C2r : C2[(v + 1) % VEC];
-                        const float SA = (a_l + a_r) + A2[v], DC = c_l - c_r;
-                        oacc[u][v] = SA + DC;
-                        oacc[(u + 2) % 3][v] += c2_l - c2_r;
-                        oacc[(u + 1) % 3][v] -= SA - DC;
+                        oacc[u][v] = R.up[v];
+                        oacc[(u + 2) % 3][v] += R.mid[v];
+                        oacc[(u + 1) % 3][v] -= R.dn[v];
                     }
                     if (j >= 2) {
                         float out[VEC];
@@ -1224,14 +1180,13 @@ static void launch_fwd_one(const LossP &P, cudaStream_t st) {
     launch_pdl(edge_loss_fwd_kernel<VEC, MODE, MASK, INV, SIG>, P.totalCtas, kRThreads, smem, st, P);
 }
 
-// launchers implemented one translation unit per (direction, VEC) so they compile in parallel
+// launchers implemented one translation unit per (direction, VEC) / kernel family so they compile in parallel
 void launch_fwd_v4(const LossP &P, int mode, bool mask, bool inv, bool sig, cudaStream_t st);
 void launch_fwd_v1(const LossP &P, int mode, bool mask, bool inv, bool sig, cudaStream_t st);
 void launch_bwd_v4(const LossP &P, int mode, bool mask, bool inv, bool sig, cudaStream_t st);
 void launch_bwd_v1(const LossP &P, int mode, bool mask, bool inv, bool sig, cudaStream_t st);
-void launch_bwd_stash_v4(const LossP &P, bool mask, bool inv, bool sig, cudaStream_t st);
-void launch_bwd_ring_v4(const LossP &P, bool mask, bool inv, bool sig, cudaStream_t st);
-void launch_bwd_stash_v1(const LossP &P, bool mask, bool inv, bool sig, cudaStream_t st);
+void launch_bwd_ring(const LossP &P, bool mask, bool inv, bool sig, cudaStream_t st);   // VEC=4
+void launch_bwd_stash(const LossP &P, bool mask, bool inv, bool sig, cudaStream_t st);  // VEC=1
 
 #define MTE_LOSS_DISPATCH_BOOL(flag, NAME, ...) \
     if (flag) { constexpr bool NAME = true; __VA_ARGS__ } else { constexpr bool NAME = false; __VA_ARGS__ }

@@ -37,7 +37,9 @@ RTOL = 1e-5
 DIR, MAG, NONE = "dir", "mag", "none"
 
 # ---- the planner, restated (csrc/edge_loss.cu make_plan, csrc/edge_loss_kernels.cuh) -------------------------------
-K_FWD_RH, K_BWD_RH = 6, 8               # MTE_FWD_RH, kBwdRH
+# K_FWD_RH: row height of the forward's shape-spread criterion (the forward itself plans strip rows, not row blocks);
+# K_BWD_RH: kBwdRH, the row height of a work item of the non-ring backward kernels
+K_FWD_RH, K_BWD_RH = 6, 8
 K_HALO_LANES = 30                       # writing lanes of an overlapped forward / stash strip
 
 
