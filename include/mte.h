@@ -163,6 +163,16 @@ int mte_canny_from_depth(const void *depth, int depth_dtype, int n_images, int H
                          uint8_t *edges, uint8_t *levels, void *workspace, size_t workspace_bytes,
                          mte_stream_t stream);
 
+/* Resize of predicted depth to the GT size in front of the Canny sweep:
+ * cv2.resize(depth, (W, H), interpolation=cv2.INTER_LINEAR) of edge.py:76-78 (twin
+ * packnet_code/packnet_sfm/utils/edge.py:76-78), bit-exact against the opencv-python 4.13.0 wheel with its IPP
+ * HAL on (DESIGN.md section 2).  src: [N,h,w] of dtype, dst: out [N,H,W] of the same dtype; src and dst must not
+ * overlap.  Takes MTE_F32 with h, w >= 2 only: MTE_F64 (or any other dtype) is MTE_ERR_ARG and a one-row or
+ * one-column source MTE_ERR_SHAPE, the inputs whose cv2.resize arithmetic is not pinned.  Both pointers must be
+ * 4-byte aligned (MTE_ERR_ALIGN).  The same shape is a device-to-device copy.  No workspace. */
+int mte_resize_linear(const void *src, int dtype, int n_images, int h, int w, void *dst, int H, int W,
+                      mte_stream_t stream);
+
 /* ------------------------------------------------------------------------
  * (2b) DEE annotation post-process.
  * normals : infer_edge_estimation.py:193-199 (= :244-250)

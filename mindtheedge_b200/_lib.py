@@ -53,6 +53,7 @@ _SIGNATURES = {
     "mte_canny_workspace_bytes": (_sz, [_i, _i, _i, _i]),
     "mte_canny_from_depth": (_i, [_vp, _i, _i, _i, _i, _d, _d, C.POINTER(C.c_int32), C.POINTER(C.c_int32), _i,
                                   _vp, _vp, _vp, _sz, _vp]),
+    "mte_resize_linear": (_i, [_vp, _i, _i, _i, _i, _vp, _i, _i, _vp]),
     "mte_dee_workspace_bytes": (_sz, [_i, _i, _i]),
     "mte_dee_postprocess": (_i, [_vp, _i, _i, _i, _i, _i, _i, _d, _d, _vp, _vp, _i, _vp, _sz, _vp]),
     "mte_pr_workspace_bytes": (_sz, [_i, _i, _i, _i, _d]),

@@ -11,8 +11,9 @@
 //                                backwards and the raw values are written, with a mark per image that has a value > 1;
 //                                then the rule.  A downsample can drop every value > 1 of an image (a later pixel of
 //                                its block wins), so the input max is not the one the rule needs here.
-// The cv2.resize of the normal maps (:201-202, 213-217) is NOT reproduced: its float64 arithmetic is not
-// bit-reproducible (DESIGN.md); the reference's own pipeline reads per-scale normal PNGs when they exist
+// The cv2.resize of the normal maps (:201-202, 213-217) is NOT reproduced: it runs in float64, where the resize rule
+// of resize.cu is not pinned against cv2.resize (DESIGN.md section 2); the reference's own pipeline reads per-scale
+// normal PNGs when they exist
 // (gta_dataset.py:416-422), which is the case this covers.
 #include <math.h>
 

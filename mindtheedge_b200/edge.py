@@ -13,9 +13,14 @@
   of depth planes and T threshold pairs in, either the T edge planes or the
   single "birth level" plane out (no host round trip).
 
-All arithmetic after the file read runs in libmte.so (``mte_canny_from_depth``);
-there is no CPU fallback.  File decode and the optional ``cv2.resize`` to the GT
-size stay on the host, as in the reference (they are IO, SURVEY.md 8a a6).
+* ``resize_linear``    ``cv2.resize(depth, (W, H), interpolation=cv2.INTER_LINEAR)`` of ``edge.py:76-78`` on the
+  device, bit-exact for float32 planes of at least 2 x 2 (``mte_resize_linear``).
+
+All arithmetic after the file read runs in libmte.so (``mte_resize_linear``, ``mte_canny_from_depth``); there is no
+CPU fallback.  File decode stays on the host (IO).  The optional resize to the GT size is per-pixel arithmetic and
+runs on the device for float32 planes of at least 2 x 2; for the inputs whose ``cv2.resize`` arithmetic is not pinned
+(float64, one-row or one-column planes, DESIGN.md section 2) it stays ``cv2.resize`` on the host, so that no result
+differs from the reference.
 """
 from __future__ import annotations
 
@@ -27,7 +32,7 @@ import torch
 
 from . import _lib, runtime
 
-__all__ = ["canny_from_depth", "edge_from_depth", "edge_from_depth_cfg", "Canny", "read_depth_file",
+__all__ = ["canny_from_depth", "resize_linear", "resize_supported", "edge_from_depth", "edge_from_depth_cfg", "Canny", "read_depth_file",
            "chamfer_counts", "chamfer_distance", "compute_edge_metrics"]
 
 _DT = {torch.float32: _lib.MTE_F32, torch.float64: _lib.MTE_F64, torch.uint8: _lib.MTE_U8}
@@ -85,6 +90,45 @@ def canny_from_depth(depth: torch.Tensor, pairs: Sequence[Tuple[int, int]], min_
     return edges if want_edges else levels
 
 
+def _resize_linear_cuda(src, H, W):
+    """CUDA implementation of ``mte::resize_linear``: src [N,h,w] -> [N,H,W] of the same dtype."""
+    with runtime.on_device(src) as dev:
+        s = src.contiguous()
+        N, h, w = s.shape
+        out = torch.empty((N, H, W), dtype=s.dtype, device=dev)
+        runtime.call("mte_resize_linear", dev, s.data_ptr(), _DT.get(s.dtype, -1), N, h, w, out.data_ptr(), H, W,
+                     runtime.current_stream_ptr(dev))
+    return out
+
+
+runtime.define_op("resize_linear(Tensor src, int H, int W) -> Tensor", _resize_linear_cuda)
+
+
+def resize_supported(dtype, shape) -> bool:
+    """Whether ``resize_linear`` takes a plane of this dtype (NumPy or torch) and [h,w] (or [N,h,w]) shape: float32
+    with h, w >= 2, the inputs on which the kernel is pinned bit for bit against ``cv2.resize``."""
+    f32 = dtype == torch.float32 if isinstance(dtype, torch.dtype) else np.dtype(dtype) == np.float32
+    return f32 and len(shape) in (2, 3) and min(shape[-2:]) >= 2
+
+
+def resize_linear(src: torch.Tensor, size) -> torch.Tensor:
+    """``cv2.resize(src, (W, H), interpolation=cv2.INTER_LINEAR)`` on the device, bit for bit.
+
+    src   CUDA float32 [N,h,w] or [h,w], h and w >= 2 (other inputs raise ``MteError``: see ``resize_supported``).
+    size  (H, W) -- rows first, unlike cv2's dsize.
+    ->    float32 [N,H,W] or [H,W] on src's device.  Torch custom op ``mte::resize_linear``."""
+    runtime.require_cuda(src, "src")
+    if src.dim() not in (2, 3):
+        raise _lib.MteError("src must be [N,h,w] or [h,w]")
+    if not resize_supported(src.dtype, tuple(src.shape)):
+        raise _lib.MteError(f"resize_linear takes float32 planes of at least 2 x 2, got {src.dtype} "
+                            f"{tuple(src.shape)}")
+    H, W = (int(v) for v in size)
+    squeeze = src.dim() == 2
+    out = torch.ops.mte.resize_linear(src.unsqueeze(0) if squeeze else src, H, W)
+    return out[0] if squeeze else out
+
+
 def read_depth_file(file: str) -> np.ndarray:
     """edge.py:95-116 (``.npy`` as stored; ``.png`` as raw integer values with 0 -> -1)."""
     ext = file.split(".")[-1]
@@ -103,12 +147,15 @@ def read_depth_file(file: str) -> np.ndarray:
 
 
 def _edges_of_array(depth_im: np.ndarray, new_shape, min_depth, max_depth, thresh_1, thresh_2) -> np.ndarray:
-    if new_shape is not None:
+    on_device = new_shape is not None and resize_supported(depth_im.dtype, depth_im.shape) and depth_im.ndim == 2
+    if new_shape is not None and not on_device:
         import cv2
         depth_im = cv2.resize(depth_im, new_shape, interpolation=cv2.INTER_LINEAR)
     if depth_im.dtype not in (np.float32, np.float64):
         depth_im = depth_im.astype(np.float64)
     d = torch.from_numpy(np.ascontiguousarray(depth_im)).cuda(non_blocking=True)
+    if on_device:   # new_shape is cv2's dsize, (width, height)
+        d = resize_linear(d, (int(new_shape[1]), int(new_shape[0])))
     e = canny_from_depth(d, [(thresh_1, thresh_2)], min_depth, max_depth)
     return e[0].cpu().numpy()
 

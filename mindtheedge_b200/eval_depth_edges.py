@@ -31,7 +31,7 @@ import numpy as np
 import torch
 
 from . import _lib, runtime
-from .edge import canny_from_depth, read_depth_file
+from .edge import canny_from_depth, read_depth_file, resize_linear, resize_supported
 
 __all__ = [
     "EvalResult", "_pred_eval", "pr_counts", "correspond_pixels_batch", "evaluate_boundaries", "evaluate_boundaries_bin",
@@ -355,15 +355,19 @@ def _sweep_chunk(depth, gt, pairs, gt_crop, min_depth, max_depth, max_dist, per_
 def sweep_counts(depth: torch.Tensor, gt: torch.Tensor, edge_thresh_range, gt_crop, min_depth, max_depth,
                  max_dist=0.002, out=None, pipeline_chunks: Optional[int] = None,
                  per_image: bool = False) -> torch.Tensor:
-    """Device part of ``pr_evaluation`` for a batch: depth [N,H,W] (already at GT size), gt [N,H,W]
-    uint8 -> int64[len(range),4].  Thresholds are swept strictest first internally (the level plane
-    needs nested pairs) and returned in the caller's order.  ``per_image`` returns the counts of every image,
+    """Device part of ``pr_evaluation`` for a batch: depth [N,h,w], gt [N,H,W] uint8 -> int64[len(range),4].
+    Depth at another size than the GT is resized to it on the device first (``resize_linear``, bit-exact
+    ``cv2.resize`` INTER_LINEAR as edge.py:76-78; float32 of at least 2 x 2 only, anything else raises).
+    Thresholds are swept strictest first internally (the level plane needs nested pairs) and returned in the
+    caller's order.  ``per_image`` returns the counts of every image,
     int64[N,len(range),4] (``_pred_eval``'s counts of image i at every setting in row i), from the same launches.
 
     ``pipeline_chunks`` > 1 cuts the batch into chunks on side streams (a chunk's NMS + hysteresis next to another
     chunk's matcher; counts are integer sums, the result does not depend on the chunking).  Measured on the bench set:
     no gain (1.686 / 1.684 / 1.690 / 1.671 ms for 1-4 chunks) -- the step is the chain NMS -> hysteresis -> matcher of
     its SLOWEST image, which no reordering of other images shortens -- so the default is one chunk."""
+    if depth.shape[-2:] != gt.shape[-2:]:   # edge.py:76-78: the prediction is resized to the GT size first
+        depth = resize_linear(depth, tuple(gt.shape[-2:]))
     order = np.argsort(-np.asarray(edge_thresh_range), kind="stable")
     pairs = [(int(edge_thresh_range[i] / 2), int(edge_thresh_range[i])) for i in order]
     N = depth.shape[0] if depth.dim() == 3 else 1
@@ -396,11 +400,49 @@ def sweep_counts(depth: torch.Tensor, gt: torch.Tensor, edge_thresh_range, gt_cr
     return c
 
 
+def _device_resizable(d: np.ndarray, H: int, W: int) -> bool:
+    """A prediction that ``resize_linear`` brings to the GT size [H,W] on the device (float32 planes of at least
+    2 x 2); every other plane of another size keeps the host ``cv2.resize``."""
+    return d.ndim == 2 and d.shape != (H, W) and resize_supported(d.dtype, d.shape)
+
+
+def _depth_planes(depths, chunk, H, W, dev):
+    """depths[i] for i in chunk at the GT size [H,W], as one device tensor [len(chunk),H,W]: float32 when every plane
+    is float32, float64 otherwise (the quantisation runs in the plane's own float type, edge.py:85-87).  Planes that
+    ``_device_resizable`` takes are uploaded at their own size and resized on the device, one ``resize_linear`` per
+    source shape; the others are resized with ``cv2.resize`` on the host (edge.py:76-78) as before."""
+    import cv2
+    host, on_dev = {}, {}
+    for j, i in enumerate(chunk):
+        d = np.asarray(depths[i])
+        if _device_resizable(d, H, W):
+            on_dev.setdefault(d.shape, []).append(j)
+            continue
+        if d.shape != (H, W):
+            d = cv2.resize(d, (W, H), interpolation=cv2.INTER_LINEAR)
+        host[j] = d if d.dtype == np.float32 else d.astype(np.float64)
+    if not on_dev:
+        return torch.from_numpy(np.stack([host[j] for j in range(len(chunk))])).to(dev, non_blocking=True)
+    dtype = torch.float32 if all(d.dtype == np.float32 for d in host.values()) else torch.float64
+    out = torch.empty((len(chunk), H, W), dtype=dtype, device=dev)
+    if host:
+        js = sorted(host)
+        out[js] = torch.from_numpy(np.stack([host[j] for j in js])).to(dev, non_blocking=True).to(dtype)
+    for js in on_dev.values():
+        src = torch.from_numpy(np.stack([np.asarray(depths[chunk[j]]) for j in js])).to(dev, non_blocking=True)
+        r = resize_linear(src, (H, W))
+        if len(js) == len(chunk):
+            return r if dtype == torch.float32 else r.to(dtype)
+        out[js] = r.to(dtype)
+    return out
+
+
 def pr_evaluation_arrays(depths: Sequence[np.ndarray], gts: Sequence[np.ndarray], edge_thresh_range=None,
                          gt_crop=(44, 1197, 153, 371), min_depth=0.0, max_depth=80.0, batch: int = 32,
                          mask: Optional[np.ndarray] = None, per_image: bool = False):
-    """Array-level ``pr_evaluation``: predicted depth maps (any size; resized to the GT size on the
-    host with cv2.INTER_LINEAR as edge.py:76-78 does) and GT edge images (uint8, >127 = edge).
+    """Array-level ``pr_evaluation``: predicted depth maps (any size; resized to the GT size with cv2.INTER_LINEAR
+    as edge.py:76-78 does -- on the device, bit-exact, for float32 maps of at least 2 x 2, with ``cv2.resize`` on the
+    host for the others) and GT edge images (uint8, >127 = edge).
     Images are sharded over ``torch.distributed`` ranks when initialised.  ``mask`` is the mask-image branch of
     ``_pred_eval`` (eval_depth_edges.py:182-186, 198-200, 209-210): a float plane in [0,1] that multiplies both maps
     instead of the crop.
@@ -411,7 +453,6 @@ def pr_evaluation_arrays(depths: Sequence[np.ndarray], gts: Sequence[np.ndarray]
     with a mask the fractional ``(gt * mask).sum()``.  Under ``torch.distributed`` every rank fills its own rows of
     zero arrays and ONE integer all-reduce sums them (exact: the result does not depend on the number of ranks);
     ``counts`` is then the sum of the rows."""
-    import cv2
     if edge_thresh_range is None:
         edge_thresh_range = list(range(20, 241, 20))
     if mask is not None:
@@ -422,22 +463,20 @@ def pr_evaluation_arrays(depths: Sequence[np.ndarray], gts: Sequence[np.ndarray]
     counts = torch.zeros((len(edge_thresh_range), 4), dtype=torch.int64, device=dev)
     rows = torch.zeros((len(depths), len(edge_thresh_range), 4), dtype=torch.int64, device=dev) if per_image else None
     mine = shard_indices(len(depths), rank, world)
-    # group by GT shape and depth dtype so every launch is a dense batch; the quantisation runs in the
-    # array's own float type (edge.py:85-87), so float32 and float64 maps must not be mixed
+    # group by GT shape, source shape (of the planes resized on the device) and depth dtype so every launch is a
+    # dense batch; the quantisation runs in the array's own float type (edge.py:85-87), so float32 and float64 maps
+    # must not be mixed
     by_shape = {}
     for i in mine:
-        dt = np.float32 if np.asarray(depths[i]).dtype == np.float32 else np.float64
-        by_shape.setdefault((tuple(gts[i].shape[:2]), dt), []).append(i)
-    for ((H, W), dtype), idx in by_shape.items():
+        d = np.asarray(depths[i])
+        dt = np.float32 if d.dtype == np.float32 else np.float64
+        H, W = gts[i].shape[:2]
+        src = d.shape if _device_resizable(d, H, W) else None
+        by_shape.setdefault(((H, W), src, dt), []).append(i)
+    for ((H, W), _src, dtype), idx in by_shape.items():
         for s in range(0, len(idx), batch):
             chunk = idx[s:s + batch]
-            dep = []
-            for i in chunk:
-                d = np.asarray(depths[i])
-                if d.shape != (H, W):
-                    d = cv2.resize(d, (W, H), interpolation=cv2.INTER_LINEAR)
-                dep.append(d)
-            d_dev = torch.from_numpy(np.stack([d.astype(dtype, copy=False) for d in dep])).to(dev, non_blocking=True)
+            d_dev = _depth_planes(depths, chunk, H, W, dev)
             # _pred_eval: value/255 > 0.5 -> edge (eval_depth_edges.py:202-205)
             g_dev = torch.from_numpy(np.stack([(np.asarray(gts[i]) > 127).astype(np.uint8) for i in chunk])).to(
                 dev, non_blocking=True)
@@ -466,7 +505,6 @@ def _masked_evaluation(depths, gts, edge_thresh_range, mask, min_depth, max_dept
     radius is that of the uncropped plane, and ``sum_r`` is the fractional ``(gt * mask).sum()`` (float64, summed per
     image, then over images in list order -- eval_depth_edges.py:138, 299).  ``per_image`` as in
     ``pr_evaluation_arrays``, ``sum_r[i]`` being image i's ``(gt * mask).sum()``."""
-    import cv2
     rank, world = _dist_info()
     dev = torch.device("cuda", torch.cuda.current_device())
     T = len(edge_thresh_range)
@@ -482,21 +520,13 @@ def _masked_evaluation(depths, gts, edge_thresh_range, mask, min_depth, max_dept
     H, W = mask.shape
     for s0 in range(0, len(mine), batch):
         chunk = mine[s0:s0 + batch]
-        dep = []
-        for i in chunk:
-            d = np.asarray(depths[i])
-            if d.shape != (H, W):
-                d = cv2.resize(d, (W, H), interpolation=cv2.INTER_LINEAR)
-            dep.append(d if d.dtype == np.float32 else d.astype(np.float64))
-        if len({d.dtype for d in dep}) > 1:
-            dep = [d.astype(np.float64) for d in dep]
+        d_dev = _depth_planes(depths, chunk, H, W, dev)
         gb = [(np.asarray(gts[i]) > 127) for i in chunk]
         for i, g in zip(chunk, gb):
             s_i = (g.astype(np.float64) * mask).sum()
             sum_r = sum_r + s_i
             if per_image:
                 sum_r_img[i] = s_i
-        d_dev = torch.from_numpy(np.stack(dep)).to(dev)
         g_dev = torch.from_numpy(np.stack(gb)).to(dev)
         levels = canny_from_depth(d_dev, pairs, min_depth, max_depth, want_edges=False, want_levels=True)
         levels = torch.where(keep_p[None], levels, torch.full_like(levels, 255))
