@@ -13,6 +13,7 @@
 
 #include <stdlib.h>
 
+#include <algorithm>
 #include <type_traits>
 
 #include "common.cuh"
@@ -800,16 +801,8 @@ int run_level_hysteresis(const unsigned char *cl, unsigned char *E, int N, int H
     P.prof = debug_knob("MTE_HYST_PROF") ? reinterpret_cast<unsigned long long *>(w + hysteresis_scratch_bytes(N, H, W) - 256) : nullptr;
     // shared-memory kernel first: bitmaps next to the per-candidate state when they leave room for a useful number of
     // candidates, otherwise (BIG) bitmaps in the image's global scratch and only the per-candidate state resident
-    int budget;
-    {
-        cudaFuncAttributes fa;
-        cudaFuncGetAttributes(&fa, canny_uf_hyst_smem_kernel<false>);
-        budget = dev_info().smemOptin - (int)fa.sharedSizeBytes - 1024;
-        if (budget > 0 && (opt_in_smem((const void *)canny_uf_hyst_smem_kernel<false>, budget) != cudaSuccess ||
-                           opt_in_smem((const void *)canny_uf_hyst_smem_kernel<true>, budget) != cudaSuccess))
-            budget = 0;
-        cudaGetLastError();
-    }
+    const int budget =
+        std::min(smem_budget(canny_uf_hyst_smem_kernel<false>), smem_budget(canny_uf_hyst_smem_kernel<true>));
     const long long nW = (long long)H * ((W + 31) / 32), nW2 = (nW + 1) / 2;  // bitmap rows padded to whole words
     // [reachable-set bitmap][rank][region X][flood worklists]; region X is the candidate bitmap during the flood,
     // then parent (2 B) + edge level (1 B) + flag (1 bit) + rank -> id (2 B) per pixel of the reachable set.  BIG:

@@ -69,6 +69,18 @@ inline cudaError_t opt_in_smem(const void *func, int bytes) {
     return r;
 }
 
+// Dynamic shared memory a kernel can use on the current device: the opt-in limit less its static shared memory and
+// 1 KB, opted in; 0 if nothing is left or the opt-in fails.
+template <typename Kernel>
+inline int smem_budget(Kernel *kernel) {
+    cudaFuncAttributes fa;
+    cudaFuncGetAttributes(&fa, kernel);
+    int budget = dev_info().smemOptin - (int)fa.sharedSizeBytes - 1024;
+    if (budget <= 0 || opt_in_smem((const void *)kernel, budget) != cudaSuccess) budget = 0;
+    cudaGetLastError();
+    return budget;
+}
+
 // Tuning / diagnostic switches exist ONLY in builds made with -DMTE_DEBUG_KNOBS (scripts/ use them through
 // MTE_NVCC_DEFS); the release library never reads the environment, so no call's result or algorithm can depend on
 // process-global state.

@@ -11,10 +11,9 @@
 // One persistent CTA per (image, threshold) problem, problems handed out through an atomic counter:
 //   scan   the cropped window once (the 2 B/px of algorithmic traffic), compact predicted pixels,
 //   greedy nearest-first proposals with 16-bit CAS on the GT side,
-//   then phases of { alternating-forest BFS from all free predicted pixels, level-synchronous with
-//   warp-per-vertex expansion, stopped at the first level that reaches a free GT pixel; one
-//   vertex-disjoint augmenting path per tree, claimed with CAS }
-//   until an (exhaustive) phase finds no free GT pixel => no augmenting path exists => maximum.
+//   then phases of { exhaustive alternating-forest BFS from all free predicted pixels, level-synchronous
+//   with warp-per-vertex expansion; one vertex-disjoint augmenting path per tree, claimed with CAS }
+//   until a phase finds no free GT pixel => no augmenting path exists => maximum.
 // Per-pixel state is 16-bit offset codes in an L2-resident per-CTA arena; nothing is allocated.
 // With apply_thinning = 1 every problem's window is thinned first (thin_window_kernel below) and the per-problem
 // matchers read the thinned bit planes.
@@ -34,7 +33,6 @@ constexpr int kThreads = 256;
 constexpr int kWarps = kThreads / 32;
 constexpr unsigned short kFree = 0xFFFF;
 constexpr unsigned short kDead = 0xFFFE;  // predicted pixel without any GT pixel in range
-constexpr int kMaxOffsets = 0xFFF0;
 constexpr int kCtasPerSm = 2;
 
 enum { IN_LEVELS = 0, IN_BINARY = 1, IN_F32 = 2, IN_F64 = 3, IN_BITS = 4 };
@@ -64,7 +62,6 @@ struct MatchP {
     const unsigned int *listCount;  // device count of problemList entries
     unsigned int *overflowCount;    // written by the shared-memory kernel, reset by the dense kernel
     int *overflowList;
-    int truncate;              // stop each BFS at the first level that reaches a free GT pixel
     unsigned int *stats;       // optional profiling counters {phases, levels, expanded vertices, free roots}
     unsigned int *trace;       // debug builds: per-item cycle stamps of the many-root phases of stage 0 (scripts/match_trace.py)
     unsigned int *nextProblem; // dynamic scheduler (self-resetting)
@@ -73,8 +70,8 @@ struct MatchP {
 
 // Small tables ride in the kernel parameters (graph-capturable, no staging copy); larger ones (radius > 7 px
 // or > kParamThr thresholds) are copied into the workspace first.  Either way the CTA stages the offsets in
-// shared memory: lanes index them divergently.
-constexpr int kParamOff = 256, kParamThr = 160, kSmemOff = 4096;
+// shared memory: lanes index them divergently.  kMaxOff holds the largest table build_offsets makes.
+constexpr int kParamOff = 256, kParamThr = 160, kMaxOff = 4096;
 struct ParamTables {
     short2 off[kParamOff];
     unsigned short neg[kParamOff];
@@ -134,40 +131,151 @@ __device__ __forceinline__ bool is_pred(const MatchP &P, int img, int t, int pro
     }
 }
 
+// ---- pieces the three matcher kernels share (NT: the kernel's threads per CTA)
+
+// stage the offsets (and the inverse-offset indices where sNeg is given, the thresholds where withThr) in shared memory
+template <int NT>
+__device__ __forceinline__ void stage_tables(const MatchP &P, const ParamTables &tabs, int tablesInParam, bool withThr,
+                                             short2 *sOff, unsigned short *sNeg, double *sThr) {
+    for (int i = threadIdx.x; i < P.noff; i += NT) {
+        sOff[i] = tablesInParam ? tabs.off[i] : P.off[i];
+        if (sNeg) sNeg[i] = tablesInParam ? tabs.neg[i] : P.neg[i];
+    }
+    if (withThr)
+        for (int i = threadIdx.x; i < P.T; i += NT) sThr[i] = tablesInParam ? tabs.thr[i] : P.thr[i];
+    __syncthreads();
+}
+
+// thread 0 draws the next ticket of the dynamic scheduler, all threads return it; through the problem list when
+// viaList (a ticket past the list's end returns P.nProblems: nothing left)
+__device__ __forceinline__ int next_ticket(const MatchP &P, bool viaList, int &sTicket) {
+    if (threadIdx.x == 0) {
+        int pr = (int)atomicAdd(P.nextProblem, 1u);
+        if (viaList) pr = (pr < (int)*P.listCount) ? P.problemList[pr] : P.nProblems;
+        sTicket = pr;
+    }
+    __syncthreads();
+    return sTicket;
+}
+
+// problems are ordered image-major so consecutive CTAs share the GT plane in L2
+__device__ __forceinline__ void decode_problem(const MatchP &P, int prob, int &img, int &t) {
+    const int g = P.probBase + prob;
+    img = (P.inMode == IN_BINARY) ? prob : g / P.T;
+    t = (P.inMode == IN_BINARY) ? 0 : g - img * P.T;
+}
+
+// warp-aggregated append to a shared counter: one atomic per warp; returns this lane's slot (valid where take)
+__device__ __forceinline__ int warp_append(int *counter, bool take) {
+    const int lane = threadIdx.x & 31;
+    const unsigned m = __ballot_sync(MTE_FULL_MASK, take);
+    int wbase = 0;
+    if (lane == 0 && m) wbase = atomicAdd(counter, __popc(m));
+    wbase = __shfl_sync(MTE_FULL_MASK, wbase, 0);
+    return wbase + __popc(m & ((1u << lane) - 1));
+}
+
+// exclusive prefix sum of one value per thread over the CTA (warp 0 scans the NT partials, NT / 32 per lane)
+template <int NT>
+__device__ __forceinline__ int block_exclusive_scan(int v, int *sScan) {
+    const int lane = threadIdx.x & 31;
+    sScan[threadIdx.x] = v;
+    __syncthreads();
+    if (threadIdx.x < 32) {
+        int loc[NT / 32], run = 0;
+#pragma unroll
+        for (int k = 0; k < NT / 32; k++) { loc[k] = run; run += sScan[lane * (NT / 32) + k]; }
+        int incl = run;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) { const int u = __shfl_up_sync(MTE_FULL_MASK, incl, o); if (lane >= o) incl += u; }
+        const int excl = incl - run;
+#pragma unroll
+        for (int k = 0; k < NT / 32; k++) sScan[lane * (NT / 32) + k] = excl + loc[k];
+    }
+    __syncthreads();
+    return sScan[threadIdx.x];
+}
+
+// Lane 0 takes the next entry of the shared work queue fa[sHead, sTail) and waits until it is published (slots hold
+// kFree until then); -2 once the queue is drained and no vertex is pending (one being expanded may still publish).
+// All lanes return the predicted vertex.
+__device__ __forceinline__ int queue_pop(int *sHead, const int *sTail, const int *sPending, const unsigned short *fa) {
+    int my = -1;
+    if ((threadIdx.x & 31) == 0) {
+        for (;;) {
+            const int hd = *(volatile int *)sHead, tl = *(volatile const int *)sTail;
+            if (hd < tl) {
+                if (atomicCAS(sHead, hd, hd + 1) == hd) { my = hd; break; }
+            } else if (*(volatile const int *)sPending == 0) {
+                my = -2;
+                break;
+            }
+        }
+        if (my >= 0) {
+            int v;
+            while ((v = ((volatile const unsigned short *)fa)[my]) == kFree) {}
+            my = v;
+        }
+    }
+    return __shfl_sync(MTE_FULL_MASK, my, 0);
+}
+
+// flip the augmenting path that ends at free GT vertex q, in compact ids (parentQ: predicted id, mateP: GT id)
+__device__ __forceinline__ void flip_path(int q, const unsigned short *parentQ, unsigned short *mateP,
+                                          unsigned short *mateQ) {
+    for (;;) {
+        const int pi = parentQ[q];
+        const unsigned short prev = mateP[pi];
+        mateP[pi] = (unsigned short)q;
+        mateQ[q] = (unsigned short)pi;
+        if (prev == kFree) break;
+        q = prev;
+    }
+}
+
+// add one problem's count_r, sum_r, count_p, sum_p to its row of P.counts
+__device__ __forceinline__ void add_counts(const MatchP &P, int img, int t, int matched, int nQ, int nP) {
+    unsigned long long *c = P.counts + (size_t)(t + img * P.countsImgStride) * 4;
+    atomicAdd(c + 0, (unsigned long long)matched);
+    atomicAdd(c + 1, (unsigned long long)nQ);
+    atomicAdd(c + 2, (unsigned long long)matched);
+    atomicAdd(c + 3, (unsigned long long)nP);
+}
+
+// last CTA out resets the scheduler so the workspace header is clean for the next launch; the launch over the
+// overflow list also clears the count of that list
+__device__ __forceinline__ void reset_scheduler(const MatchP &P, bool clearOverflow) {
+    if (threadIdx.x == 0) {
+        __threadfence();
+        const unsigned d = atomicAdd(P.doneCtas, 1u);
+        if (d == gridDim.x - 1) {
+            *P.nextProblem = 0u;
+            *P.doneCtas = 0u;
+            if (clearOverflow) *P.overflowCount = 0u;
+        }
+    }
+}
+
 __global__ void __launch_bounds__(kThreads) match_kernel(const __grid_constant__ MatchP Pin,
                                                          const __grid_constant__ ParamTables tabs, int tablesInParam) {
     __shared__ int sProblem, sNP, sNQ, sCntA, sCntB, sEnds, sMatched;
-    __shared__ short2 sOff[kSmemOff];
-    __shared__ unsigned short sNeg[kSmemOff];
+    __shared__ short2 sOff[kMaxOff];
+    __shared__ unsigned short sNeg[kMaxOff];
     __shared__ double sThr[MTE_MAX_THRESHOLDS];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     MatchP P = Pin;
     const int w = P.w, h = P.h;
     const Arena A = carve(P.arena + (size_t)blockIdx.x * P.arenaBytes, h, w);
-    for (int i = threadIdx.x; i < P.noff; i += kThreads) {
-        sOff[i] = tablesInParam ? tabs.off[i] : P.off[i];
-        sNeg[i] = tablesInParam ? tabs.neg[i] : P.neg[i];
-    }
-    if (P.inMode == IN_F32 || P.inMode == IN_F64)
-        for (int i = threadIdx.x; i < P.T; i += kThreads) sThr[i] = tablesInParam ? tabs.thr[i] : P.thr[i];
+    stage_tables<kThreads>(P, tabs, tablesInParam, P.inMode == IN_F32 || P.inMode == IN_F64, sOff, sNeg, sThr);
     P.off = sOff;
     P.neg = sNeg;
     P.thr = sThr;
-    __syncthreads();
 
     for (;;) {
-        if (threadIdx.x == 0) {
-            int pr = (int)atomicAdd(P.nextProblem, 1u);
-            if (P.problemList) pr = (pr < (int)*P.listCount) ? P.problemList[pr] : P.nProblems;
-            sProblem = pr;
-        }
-        __syncthreads();
-        const int prob = sProblem;
+        const int prob = next_ticket(P, P.problemList != nullptr, sProblem);
         if (prob >= P.nProblems) break;
-        // problems are ordered image-major so consecutive CTAs share the GT plane in L2
-        const int g = P.probBase + prob;
-        const int img = (P.inMode == IN_BINARY) ? prob : g / P.T;
-        const int t = (P.inMode == IN_BINARY) ? 0 : g - img * P.T;
+        int img, t;
+        decode_problem(P, prob, img, t);
         const unsigned char *gt = P.gt + (size_t)img * P.H * P.W;
         if (threadIdx.x == 0) { sNP = 0; sNQ = 0; sMatched = 0; }
         __syncthreads();
@@ -188,11 +296,8 @@ __global__ void __launch_bounds__(kThreads) match_kernel(const __grid_constant__
                 }
                 if (isP) { A.mateP[i] = kFree; A.claimP[i] = 0; }
             }
-            const unsigned m = __ballot_sync(MTE_FULL_MASK, isP);
-            int wbase = 0;
-            if (lane == 0 && m) wbase = atomicAdd(&sNP, __popc(m));
-            wbase = __shfl_sync(MTE_FULL_MASK, wbase, 0);
-            if (isP) A.plist[wbase + __popc(m & ((1u << lane) - 1))] = i;
+            const int slot = warp_append(&sNP, isP);
+            if (isP) A.plist[slot] = i;
         }
         myQ = __reduce_add_sync(MTE_FULL_MASK, myQ);
         if (lane == 0 && myQ) atomicAdd(&sNQ, myQ);
@@ -244,11 +349,8 @@ __global__ void __launch_bounds__(kThreads) match_kernel(const __grid_constant__
                 bool fr = false;
                 int p = 0;
                 if (pi < nP) { p = A.plist[pi]; fr = A.mateP[p] == kFree; }
-                const unsigned m = __ballot_sync(MTE_FULL_MASK, fr);
-                int wbase = 0;
-                if (lane == 0 && m) wbase = atomicAdd(&sCntA, __popc(m));
-                wbase = __shfl_sync(MTE_FULL_MASK, wbase, 0);
-                if (fr) A.fa[wbase + __popc(m & ((1u << lane) - 1))] = p;
+                const int slot = warp_append(&sCntA, fr);
+                if (fr) A.fa[slot] = p;
             }
             __syncthreads();
             int *cur = A.fa, *nxt = A.fb;
@@ -284,9 +386,7 @@ __global__ void __launch_bounds__(kThreads) match_kernel(const __grid_constant__
                     }
                 }
                 __syncthreads();
-                // shortest augmenting paths first (Hopcroft-Karp layering): stop at the first level that reaches a
-                // free GT pixel; only the last phase, which finds none, explores the forest exhaustively
-                nCur = (P.truncate && sEnds > 0) ? 0 : sCntB;
+                nCur = sCntB;
                 if (P.stats && threadIdx.x == 0) { atomicAdd(P.stats + 1, 1u); atomicAdd(P.stats + 2, (unsigned)sCntB); }
                 int *tmp = cur; cur = nxt; nxt = tmp;
                 __syncthreads();
@@ -335,13 +435,7 @@ __global__ void __launch_bounds__(kThreads) match_kernel(const __grid_constant__
         // ---- results
         const int matched = sMatched;
         if (threadIdx.x == 0) {
-            if (P.counts) {
-                unsigned long long *c = P.counts + (size_t)(t + img * P.countsImgStride) * 4;
-                atomicAdd(c + 0, (unsigned long long)matched);
-                atomicAdd(c + 1, (unsigned long long)nQ);
-                atomicAdd(c + 2, (unsigned long long)matched);
-                atomicAdd(c + 3, (unsigned long long)nP);
-            }
+            if (P.counts) add_counts(P, img, t, matched, nQ, nP);
             if (P.countPerProblem) P.countPerProblem[prob] = matched;
         }
         if (P.matchA || P.matchB) {
@@ -360,16 +454,7 @@ __global__ void __launch_bounds__(kThreads) match_kernel(const __grid_constant__
         }
         __syncthreads();
     }
-    // last CTA out resets the scheduler so the workspace header is clean for the next launch
-    if (threadIdx.x == 0) {
-        __threadfence();
-        const unsigned d = atomicAdd(P.doneCtas, 1u);
-        if (d == gridDim.x - 1) {
-            *P.nextProblem = 0u;
-            *P.doneCtas = 0u;
-            if (P.problemList) *P.overflowCount = 0u;
-        }
-    }
+    reset_scheduler(P, P.problemList != nullptr);
 }
 
 // ---------------------------------------------------------------------------
@@ -408,16 +493,12 @@ __global__ void __launch_bounds__(kSmThreads, 1) match_smem_kernel(const __grid_
     unsigned short *mateP = reinterpret_cast<unsigned short *>(dyn + SL.oMateP);
     unsigned short *claimP = reinterpret_cast<unsigned short *>(dyn + SL.oClaimP);
     unsigned short *fa = reinterpret_cast<unsigned short *>(dyn + SL.oFa);
-    unsigned short *fb = reinterpret_cast<unsigned short *>(dyn + SL.oFb);
     unsigned short *mateQ = reinterpret_cast<unsigned short *>(dyn + SL.oMateQ);
     unsigned short *parentQ = reinterpret_cast<unsigned short *>(dyn + SL.oParentQ);
     unsigned short *stampQ = reinterpret_cast<unsigned short *>(dyn + SL.oStampQ);
     unsigned short *ends = reinterpret_cast<unsigned short *>(dyn + SL.oEnds);
-    for (int i = threadIdx.x; i < P.noff; i += kSmThreads) sOff[i] = tablesInParam ? tabs.off[i] : P.off[i];
-    if (P.inMode == IN_F32 || P.inMode == IN_F64)
-        for (int i = threadIdx.x; i < P.T; i += kSmThreads) sThr[i] = tablesInParam ? tabs.thr[i] : P.thr[i];
+    stage_tables<kSmThreads>(P, tabs, tablesInParam, P.inMode == IN_F32 || P.inMode == IN_F64, sOff, nullptr, sThr);
     P.thr = sThr;
-    __syncthreads();
     const int noff = P.noff;
 
     // GT vertex id of window pixel q (caller has checked the bit)
@@ -427,13 +508,10 @@ __global__ void __launch_bounds__(kSmThreads, 1) match_smem_kernel(const __grid_
     };
 
     for (;;) {
-        if (threadIdx.x == 0) sProblem = (int)atomicAdd(P.nextProblem, 1u);
-        __syncthreads();
-        const int prob = sProblem;
+        const int prob = next_ticket(P, false, sProblem);
         if (prob >= P.nProblems) break;
-        const int g = P.probBase + prob;
-        const int img = (P.inMode == IN_BINARY) ? prob : g / P.T;
-        const int t = (P.inMode == IN_BINARY) ? 0 : g - img * P.T;
+        int img, t;
+        decode_problem(P, prob, img, t);
         const unsigned char *gt = P.gt + (size_t)img * P.H * P.W;
         if (threadIdx.x == 0) { sNP = 0; sNQ = 0; sMatched = 0; }
         __syncthreads();
@@ -458,18 +536,12 @@ __global__ void __launch_bounds__(kSmThreads, 1) match_smem_kernel(const __grid_
                 const int i = base + u * kSmThreads + threadIdx.x;
                 if (base + u * kSmThreads >= SL.nW * 32) break;  // warp-uniform
                 const unsigned mq = __ballot_sync(MTE_FULL_MASK, isQk[u]);
-                const unsigned mp = __ballot_sync(MTE_FULL_MASK, isPk[u]);
-                int wbase = 0;
                 if (lane == 0) {
                     qbits[i >> 5] = mq;
                     if (mq) atomicAdd(&sNQ, __popc(mq));
-                    if (mp) wbase = atomicAdd(&sNP, __popc(mp));
                 }
-                wbase = __shfl_sync(MTE_FULL_MASK, wbase, 0);
-                if (isPk[u]) {
-                    const int slot = wbase + __popc(mp & ((1u << lane) - 1));
-                    if (slot < SL.capP) { ppix[slot] = (unsigned)i; mateP[slot] = kFree; claimP[slot] = 0; }
-                }
+                const int slot = warp_append(&sNP, isPk[u]);
+                if (isPk[u] && slot < SL.capP) { ppix[slot] = (unsigned)i; mateP[slot] = kFree; claimP[slot] = 0; }
             }
         }
         __syncthreads();
@@ -485,21 +557,7 @@ __global__ void __launch_bounds__(kSmThreads, 1) match_smem_kernel(const __grid_
             const int w0 = threadIdx.x * per, w1 = min(w0 + per, SL.nW);
             int sum = 0;
             for (int k = w0; k < w1; k++) sum += __popc(qbits[k]);
-            sScan[threadIdx.x] = sum;
-            __syncthreads();
-            if (warp == 0) {  // 512 partials: 16 per lane
-                int loc[kSmThreads / 32], run = 0;
-#pragma unroll
-                for (int k = 0; k < kSmThreads / 32; k++) { loc[k] = run; run += sScan[lane * (kSmThreads / 32) + k]; }
-                int incl = run;
-#pragma unroll
-                for (int o = 1; o < 32; o <<= 1) { const int v = __shfl_up_sync(MTE_FULL_MASK, incl, o); if (lane >= o) incl += v; }
-                const int excl = incl - run;
-#pragma unroll
-                for (int k = 0; k < kSmThreads / 32; k++) sScan[lane * (kSmThreads / 32) + k] = excl + loc[k];
-            }
-            __syncthreads();
-            int run = sScan[threadIdx.x];
+            int run = block_exclusive_scan<kSmThreads>(sum, sScan);
             for (int k = w0; k < w1; k++) { qrank[k] = (unsigned short)run; run += __popc(qbits[k]); }
         }
         for (int k = threadIdx.x; k < nQ; k += kSmThreads) { mateQ[k] = kFree; stampQ[k] = 0; }
@@ -548,11 +606,8 @@ __global__ void __launch_bounds__(kSmThreads, 1) match_smem_kernel(const __grid_
             for (int base = 0; base < nP; base += kSmThreads) {
                 const int pi = base + threadIdx.x;
                 const bool fr = pi < nP && mateP[pi] == kFree;
-                const unsigned m = __ballot_sync(MTE_FULL_MASK, fr);
-                int wbase = 0;
-                if (lane == 0 && m) wbase = atomicAdd(&sCntA, __popc(m));
-                wbase = __shfl_sync(MTE_FULL_MASK, wbase, 0);
-                if (fr) fa[wbase + __popc(m & ((1u << lane) - 1))] = (unsigned short)pi;
+                const int slot = warp_append(&sCntA, fr);
+                if (fr) fa[slot] = (unsigned short)pi;
             }
             __syncthreads();
             const int nRoots = sCntA;
@@ -566,26 +621,8 @@ __global__ void __launch_bounds__(kSmThreads, 1) match_smem_kernel(const __grid_
             if (threadIdx.x == 0) { sHead = 0; sTail = nRoots; sPending = nRoots; }
             __syncthreads();
             for (;;) {
-                int my = -1;
-                if (lane == 0) {
-                    for (;;) {
-                        const int hd = *(volatile int *)&sHead, tl = *(volatile int *)&sTail;
-                        if (hd < tl) {
-                            if (atomicCAS(&sHead, hd, hd + 1) == hd) { my = hd; break; }
-                        } else if (*(volatile int *)&sPending == 0) {
-                            my = -2;
-                            break;
-                        }
-                    }
-                    if (my >= 0) {
-                        int v;
-                        while ((v = ((volatile unsigned short *)fa)[my]) == kFree) {}
-                        my = v;
-                    }
-                }
-                my = __shfl_sync(MTE_FULL_MASK, my, 0);
-                if (my == -2) break;
-                const int pi = my;
+                const int pi = queue_pop(&sHead, &sTail, &sPending, fa);
+                if (pi == -2) break;
                 const int p = (int)ppix[pi];
                 const int py = p / w, px = p - py * w;
                 for (int k = lane; k < noff; k += 32) {
@@ -631,15 +668,7 @@ __global__ void __launch_bounds__(kSmThreads, 1) match_smem_kernel(const __grid_
                     q = mp;
                 }
                 if (!ok) continue;
-                q = qEnd;
-                for (;;) {  // flip walk
-                    const int pi = parentQ[q];
-                    const unsigned short prev = mateP[pi];
-                    mateP[pi] = (unsigned short)q;
-                    mateQ[q] = (unsigned short)pi;
-                    if (prev == kFree) break;
-                    q = prev;
-                }
+                flip_path(qEnd, parentQ, mateP, mateQ);
                 atomicAdd(&sMatched, 1);
             }
             __syncthreads();
@@ -650,13 +679,7 @@ __global__ void __launch_bounds__(kSmThreads, 1) match_smem_kernel(const __grid_
         // ---- results
         const int matched = sMatched;
         if (threadIdx.x == 0) {
-            if (P.counts) {
-                unsigned long long *c = P.counts + (size_t)(t + img * P.countsImgStride) * 4;
-                atomicAdd(c + 0, (unsigned long long)matched);
-                atomicAdd(c + 1, (unsigned long long)nQ);
-                atomicAdd(c + 2, (unsigned long long)matched);
-                atomicAdd(c + 3, (unsigned long long)nP);
-            }
+            if (P.counts) add_counts(P, img, t, matched, nQ, nP);
             if (P.countPerProblem) P.countPerProblem[prob] = matched;
         }
         if (P.matchA) {
@@ -674,14 +697,7 @@ __global__ void __launch_bounds__(kSmThreads, 1) match_smem_kernel(const __grid_
         }
         __syncthreads();
     }
-    if (threadIdx.x == 0) {
-        __threadfence();
-        const unsigned d = atomicAdd(P.doneCtas, 1u);
-        if (d == gridDim.x - 1) {
-            *P.nextProblem = 0u;
-            *P.doneCtas = 0u;
-        }
-    }
+    reset_scheduler(P, false);
 }
 
 // ---------------------------------------------------------------------------
@@ -703,11 +719,7 @@ __global__ void __launch_bounds__(kSmThreads, 1) match_smem_kernel(const __grid_
 constexpr unsigned kDeadStamp = 0xFFFFFFFFu;   // GT stamp word: phase << 16 | root (predicted vertex id of the tree)
 constexpr unsigned short kFailed = 0xFFFD;     // predicted pixel whose search failed conclusively (Kuhn: for good)
 enum { RF_FOUND = 1u, RF_CLASS_FOUND = 2u };
-#ifndef MTE_SWEEP_THREADS
-#define MTE_SWEEP_THREADS 512
-#endif
-
-constexpr int kSwThreads = MTE_SWEEP_THREADS, kSwWarps = kSwThreads / 32;
+constexpr int kSwThreads = 512, kSwWarps = kSwThreads / 32;
 constexpr int kEndsCap = 2048;  // free GT pixels recorded per phase (further ones wait for the next phase)
 
 struct SweepLayout {
@@ -745,11 +757,8 @@ __global__ void __launch_bounds__(kSwThreads, 1) match_sweep_kernel(const __grid
     unsigned short *rootP = reinterpret_cast<unsigned short *>(dyn + SL.oRootP);
     unsigned *rflagW = reinterpret_cast<unsigned *>(dyn + SL.oRflag);  // one flag byte per predicted vertex
     unsigned short *ends = reinterpret_cast<unsigned short *>(dyn + SL.oEnds);
-    for (int i = threadIdx.x; i < P.noff; i += kSwThreads) sOff[i] = tablesInParam ? tabs.off[i] : P.off[i];
     const bool levels = P.inMode == IN_LEVELS;
-    if (!levels)
-        for (int i = threadIdx.x; i < T; i += kSwThreads) sThr[i] = tablesInParam ? tabs.thr[i] : P.thr[i];
-    __syncthreads();
+    stage_tables<kSwThreads>(P, tabs, tablesInParam, !levels, sOff, nullptr, sThr);
     const int noff = P.noff;
 #ifdef MTE_DEBUG_KNOBS
     const long long tZero = clock64();
@@ -824,9 +833,7 @@ __global__ void __launch_bounds__(kSwThreads, 1) match_sweep_kernel(const __grid
     const short2 off0 = sOff[min(lane, noff - 1)];  // lane's own entry of the first 32 offsets (all of them at KITTI radius)
 
     for (;;) {
-        if (threadIdx.x == 0) sImage = (int)atomicAdd(P.nextProblem, 1u);
-        __syncthreads();
-        const int img = sImage;
+        const int img = next_ticket(P, false, sImage);
         if (img >= P.N) break;
         const unsigned char *gt = P.gt + (size_t)img * P.H * P.W;
         if (threadIdx.x == 0) { sNQ = 0; sMatched = 0; }
@@ -861,10 +868,7 @@ __global__ void __launch_bounds__(kSwThreads, 1) match_sweep_kernel(const __grid
             const int nChunks = cpr * h;
             // kScanU independent word pairs per thread in flight: the scan is one CTA streaming 0.5 MB, i.e. latency-
             // bound (4 in flight: 31 round trips for the KITTI crop, 80 us of every image's critical path)
-#ifndef MTE_SCAN_U
-#define MTE_SCAN_U 12
-#endif
-            constexpr int kScanU = MTE_SCAN_U;
+            constexpr int kScanU = 12;
             for (int base = 0; base < nChunks; base += kScanU * kSwThreads) {
                 unsigned lw[kScanU], gw[kScanU];
 #pragma unroll
@@ -981,21 +985,7 @@ __global__ void __launch_bounds__(kSwThreads, 1) match_sweep_kernel(const __grid
             auto pc2 = [&](int k2) { return __popc(qbits[2 * k2]) + (2 * k2 + 1 < SL.nW ? __popc(qbits[2 * k2 + 1]) : 0); };
             int sum = 0;
             for (int k2 = w0; k2 < w1; k2++) sum += pc2(k2);
-            sScan[threadIdx.x] = sum;
-            __syncthreads();
-            if (warp == 0) {
-                int loc[kSwThreads / 32], run = 0;
-#pragma unroll
-                for (int q = 0; q < kSwThreads / 32; q++) { loc[q] = run; run += sScan[lane * (kSwThreads / 32) + q]; }
-                int incl = run;
-#pragma unroll
-                for (int o = 1; o < 32; o <<= 1) { const int v = __shfl_up_sync(MTE_FULL_MASK, incl, o); if (lane >= o) incl += v; }
-                const int excl = incl - run;
-#pragma unroll
-                for (int q = 0; q < kSwThreads / 32; q++) sScan[lane * (kSwThreads / 32) + q] = excl + loc[q];
-            }
-            __syncthreads();
-            int run = sScan[threadIdx.x];
+            int run = block_exclusive_scan<kSwThreads>(sum, sScan);
             for (int k2 = w0; k2 < w1; k2++) { qrank[k2] = (unsigned short)run; run += pc2(k2); }
         }
         for (int k = threadIdx.x; k < nQ; k += kSwThreads) { mateQ[k] = kFree; stamp[k] = 0u; }
@@ -1084,12 +1074,9 @@ __global__ void __launch_bounds__(kSwThreads, 1) match_sweep_kernel(const __grid
                     for (int base = p0; base < p1; base += kSwThreads) {
                         const int pi = base + threadIdx.x;
                         const bool fr = pi < p1 && mateP[pi] == kFree;
-                        const unsigned m = __ballot_sync(MTE_FULL_MASK, fr);
-                        int wbase = 0;
-                        if (lane == 0 && m) wbase = atomicAdd(&sCntA, __popc(m));
-                        wbase = __shfl_sync(MTE_FULL_MASK, wbase, 0);
+                        const int slot = warp_append(&sCntA, fr);
                         if (fr) {
-                            fa[wbase + __popc(m & ((1u << lane) - 1))] = (unsigned short)pi;
+                            fa[slot] = (unsigned short)pi;
                             rootP[pi] = (unsigned short)pi;
                             classP[pi] = (unsigned short)pi;
                         }
@@ -1111,27 +1098,10 @@ __global__ void __launch_bounds__(kSwThreads, 1) match_sweep_kernel(const __grid
                     __syncthreads();
                     tick(6);
                     for (;;) {
-                        int my = -1;
 #ifdef MTE_DEBUG_KNOBS
                         const long long tWait = (P.trace && lane == 0) ? clock64() : 0;
 #endif
-                        if (lane == 0) {
-                            for (;;) {
-                                const int hd = *(volatile int *)&sHead, tl = *(volatile int *)&sTail;
-                                if (hd < tl) {
-                                    if (atomicCAS(&sHead, hd, hd + 1) == hd) { my = hd; break; }
-                                } else if (*(volatile int *)&sPending == 0) {
-                                    my = -2;
-                                    break;
-                                }
-                            }
-                            if (my >= 0) {
-                                int v;
-                                while ((v = ((volatile unsigned short *)fa)[my]) == kFree) {}
-                                my = v;
-                            }
-                        }
-                        my = __shfl_sync(MTE_FULL_MASK, my, 0);
+                        const int my = queue_pop(&sHead, &sTail, &sPending, fa);
                         if (my == -2) break;
 #ifdef MTE_DEBUG_KNOBS   // profiling: queue items (roots + published successors)
                         if (P.stats && lane == 0) atomicAdd(P.stats + 22, 1u);
@@ -1288,15 +1258,7 @@ __global__ void __launch_bounds__(kSwThreads, 1) match_sweep_kernel(const __grid
                     __syncthreads();
                     if (nEnds == 0) { tick(8); break; }
                     for (int ei = threadIdx.x; ei < nEnds; ei += kSwThreads) {
-                        int q = ends[ei];
-                        for (;;) {  // flip walk (one path per tree, see above)
-                            const int pi = parentQ[q];
-                            const unsigned short prev = mateP[pi];
-                            mateP[pi] = (unsigned short)q;
-                            mateQ[q] = (unsigned short)pi;
-                            if (prev == kFree) break;
-                            q = prev;
-                        }
+                        flip_path(ends[ei], parentQ, mateP, mateQ);  // one path per tree, see above
                         atomicAdd(&sMatched, 1);
                     }
                     __syncthreads();
@@ -1337,27 +1299,12 @@ __global__ void __launch_bounds__(kSwThreads, 1) match_sweep_kernel(const __grid
                 atomicAdd(P.stats + 9 + min(s, 11), (unsigned)((clock64() - tStage) >> 8));
                 if (s == 0) atomicAdd(P.stats + 21, (unsigned)(G1 - G0));
             }
-            if (threadIdx.x == 0) {
-                const int t = levels ? s : T - 1 - s;
-                const int matched = sMatched;
-                // per-image rows: the image this CTA is sweeping (thread 0 wrote sImage)
-                unsigned long long *c = P.counts + (size_t)(t + sImage * P.countsImgStride) * 4;
-                atomicAdd(c + 0, (unsigned long long)matched);
-                atomicAdd(c + 1, (unsigned long long)nQ);
-                atomicAdd(c + 2, (unsigned long long)matched);
-                atomicAdd(c + 3, (unsigned long long)G1);
-            }
+            // per-image rows: the image this CTA is sweeping (thread 0 wrote sImage)
+            if (threadIdx.x == 0) add_counts(P, sImage, levels ? s : T - 1 - s, sMatched, nQ, G1);
         }
         __syncthreads();
     }
-    if (threadIdx.x == 0) {
-        __threadfence();
-        const unsigned d = atomicAdd(P.doneCtas, 1u);
-        if (d == gridDim.x - 1) {
-            *P.nextProblem = 0u;
-            *P.doneCtas = 0u;
-        }
-    }
+    reset_scheduler(P, false);
 }
 
 // ---------------------------------------------------------------------------
@@ -1409,8 +1356,8 @@ __global__ void __launch_bounds__(thin::kThreads) thin_window_kernel(const __gri
 // ---------------------------------------------------------------------------
 struct OffsetTable {
     int n;
-    short2 off[4096];
-    unsigned short neg[4096];
+    short2 off[kMaxOff];
+    unsigned short neg[kMaxOff];
 };
 
 static int build_offsets(double radius, OffsetTable &tb) {
@@ -1437,66 +1384,71 @@ struct Layout {
     int nArenas;
 };
 
-// carve the dynamic shared memory of match_smem_kernel for a w x h window; capP = capQ = 0 if it cannot fit
+// The dynamic shared memory of the resident matchers, for a w x h window (nW bitmap words).  vertex_cap: the
+// capacity, equal for both sides, that the budget leaves after the fixed bytes at perVertex bytes per predicted + GT
+// vertex; 0 (the kernel is not used) below 512.  Carve hands out 16 B aligned regions one after another.
+static int vertex_cap(int budget, long long fixed, int perVertex) {
+    const long long cap = (budget - fixed) / perVertex;
+    return cap < 512 ? 0 : (int)(cap > 0xFFF0 ? 0xFFF0 : cap) & ~7;
+}
+struct Carve {
+    unsigned o = 0;
+    unsigned take(unsigned bytes) { const unsigned r = o; o += (bytes + 15u) & ~15u; return r; }
+};
+
+// capP = capQ = 0 if the window cannot fit
 static SmemLayout smem_layout(int h, int w, int budget) {
     SmemLayout S;
     memset(&S, 0, sizeof(S));
-    const long long hw = (long long)h * w;
-    S.nW = (int)((hw + 31) / 32);
-    const long long fixed = (long long)S.nW * 4 + (((long long)S.nW * 2 + 15) / 16) * 16 + 256;
-    const long long cap = (budget - fixed) / 20;  // 12 B per predicted vertex + 8 B per GT vertex, equal capacities
-    if (cap < 512) return S;
-    S.capP = S.capQ = (int)(cap > 0xFFF0 ? 0xFFF0 : cap) & ~7;
-    unsigned o = 0;
-    auto take = [&](unsigned bytes) { const unsigned r = o; o += (bytes + 15u) & ~15u; return r; };
-    S.oBits = take(S.nW * 4);
-    S.oRank = take(S.nW * 2);
-    S.oPpix = take(S.capP * 4);
-    S.oMateP = take(S.capP * 2);
-    S.oClaimP = take(S.capP * 2);
-    S.oFa = take(S.capP * 2);
-    S.oFb = take(S.capP * 2);
-    S.oMateQ = take(S.capQ * 2);
-    S.oParentQ = take(S.capQ * 2);
-    S.oStampQ = take(S.capQ * 2);
-    S.oEnds = take(S.capQ * 2);
-    S.total = o;
+    S.nW = (int)(((long long)h * w + 31) / 32);
+    // 12 B per predicted vertex + 8 B per GT vertex
+    S.capP = S.capQ = vertex_cap(budget, (long long)S.nW * 4 + (((long long)S.nW * 2 + 15) / 16) * 16 + 256, 20);
+    if (S.capP == 0) return S;
+    Carve C;
+    S.oBits = C.take(S.nW * 4);
+    S.oRank = C.take(S.nW * 2);
+    S.oPpix = C.take(S.capP * 4);
+    S.oMateP = C.take(S.capP * 2);
+    S.oClaimP = C.take(S.capP * 2);
+    S.oFa = C.take(S.capP * 2);
+    S.oFb = C.take(S.capP * 2);  // read by nothing, but its 2 B per vertex are part of capP
+    S.oMateQ = C.take(S.capQ * 2);
+    S.oParentQ = C.take(S.capQ * 2);
+    S.oStampQ = C.take(S.capQ * 2);
+    S.oEnds = C.take(S.capQ * 2);
+    S.total = C.o;
     return S;
 }
 
 static SweepLayout sweep_layout(int h, int w, int budget) {
     SweepLayout S;
     memset(&S, 0, sizeof(S));
-    const long long hw = (long long)h * w;
-    S.nW = (int)((hw + 31) / 32);
-    const long long fixed = (long long)S.nW * 4 + (long long)S.nW + 2 * kEndsCap + 512;
-    // 13 B per predicted vertex, 8 B per GT vertex, equal capacities
-    const long long cap = (budget - fixed) / 21;
-    if (cap < 512) return S;
-    S.capP = S.capQ = (int)(cap > 0xFFF0 ? 0xFFF0 : cap) & ~7;
-    unsigned o = 0;
-    auto take = [&](unsigned bytes) { const unsigned r = o; o += (bytes + 15u) & ~15u; return r; };
-    S.oBits = take(S.nW * 4);
-    S.oRank = take(((S.nW + 1) / 2) * 2);
-    S.oPpix = take(S.capP * 4);
-    S.oMateP = take(S.capP * 2);
-    S.oClassP = take(S.capP * 2);
-    S.oFa = take(S.capP * 2);
-    S.oRootP = take(S.capP * 2);
-    S.oRflag = take(S.capP + 4);
-    S.oMateQ = take(S.capQ * 2);
-    S.oParentQ = take(S.capQ * 2);
-    S.oStamp = take(S.capQ * 4);
-    S.oEnds = take(kEndsCap * 2);
-    S.total = o;
+    S.nW = (int)(((long long)h * w + 31) / 32);
+    // 13 B per predicted vertex, 8 B per GT vertex
+    S.capP = S.capQ = vertex_cap(budget, (long long)S.nW * 4 + (long long)S.nW + 2 * kEndsCap + 512, 21);
+    if (S.capP == 0) return S;
+    Carve C;
+    S.oBits = C.take(S.nW * 4);
+    S.oRank = C.take(((S.nW + 1) / 2) * 2);
+    S.oPpix = C.take(S.capP * 4);
+    S.oMateP = C.take(S.capP * 2);
+    S.oClassP = C.take(S.capP * 2);
+    S.oFa = C.take(S.capP * 2);
+    S.oRootP = C.take(S.capP * 2);
+    S.oRflag = C.take(S.capP + 4);
+    S.oMateQ = C.take(S.capQ * 2);
+    S.oParentQ = C.take(S.capQ * 2);
+    S.oStamp = C.take(S.capQ * 4);
+    S.oEnds = C.take(kEndsCap * 2);
+    S.total = C.o;
     return S;
 }
 
 static Layout layout(int nProblems, int h, int w, int T) {
     Layout L;
     size_t off = MTE_WS_HEADER_BYTES;
-    L.offTable = off; off += align_up(sizeof(short2) * 4096, 256);
-    L.offNeg = off; off += align_up(sizeof(unsigned short) * 4096, 256);
+    L.offTable = off; off += align_up(sizeof(short2) * kMaxOff, 256);
+    L.offNeg = off; off += align_up(sizeof(unsigned short) * kMaxOff, 256);
     L.offThr = off; off += align_up(sizeof(double) * (size_t)(T > 0 ? T : 1), 256);
     L.offOverflow = off; off += align_up(sizeof(int) * (size_t)(nProblems > 0 ? nProblems : 1), 256);
     L.arenaBytes = align_up(arena_bytes(h, w), 256);
@@ -1559,7 +1511,6 @@ static int launch(MatchP &P, const Layout &L, char *ws, double max_dist, const d
     P.arena = ws + L.offArena;
     P.arenaBytes = L.arenaBytes;
     WsHeader *hdr = reinterpret_cast<WsHeader *>(ws);
-    P.truncate = debug_knob("MTE_MATCH_TRUNCATE") ? 1 : 0;
     P.stats = debug_knob("MTE_MATCH_STATS") ? hdr->pad : nullptr;
     P.trace = nullptr;
     if (debug_knob("MTE_MATCH_TRACE") && L.nArenas >= 2)   // the last arena is idle when a single image is matched
@@ -1571,52 +1522,23 @@ static int launch(MatchP &P, const Layout &L, char *ws, double max_dist, const d
     P.problemList = nullptr;
     P.listCount = nullptr;
     // shared-memory kernel first (one CTA per SM, ~200 KB of state), the dense L2 kernel mops up what did not fit
-    int smemBudget;
-    {
-        cudaFuncAttributes fa;
-        cudaFuncGetAttributes(&fa, match_smem_kernel);
-        smemBudget = dev_info().smemOptin - (int)fa.sharedSizeBytes - 1024;
-        if (smemBudget > 0 && opt_in_smem((const void *)match_smem_kernel, smemBudget) != cudaSuccess) smemBudget = 0;
-        cudaGetLastError();
-    }
-    const SmemLayout SL = smem_layout(P.h, P.w, smemBudget);
-    const bool useSmem = SL.capP > 0 && tb.n <= kSmemTableOff && !debug_knob("MTE_MATCH_DENSE");
+    const SmemLayout SL = smem_layout(P.h, P.w, smem_budget(match_smem_kernel));
+    const bool useSmem = SL.capP > 0 && tb.n <= kSmemTableOff;
     // threshold sweeps (level planes; strength maps with ascending thresholds): one CTA per image solves all T nested
     // problems incrementally; what does not fit falls through to the per-problem kernels via the overflow list
     // (thinned sets are not nested: the bits mode never sweeps)
-    bool sweep = useSmem && P.counts && !P.matchA && !P.matchB && P.inMode != IN_BINARY && P.inMode != IN_BITS &&
-                 P.T > 1 && !debug_knob("MTE_MATCH_NO_SWEEP");
+    bool sweep = useSmem && P.counts && !P.matchA && !P.matchB && P.inMode != IN_BINARY && P.inMode != IN_BITS && P.T > 1;
     if (sweep && P.inMode != IN_LEVELS)
         for (int t = 1; t < P.T; t++)
             if (!(thr_host[t] > thr_host[t - 1])) sweep = false;
-    if (sweep) {
-        int sweepBudget;
-        {
-            cudaFuncAttributes fa;
-            cudaFuncGetAttributes(&fa, match_sweep_kernel);
-            sweepBudget = dev_info().smemOptin - (int)fa.sharedSizeBytes - 1024;
-            if (sweepBudget > 0 && opt_in_smem((const void *)match_sweep_kernel, sweepBudget) != cudaSuccess) sweepBudget = 0;
-            cudaGetLastError();
-        }
-        const SweepLayout SW = sweep_layout(P.h, P.w, sweepBudget);
-        if (SW.capP > 0) {
-            int grid = num_sms();
-            if (grid > P.N) grid = P.N;
-            match_sweep_kernel<<<grid, kSwThreads, SW.total, st>>>(P, pt, inParam ? 1 : 0, SW);
-            MTE_RETURN_IF_CUDA_ERROR();
-            // the overflowed problems (usually none) go to the dense kernel
-            P.problemList = P.overflowList;
-            P.listCount = P.overflowCount;
-            match_kernel<<<L.nArenas, kThreads, 0, st>>>(P, pt, inParam ? 1 : 0);
-            MTE_RETURN_IF_CUDA_ERROR();
-            return MTE_OK;
-        }
-    }
+    const SweepLayout SW = sweep ? sweep_layout(P.h, P.w, smem_budget(match_sweep_kernel)) : SweepLayout{};
     if (useSmem) {
-        int grid = num_sms();
-        if (grid > P.nProblems) grid = P.nProblems;
-        match_smem_kernel<<<grid, kSmThreads, SL.total, st>>>(P, pt, inParam ? 1 : 0, SL);
+        if (SW.capP > 0)
+            match_sweep_kernel<<<std::min(num_sms(), P.N), kSwThreads, SW.total, st>>>(P, pt, inParam ? 1 : 0, SW);
+        else
+            match_smem_kernel<<<std::min(num_sms(), P.nProblems), kSmThreads, SL.total, st>>>(P, pt, inParam ? 1 : 0, SL);
         MTE_RETURN_IF_CUDA_ERROR();
+        // the overflowed problems (usually none) go to the dense kernel
         P.problemList = P.overflowList;
         P.listCount = P.overflowCount;
     }
