@@ -12,14 +12,20 @@
 // like the separate multiply and add), so the Sobel responses are bit-identical to OpenCV's and the orientation bins /
 // uint8 normals follow.
 //
-// Kernels:  dee_front_tma_kernel (fp32 planes: TMA halo tile, Sobel5 + normals + NMS + hysteresis labels out of a register
-//                                 window, candidate-only fast paths, flagged pixels redone by dee_pixel_exact)
+// Kernels:  dee_tables_kernel    (the 255 level-threshold directions of the normals)
+//           dee_front_tma_kernel (fp32 planes: TMA halo tile, Sobel5 + normals + NMS + hysteresis labels out of a register
+//                                 window; with NMS a straight-line row loop whose undecided pixels are redone by
+//                                 dee_pixel_exact, without NMS a generic row loop that decides each pixel in line)
 //           dee_front_kernel     (fp64 planes and odd shapes: shared-memory halo tile, same decisions)
 //           canny::run_level_hysteresis (shared 8-connected flood / union-find hysteresis)
 //           dee_finish_kernel    (img * labels / max(labels), the reference's normalisation quirk included)
+//           dee_convert_kernel   (NMS only, into the other float type)
+// Both front kernels call the same __forceinline__ helpers for the Sobel passes, the zero-gradient level and the NMS bin.
 #include <cuda.h>
 #include <math.h>
 #include <string.h>
+
+#include <type_traits>
 
 #include "common.cuh"
 
@@ -99,6 +105,83 @@ __global__ void dee_tables_kernel(DeeTab *tab) {
     }
 }
 
+// ---- arithmetic shared by the front kernels ---------------------------------------------------------------------
+// cv2.Sobel's row pass over five consecutive values, tap by tap: d with the derivative taps, m with the smoothing taps.
+// FUSED: the inputs are fp32 values, so every product with a tap (0, +-1, +-2, 4, 6) is EXACT in fp64 and a fused
+// multiply-add rounds exactly once, like the separate add of the exact product: bit-identical to the mul + add sequence
+// (signs of zero and NaN / Inf included; tests/test_oracle_cpu.py::test_sobel5_fused_taps), half the instructions.
+// dee_front_kernel keeps the mul + add form for both input types: for an fp64 value 6 * a is not exact.
+template <bool FUSED>
+__device__ __forceinline__ void sobel5_row(double a0, double a1, double a2, double a3, double a4, double &d, double &m) {
+    if (FUSED) {
+        d = __fma_rn(-2.0, a1, -a0);
+        d = __fma_rn(0.0, a2, d);
+        d = __fma_rn(2.0, a3, d);
+        d = __dadd_rn(d, a4);
+        m = __fma_rn(4.0, a1, a0);
+        m = __fma_rn(6.0, a2, m);
+        m = __fma_rn(4.0, a3, m);
+        m = __dadd_rn(m, a4);
+    } else {
+        d = __dmul_rn(-1.0, a0);
+        d = __dadd_rn(d, __dmul_rn(-2.0, a1));
+        d = __dadd_rn(d, __dmul_rn(0.0, a2));
+        d = __dadd_rn(d, __dmul_rn(2.0, a3));
+        d = __dadd_rn(d, __dmul_rn(1.0, a4));
+        m = __dmul_rn(1.0, a0);
+        m = __dadd_rn(m, __dmul_rn(4.0, a1));
+        m = __dadd_rn(m, __dmul_rn(6.0, a2));
+        m = __dadd_rn(m, __dmul_rn(4.0, a3));
+        m = __dadd_rn(m, __dmul_rn(1.0, a4));
+    }
+}
+
+// cv2.Sobel's column pass over the row-pass results of five consecutive rows, D(i) / S(i) for i = 0 .. 4 (S(2) has tap
+// 0): symmetric on the derivative rows (-> sx), anti-symmetric on the smoothed rows (-> sy); returns (sx, sy).  FUSED:
+// products with a power of two are exact for any double, so they fuse as well (6 * D(2) is rounded on its own, as in
+// OpenCV).  The rows come through accessors so that each is read where the arithmetic uses it.
+template <bool FUSED, class RowD, class RowS>
+__device__ __forceinline__ double2 sobel5_col(RowD D, RowS S) {
+    double sx, sy;
+    if (FUSED) {
+        sx = __fma_rn(4.0, __dadd_rn(D(3), D(1)), __dmul_rn(6.0, D(2)));
+        sx = __dadd_rn(sx, __dadd_rn(D(4), D(0)));
+        sy = __fma_rn(2.0, __dsub_rn(S(3), S(1)), __dsub_rn(S(4), S(0)));
+    } else {
+        sx = __dmul_rn(6.0, D(2));
+        sx = __dadd_rn(sx, __dmul_rn(4.0, __dadd_rn(D(3), D(1))));
+        sx = __dadd_rn(sx, __dmul_rn(1.0, __dadd_rn(D(4), D(0))));
+        sy = __dmul_rn(2.0, __dsub_rn(S(3), S(1)));
+        sy = __dadd_rn(sy, __dmul_rn(1.0, __dsub_rn(S(4), S(0))));
+    }
+    return make_double2(sx, sy);
+}
+
+// level of a zero gradient, by the sign bits of (sy, sx)
+__device__ __forceinline__ int zero_level(double sx, double sy, const unsigned char *sZero) {
+    return sZero[(int)(__double2hiint(sy) < 0) | ((int)(__double2hiint(sx) < 0) << 1)];
+}
+
+// NMS bin of atan2(sy, sx): 0 = [0, 22.5) u [157.5, 180], 1 = [22.5, 67.5), 2 = [67.5, 112.5), 3 = [112.5, 157.5),
+// 4 = none.  |sy| against |sx| tan(22.5 / 67.5 deg) in fp64 with a 2^-40 guard band, and inside that band (or for NaN,
+// Inf / Inf) the reference's own expression (tools.py:12-17, 24-38)
+__device__ __forceinline__ int bin_exact(double sx, double sy) {
+    const double ax = fabs(sx), ay = fabs(sy);
+    const double t1 = ax * 0.41421356237309503, t2 = ax * 2.4142135623730951;   // tan 22.5, tan 67.5
+    constexpr double lo = 1.0 - 0x1p-40, hi = 1.0 + 0x1p-40;
+    if (ax == 0.0 && ay == 0.0) return 0;   // atan2(+-0, +-0) is 0 or +-pi: bin 0 either way
+    if (ay < t1 * lo) return 0;
+    if (ay > t1 * hi && ay < t2 * lo) return ((sx < 0.0) != (sy < 0.0)) ? 3 : 1;
+    if (ay > t2 * hi) return 2;
+    double a = __dmul_rn(atan2(sy, sx), 180.0 / M_PI);
+    if (a < 0.0) a = __dadd_rn(a, 180.0);
+    if ((0.0 <= a && a < 22.5) || (157.5 <= a && a <= 180.0)) return 0;
+    if (22.5 <= a && a < 67.5) return 1;
+    if (67.5 <= a && a < 112.5) return 2;
+    if (112.5 <= a && a < 157.5) return 3;
+    return 4;
+}
+
 // T = type of the input map (the reference passes float32 network outputs; float64 accepted)
 template <typename T>
 __global__ void __launch_bounds__(kThreads) dee_front_kernel(const DeeTab *__restrict__ tab,
@@ -141,17 +224,8 @@ __global__ void __launch_bounds__(kThreads) dee_front_kernel(const DeeTab *__res
     if (needSobel) {
         for (int i = threadIdx.x; i < (TH + 4) * TW; i += kThreads) {
             const int r = i / TW, c = i - r * TW;
-            const double a0 = s[r][c], a1 = s[r][c + 1], a2 = s[r][c + 2], a3 = s[r][c + 3], a4 = s[r][c + 4];
-            double d = __dmul_rn(-1.0, a0);
-            d = __dadd_rn(d, __dmul_rn(-2.0, a1));
-            d = __dadd_rn(d, __dmul_rn(0.0, a2));
-            d = __dadd_rn(d, __dmul_rn(2.0, a3));
-            d = __dadd_rn(d, __dmul_rn(1.0, a4));
-            double m = __dmul_rn(1.0, a0);
-            m = __dadd_rn(m, __dmul_rn(4.0, a1));
-            m = __dadd_rn(m, __dmul_rn(6.0, a2));
-            m = __dadd_rn(m, __dmul_rn(4.0, a3));
-            m = __dadd_rn(m, __dmul_rn(1.0, a4));
+            double d, m;
+            sobel5_row<false>(s[r][c], s[r][c + 1], s[r][c + 2], s[r][c + 3], s[r][c + 4], d, m);
             rowD[r][c] = d;
             rowS[r][c] = m;
         }
@@ -165,18 +239,15 @@ __global__ void __launch_bounds__(kThreads) dee_front_kernel(const DeeTab *__res
         const T v = (T)s[r + 2][c + 2];   // the tile holds the exact input value
         double sx = 0.0, sy = 0.0;
         if (needSobel) {
-            // symmetric column pass on the derivative rows, anti-symmetric on the smoothed rows
-            sx = __dmul_rn(6.0, rowD[r + 2][c]);
-            sx = __dadd_rn(sx, __dmul_rn(4.0, __dadd_rn(rowD[r + 3][c], rowD[r + 1][c])));
-            sx = __dadd_rn(sx, __dmul_rn(1.0, __dadd_rn(rowD[r + 4][c], rowD[r][c])));
-            sy = __dmul_rn(2.0, __dsub_rn(rowS[r + 3][c], rowS[r + 1][c]));
-            sy = __dadd_rn(sy, __dmul_rn(1.0, __dsub_rn(rowS[r + 4][c], rowS[r][c])));
+            const double2 grad = sobel5_col<false>([&](int i) { return rowD[r + i][c]; }, [&](int i) { return rowS[r + i][c]; });
+            sx = grad.x;
+            sy = grad.y;
         }
         if (normals) {
             const double X = sx, Y = -sy;
             int lvl = -1;
             if (X == 0.0 && Y == 0.0) {
-                lvl = sZero[(int)(__double2hiint(sy) < 0) | ((int)(__double2hiint(sx) < 0) << 1)];
+                lvl = zero_level(sx, sy, sZero);
             } else {
                 const float a32 = atan2f((float)Y, (float)X);
                 const int k0 = min(max((int)((a32 * 57.29577951f + 180.f) * (255.f / 360.f)), 0), 255);
@@ -194,26 +265,7 @@ __global__ void __launch_bounds__(kThreads) dee_front_kernel(const DeeTab *__res
         if (doNms) {
             keep = (T)0;
             if (interior) {
-                // bin: 0 = [0, 22.5) u [157.5, 180], 1 = [22.5, 67.5), 2 = [67.5, 112.5), 3 = [112.5, 157.5), 4 = none
-                int bin = -1;
-                {
-                    const double ax = fabs(sx), ay = fabs(sy);
-                    const double t1 = ax * 0.41421356237309503, t2 = ax * 2.4142135623730951;   // tan 22.5, tan 67.5
-                    constexpr double lo = 1.0 - 0x1p-40, hi = 1.0 + 0x1p-40;
-                    if (ax == 0.0 && ay == 0.0) bin = 0;            // atan2(+-0, +-0) is 0 or +-pi: bin 0 either way
-                    else if (ay < t1 * lo) bin = 0;
-                    else if (ay > t1 * hi && ay < t2 * lo) bin = ((sx < 0.0) != (sy < 0.0)) ? 3 : 1;
-                    else if (ay > t2 * hi) bin = 2;
-                }
-                if (bin < 0) {  // inside a guard band, NaN or Inf / Inf: the reference's own expression
-                    double a = __dmul_rn(atan2(sy, sx), 180.0 / M_PI);
-                    if (a < 0.0) a = __dadd_rn(a, 180.0);
-                    bin = 4;
-                    if ((0.0 <= a && a < 22.5) || (157.5 <= a && a <= 180.0)) bin = 0;
-                    else if (22.5 <= a && a < 67.5) bin = 1;
-                    else if (67.5 <= a && a < 112.5) bin = 2;
-                    else if (112.5 <= a && a < 157.5) bin = 3;
-                }
+                const int bin = bin_exact(sx, sy);
                 T q = (T)1, rr = (T)1;  // tools.py:22-23: no bin (NaN angle) compares against 1
                 const int cr = r + 2, cc = c + 2;
                 if (bin == 0) { q = (T)s[cr][cc + 1]; rr = (T)s[cr][cc - 1]; }
@@ -248,24 +300,19 @@ __global__ void __launch_bounds__(kThreads) dee_front_kernel(const DeeTab *__res
 // patched with the REFLECT_101 values from inside the tile), and the separable Sobel runs out of a REGISTER window:
 // a thread owns one column, walks down the tile rows, computes the two fp64 row filters of a row from five shared
 // floats and keeps the last five results in registers for the column filter -- no fp64 round trip through shared
-// memory, no per-element index arithmetic.  Arithmetic (operation order of cv2.Sobel, quantisation, NMS, labels) is
-// the same as dee_front_kernel's; that kernel stays for fp64 inputs and odd shapes.
+// memory, no per-element index arithmetic.  With the NMS the row loop is straight-line code that only flags the pixels
+// its fp32 candidates cannot decide, and dee_pixel_exact redoes them after the loop; without it (normals only, or the
+// hysteresis of the raw map) a generic row loop decides each pixel in line.  Both use the shared Sobel passes and exact
+// decisions, so they make dee_front_kernel's decisions; that kernel stays for fp64 inputs and odd shapes.
 // ---------------------------------------------------------------------------
 // The innermost box coordinate of a bulk-tensor copy must be 16-byte aligned (x0 - 2 traps with "illegal
 // instruction"; probed with scripts/ubench/tma_test.cu), so the box starts at x0 - 4 and is 8 columns wider than the tile.
-#ifndef MTE_DEE_XH
-#define MTE_DEE_XH 31
-#endif
-constexpr int XW = 128, XH = MTE_DEE_XH, XROWS = XH + 4, XPAD = 4, XCOLS = XW + 2 * XPAD, kXThreads = XW;   // 35 tile rows = 7 groups of 5
+constexpr int XW = 128, XH = 31, XROWS = XH + 4, XPAD = 4, XCOLS = XW + 2 * XPAD, kXThreads = XW;   // 35 tile rows = 7 groups of 5
 static_assert(XROWS % 5 == 0, "the register window rotates with period 5");
+constexpr int kXMinBlocks = 6;   // CTAs per SM the TMA front is compiled for: at most 80 registers a thread
 
 __device__ __forceinline__ unsigned smem_u32(const void *p) { return (unsigned)__cvta_generic_to_shared(p); }
 // cond ? a : b as a real SELP (keeps ptxas from turning value selections into divergent branches)
-__device__ __forceinline__ float selp(bool cond, float a, float b) {
-    float r;
-    asm("{\n\t.reg .pred p;\n\tsetp.ne.s32 p, %3, 0;\n\tselp.f32 %0, %1, %2, p;\n\t}" : "=f"(r) : "f"(a), "f"(b), "r"((int)cond));
-    return r;
-}
 __device__ __forceinline__ unsigned selp(bool cond, unsigned a, unsigned b) {
     unsigned r;
     asm("{\n\t.reg .pred p;\n\tsetp.ne.s32 p, %3, 0;\n\tselp.u32 %0, %1, %2, p;\n\t}" : "=r"(r) : "r"(a), "r"(b), "r"((int)cond));
@@ -295,11 +342,34 @@ __device__ __forceinline__ float atan2_candidate(float y, float x) {
     return y < 0.f ? -p : p;
 }
 
+// angle of the normal, atan2(-sy, sx), as an fp32 CANDIDATE (|error| < 3e-6 rad on [1e-30, 1e30]:
+// tests/test_host_cpu.py::test_atan2_candidate_error_bound).  Outside that range the fast division flushes or
+// overflows: the candidate becomes NaN and every decision takes its exact path.
+__device__ __forceinline__ float angle_candidate(double sx, double sy) {
+    const float fx = (float)sx, fy = (float)-sy;
+    const float big = fmaxf(fabsf(fx), fabsf(fy));
+    const float a32 = atan2_candidate(fy, fx);
+    return (big > 1e-30f && big < 1e30f) ? a32 : __int_as_float(0x7fc00000);
+}
+
+// level = trunc(lv(A)), lv(A) = A * 255 / (2 pi) + 127.5, from the fp32 candidate a32.  The candidate level decides
+// alone (`decided`) when its fractional part is at least 1e-3 away from an integer (8x the candidate's 1.2e-4 levels of
+// error + the fp32 rounding of lv); the rest (0.2 % of the pixels, zero gradients, NaN / Inf) is proved by
+// dee_level_exact.  `valid` is false for a NaN candidate.
+__device__ __forceinline__ int level_candidate(float a32, bool &decided, bool &valid) {
+    const float lv = fmaf(a32, 40.5845105f, 127.5f);
+    const int k0 = (int)lv;
+    const float fl = lv - (float)k0;
+    decided = fl >= 1e-3f && fl <= 1.f - 1e-3f && (unsigned)k0 <= 254u;
+    valid = fl == fl;
+    return k0;
+}
+
 // The exact decisions of the pixels whose fp32 candidate is too close to a boundary (or is NaN: zero gradient, NaN /
 // Inf, values outside the fast division's range).  Rare, so they are real calls: ten inlined copies of the double
 // atan2 made the row loop 60 KB of code.
 __device__ __noinline__ int dee_level_exact(double sx, double sy, int k0, const double2 *sDir, const unsigned char *sZero) {
-    if (sx == 0.0 && sy == 0.0) return sZero[(int)(__double2hiint(sy) < 0) | ((int)(__double2hiint(sx) < 0) << 1)];
+    if (sx == 0.0 && sy == 0.0) return zero_level(sx, sy, sZero);
     const double X = sx, Y = -sy;
     const int kc = min(max(k0, 0), 255);
     const double m = (fabs(X) + fabs(Y)) * 0x1p-44;
@@ -307,6 +377,8 @@ __device__ __noinline__ int dee_level_exact(double sx, double sy, int k0, const 
     // try kc, kc - 1, kc + 1.  Two fp64 cross products against the neighbouring threshold DIRECTIONS prove a level
     // (sin(A - theta) = (Y cos theta - X sin theta) / r) -- ONLY for an angle known to lie near theta: the sign of a
     // sine says nothing half a turn away, so without a candidate (k0 < 0) the reference's expression decides.
+    // dee_front_kernel proves its candidate with its own copy of these products, which loads only the directions it
+    // needs: neither form as a shared helper compiles both kernels to the same code as their own copies.
     for (int t = 0; t < 3 && k0 >= 0; t++) {
         const int kk = kc + (t == 0 ? 0 : (t == 1 ? -1 : 1));
         if (kk < 0 || kk > 255) continue;
@@ -318,24 +390,7 @@ __device__ __noinline__ int dee_level_exact(double sx, double sy, int k0, const 
     return (int)normal_level_value(atan2(-sy, sx));  // inside a 2^-44 guard band, NaN / Inf: the reference's expression
 }
 
-__device__ __noinline__ int dee_bin_exact(double sx, double sy) {
-    // |sy| against |sx| tan(22.5 / 67.5 deg) in fp64 with a 2^-40 guard band, and inside that band the reference's own
-    // expression (tools.py:12-17, 24-38)
-    const double ax = fabs(sx), ay = fabs(sy);
-    const double t1 = ax * 0.41421356237309503, t2 = ax * 2.4142135623730951;
-    constexpr double lo = 1.0 - 0x1p-40, hi = 1.0 + 0x1p-40;
-    if (ax == 0.0 && ay == 0.0) return 0;   // atan2(+-0, +-0) is 0 or +-pi: bin 0 either way
-    if (ay < t1 * lo) return 0;
-    if (ay > t1 * hi && ay < t2 * lo) return ((sx < 0.0) != (sy < 0.0)) ? 3 : 1;
-    if (ay > t2 * hi) return 2;
-    double a = __dmul_rn(atan2(sy, sx), 180.0 / M_PI);
-    if (a < 0.0) a = __dadd_rn(a, 180.0);
-    if ((0.0 <= a && a < 22.5) || (157.5 <= a && a <= 180.0)) return 0;
-    if (22.5 <= a && a < 67.5) return 1;
-    if (67.5 <= a && a < 112.5) return 2;
-    if (112.5 <= a && a < 157.5) return 3;
-    return 4;
-}
+__device__ __noinline__ int dee_bin_exact(double sx, double sy) { return bin_exact(sx, sy); }
 
 // One output pixel entirely by the exact paths, straight from the halo tile (tile rows j .. j + 4 around output row j,
 // tile columns c + XPAD - 2 .. + 2): used by the straight-line row loop for the few pixels its fp32 candidate could not
@@ -348,19 +403,10 @@ __device__ __noinline__ bool dee_pixel_exact(const float *tile, int j, int c, bo
 #pragma unroll
     for (int r = 0; r < 5; r++) {
         const float *tr = tile + (j + r) * XCOLS + c + XPAD - 2;
-        const double a0 = (double)tr[0], a1 = (double)tr[1], a2 = (double)tr[2], a3 = (double)tr[3], a4 = (double)tr[4];
-        double dd = __fma_rn(-2.0, a1, -a0);
-        dd = __fma_rn(0.0, a2, dd);
-        dd = __fma_rn(2.0, a3, dd);
-        d[r] = __dadd_rn(dd, a4);
-        double mm = __fma_rn(4.0, a1, a0);
-        mm = __fma_rn(6.0, a2, mm);
-        mm = __fma_rn(4.0, a3, mm);
-        m[r] = __dadd_rn(mm, a4);
+        sobel5_row<true>(tr[0], tr[1], tr[2], tr[3], tr[4], d[r], m[r]);
     }
-    double sx = __fma_rn(4.0, __dadd_rn(d[3], d[1]), __dmul_rn(6.0, d[2]));
-    sx = __dadd_rn(sx, __dadd_rn(d[4], d[0]));
-    const double sy = __fma_rn(2.0, __dsub_rn(m[3], m[1]), __dsub_rn(m[4], m[0]));
+    const double2 grad = sobel5_col<true>([&](int i) { return d[i]; }, [&](int i) { return m[i]; });
+    const double sx = grad.x, sy = grad.y;
     if (NRM) nrmB[off] = (unsigned char)dee_level_exact(sx, sy, -1, sDir, sZero);
     const int cr = j + 2, cc = c + XPAD;
     const float v = tile[cr * XCOLS + cc];
@@ -384,11 +430,8 @@ __device__ __noinline__ bool dee_pixel_exact(const float *tile, int j, int c, bo
     return strong;
 }
 
-#ifndef MTE_DEE_MINB
-#define MTE_DEE_MINB 6
-#endif
 template <bool NRM, bool NMS, bool HYST>
-__global__ void __launch_bounds__(kXThreads, MTE_DEE_MINB) dee_front_tma_kernel(const __grid_constant__ CUtensorMap tmap,
+__global__ void __launch_bounds__(kXThreads, kXMinBlocks) dee_front_tma_kernel(const __grid_constant__ CUtensorMap tmap,
                                                                   const DeeTab *__restrict__ tab, int N, int H, int W,
                                                                   double tLow, double tHigh,
                                                                   unsigned char *__restrict__ normals,
@@ -442,7 +485,6 @@ __global__ void __launch_bounds__(kXThreads, MTE_DEE_MINB) dee_front_tma_kernel(
     __syncthreads();
 
     const int c = threadIdx.x, x = x0 + c;
-    constexpr bool SOBEL = NRM || NMS;
     const bool colIn = x < W;
     const bool xInterior = x >= 1 && x < W - 1;
     const int jEnd = min(XH, H - y0);   // output rows of this tile
@@ -477,44 +519,33 @@ __global__ void __launch_bounds__(kXThreads, MTE_DEE_MINB) dee_front_tma_kernel(
             const float t0 = tr[0], t1 = tr[1], t2 = tr[2], t3 = tr[3], t4 = tr[4];
             tr += XCOLS;
             f[u][0] = t1; f[u][1] = t2; f[u][2] = t3;
-            const double a0 = (double)t0, a1 = (double)t1, a2 = (double)t2, a3 = (double)t3, a4 = (double)t4;
-            double d = __fma_rn(-2.0, a1, -a0);   // exact products: see the generic loop at the end of the kernel
-            d = __fma_rn(0.0, a2, d);
-            d = __fma_rn(2.0, a3, d);
-            wD[u] = __dadd_rn(d, a4);
-            double m = __fma_rn(4.0, a1, a0);
-            m = __fma_rn(6.0, a2, m);
-            m = __fma_rn(4.0, a3, m);
-            wS[u] = __dadd_rn(m, a4);
+            sobel5_row<true>(t0, t1, t2, t3, t4, wD[u], wS[u]);
         };
         unsigned long long flagged = 0ull;
         const float zl0 = (float)sZero[0], zl1 = (float)sZero[1], zl2 = (float)sZero[2], zl3 = (float)sZero[3];
         auto out_row = [&](int u, int j, unsigned &gmask) {   // output row j of the tile; tile row j + 4 is in slot u
             const int y = y0 + j;
             const float v = f[(u + 3) % 5][1];
-            const double d0 = wD[(u + 1) % 5], d1 = wD[(u + 2) % 5], d2 = wD[(u + 3) % 5], d3 = wD[(u + 4) % 5], d4 = wD[u];
-            const double s0 = wS[(u + 1) % 5], s1 = wS[(u + 2) % 5], s3 = wS[(u + 4) % 5], s4 = wS[u];
-            double sx = __fma_rn(4.0, __dadd_rn(d3, d1), __dmul_rn(6.0, d2));
-            sx = __dadd_rn(sx, __dadd_rn(d4, d0));
-            const double sy = __fma_rn(2.0, __dsub_rn(s3, s1), __dsub_rn(s4, s0));
-            const float fx = (float)sx, fy = (float)-sy;
-            const float big = fmaxf(fabsf(fx), fabsf(fy));
-            float a32 = atan2_candidate(fy, fx);
-            a32 = (big > 1e-30f && big < 1e30f) ? a32 : __int_as_float(0x7fc00000);
+            // rows j .. j+4 of the row filters sit in slots (u+1)%5 .. (u+5)%5
+            const double2 grad = sobel5_col<true>([&](int i) { return wD[(u + 1 + i) % 5]; },
+                                                  [&](int i) { return wS[(u + 1 + i) % 5]; });
+            const double sx = grad.x, sy = grad.y;
+            const float a32 = angle_candidate(sx, sy);
             const bool zero = sx == 0.0 && sy == 0.0;
             bool decided = true;
             int lvl = 0;
             if (NRM) {
-                const float lv = fmaf(a32, 40.5845105f, 127.5f);
-                const int k0 = (int)lv;
-                const float fl = lv - (float)k0;
-                decided = fl >= 1e-3f && fl <= 1.f - 1e-3f && (unsigned)k0 <= 254u;
+                bool valid;
+                const int k0 = level_candidate(a32, decided, valid);
                 // zero gradient: level by the signs of the two zeros (sZero), picked with selects
                 const bool ny = __double2hiint(sy) < 0, nx = __double2hiint(sx) < 0;
                 const float zl = nx ? (ny ? zl3 : zl2) : (ny ? zl1 : zl0);
                 lvl = zero ? (int)zl : k0;
             }
-            const float uu = fmaf(-a32, 1.27323954f, 4.5f);   // bin boundaries at the integers, period 4 (see the generic loop)
+            // bin of atan2(sy, sx) = -a32 (mod pi): in units of pi / 4 shifted by half a bin the boundaries are the
+            // integers and the bins repeat with period 4: the fp32 candidate decides when it is at least 5e-5 (4e-5 rad,
+            // > 10x its error) away from every boundary
+            const float uu = fmaf(-a32, 1.27323954f, 4.5f);   // in (0.5, 8.5)
             const int iu = (int)uu;
             const float fu = uu - (float)iu;
             decided = decided && fu >= 5e-5f && fu <= 1.f - 5e-5f;
@@ -584,95 +615,28 @@ __global__ void __launch_bounds__(kXThreads, MTE_DEE_MINB) dee_front_tma_kernel(
             const int k = g * 5 + u;   // tile row k = image row y0 - 2 + k
             {
                 const float t0 = tr[0], t1 = tr[1], t2 = tr[2], t3 = tr[3], t4 = tr[4];
-                f[u][0] = t1; f[u][1] = t2; f[u][2] = t3;
-                if (SOBEL) {
-                    const double a0 = (double)t0, a1 = (double)t1, a2 = (double)t2, a3 = (double)t3, a4 = (double)t4;
-                    // cv2.Sobel's row pass, tap by tap.  The inputs are fp32 values, so every product with a tap (0,
-                    // +-1, +-2, 4, 6) is EXACT in fp64 and a fused multiply-add rounds exactly once, like the separate
-                    // add of the exact product: bit-identical to the mul + add sequence (signs of zero and NaN / Inf
-                    // included; tests/test_oracle_cpu.py::test_sobel5_fused_taps), half the instructions.
-                    double d = __fma_rn(-2.0, a1, -a0);
-                    d = __fma_rn(0.0, a2, d);
-                    d = __fma_rn(2.0, a3, d);
-                    d = __dadd_rn(d, a4);
-                    double m = __fma_rn(4.0, a1, a0);
-                    m = __fma_rn(6.0, a2, m);
-                    m = __fma_rn(4.0, a3, m);
-                    m = __dadd_rn(m, a4);
-                    wD[u] = d;
-                    wS[u] = m;
-                }
+                f[u][1] = t2;
+                if (NRM) sobel5_row<true>(t0, t1, t2, t3, t4, wD[u], wS[u]);
             }
             const int j = k - 4;           // output row of the tile, image row y0 + j; its centre is tile row k - 2
             if (j >= 0 && j < jEnd && colIn) {
                 const int y = y0 + j;
-                const float v = f[(u + 3) % 5][1];
-                double sx = 0.0, sy = 0.0;
-                float a32 = 0.f;
-                if (SOBEL) {
-                    // rows j .. j+4 of the row filters sit in slots (u+1)%5 .. (u+5)%5
-                    const double d0 = wD[(u + 1) % 5], d1 = wD[(u + 2) % 5], d2 = wD[(u + 3) % 5], d3 = wD[(u + 4) % 5], d4 = wD[u];
-                    const double s0 = wS[(u + 1) % 5], s1 = wS[(u + 2) % 5], s3 = wS[(u + 4) % 5], s4 = wS[u];
-                    // column pass: products with a power of two are exact for any double, so they fuse as well
-                    // (6 * d2 is rounded on its own, as in OpenCV)
-                    sx = __fma_rn(4.0, __dadd_rn(d3, d1), __dmul_rn(6.0, d2));
-                    sx = __dadd_rn(sx, __dadd_rn(d4, d0));
-                    sy = __fma_rn(2.0, __dsub_rn(s3, s1), __dsub_rn(s4, s0));
-                    // angle of the normal, atan2(-sy, sx), as an fp32 CANDIDATE (|error| < 3e-6 rad on [1e-30, 1e30]:
-                    // tests/test_host_cpu.py::test_atan2_candidate_error_bound).  Outside that range the fast division
-                    // flushes or overflows: the candidate becomes NaN and every decision takes its exact path.
-                    const float fx = (float)sx, fy = (float)-sy;
-                    const float big = fmaxf(fabsf(fx), fabsf(fy));
-                    a32 = atan2_candidate(fy, fx);
-                    a32 = (big > 1e-30f && big < 1e30f) ? a32 : __int_as_float(0x7fc00000);
-                }
+                const float keep = f[(u + 3) % 5][1];   // no NMS: the raw value
                 if (NRM) {
-                    // level = trunc(lv(A)), lv(A) = A * 255 / (2 pi) + 127.5.  The candidate decides alone when its
-                    // fractional part is at least 1e-3 away from an integer (8x the candidate's 1.2e-4 levels of
-                    // error + the fp32 rounding of lv); the rest (0.2 % of the pixels, zero gradients, NaN / Inf) is
-                    // proved with two fp64 cross products against the neighbouring threshold DIRECTIONS, and inside
-                    // their 2^-44 guard band by the reference's own double atan2 expression.
-                    const float lv = fmaf(a32, 40.5845105f, 127.5f);
-                    const int k0 = (int)lv;
-                    const float fl = lv - (float)k0;
-                    int lvl = k0;
-                    if (!(fl >= 1e-3f && fl <= 1.f - 1e-3f && (unsigned)k0 <= 254u)) {
+                    // rows j .. j+4 of the row filters sit in slots (u+1)%5 .. (u+5)%5
+                    const double2 grad = sobel5_col<true>([&](int i) { return wD[(u + 1 + i) % 5]; },
+                                                          [&](int i) { return wS[(u + 1 + i) % 5]; });
+                    const double sx = grad.x, sy = grad.y;
+                    bool decided, valid;
+                    int lvl = level_candidate(angle_candidate(sx, sy), decided, valid);
+                    if (!decided) {
                         // flat regions (zero gradient) are common in real maps: decided here, without the call
-                        if (sx == 0.0 && sy == 0.0) lvl = sZero[(int)(__double2hiint(sy) < 0) | ((int)(__double2hiint(sx) < 0) << 1)];
-                        else lvl = dee_level_exact(sx, sy, (fl == fl) ? k0 : -1, sDir, sZero);   // NaN candidate: none
+                        if (sx == 0.0 && sy == 0.0) lvl = zero_level(sx, sy, sZero);
+                        else lvl = dee_level_exact(sx, sy, valid ? lvl : -1, sDir, sZero);   // NaN candidate: none
                     }
                     st8(nrmB, oi, (unsigned)lvl);
                 }
                 const bool interior = xInterior && y >= 1 && y < H - 1;
-                float keep = v;
-                if (NMS) {
-                    keep = 0.f;
-                    if (interior) {
-                        // bin of atan2(sy, sx) = -a32 (mod pi): 0 = [0, 22.5) u [157.5, 180], 1 = [22.5, 67.5),
-                        // 2 = [67.5, 112.5), 3 = [112.5, 157.5), 4 = none.  In units of pi / 4 shifted by half a bin the
-                        // boundaries are the integers and the bins repeat with period 4: the fp32 candidate decides
-                        // when it is at least 5e-5 (4e-5 rad, > 10x its error) away from every boundary.
-                        const float uu = fmaf(-a32, 1.27323954f, 4.5f);   // in (0.5, 8.5)
-                        const int iu = (int)uu;
-                        const float fu = uu - (float)iu;
-                        int bin = iu & 3;
-                        if (!(fu >= 5e-5f && fu <= 1.f - 5e-5f))   // near a boundary, zero gradient (flat: no call), NaN / Inf
-                            bin = (sx == 0.0 && sy == 0.0) ? 0 : dee_bin_exact(sx, sy);
-                        // neighbours (q, r): bin 0 (E, W), 1 (NW, SE), 2 (S, N), 3 (SW, NE); no bin -> 1 (tools.py:22-23),
-                        // out of the register window: rows above / at / below the centre are slots u+2, u+3, u+4
-                        const float(&up)[3] = f[(u + 2) % 5];
-                        const float(&md)[3] = f[(u + 3) % 5];
-                        const float(&dn)[3] = f[(u + 4) % 5];
-                        // (real selects: as ternaries the compiler builds a branch tree with register moves, 25
-                        // instructions per pixel)
-                        const bool b0 = bin == 0, b1 = bin == 1, b2 = bin == 2, b4 = bin == 4;
-                        float q = selp(b2, dn[1], dn[0]), rr = selp(b2, up[1], up[2]);
-                        q = selp(b1, up[0], q); rr = selp(b1, dn[2], rr);
-                        q = selp(b0, md[2], q); rr = selp(b0, md[0], rr);
-                        q = selp(b4, 1.f, q); rr = selp(b4, 1.f, rr);
-                        keep = selp(v >= q && v >= rr, v, 0.f);
-                    }
-                }
                 if (nmsOut) st32(nmsB, oi, keep);
                 if (HYST) {
                     if (interior) {
@@ -857,20 +821,19 @@ static int run(const T *prob, int N, int H, int W, int do_nms, int do_hyst, doub
     bool tma = false;
     if constexpr (sizeof(T) == 4) {
         CUtensorMap map;
-        if (!debug_knob("MTE_DEE_NO_TMA") && make_plane_map(map, reinterpret_cast<const float *>(prob), N, H, W)) {
+        if (make_plane_map(map, reinterpret_cast<const float *>(prob), N, H, W)) {
+            // indexed by NRM * 4 + NMS * 2 + HYST.  No entry 0: without normals the edges are asked for, and
+            // mte_dee_postprocess rejects edges without NMS or hysteresis.
+            static constexpr decltype(&dee_front_tma_kernel<true, true, true>) kFront[8] = {
+                nullptr,
+                dee_front_tma_kernel<false, false, true>, dee_front_tma_kernel<false, true, false>,
+                dee_front_tma_kernel<false, true, true>, dee_front_tma_kernel<true, false, false>,
+                dee_front_tma_kernel<true, false, true>, dee_front_tma_kernel<true, true, false>,
+                dee_front_tma_kernel<true, true, true>};
             const int xt = ceil_div(W, XW) * ceil_div(H, XH) * N;
-            const bool nr = normals != nullptr, nm = do_nms != 0, hy = do_hyst && wantVal;
-            float *dst = reinterpret_cast<float *>(nmsDst);
-#define MTE_DEE_LAUNCH(A, B, C) dee_front_tma_kernel<A, B, C><<<xt, kXThreads, 0, st>>>(map, tab, N, H, W, lo, hi, normals, dst, cl, E, stats)
-            if (nr && nm && hy) MTE_DEE_LAUNCH(true, true, true);
-            else if (nr && nm) MTE_DEE_LAUNCH(true, true, false);
-            else if (nr && hy) MTE_DEE_LAUNCH(true, false, true);
-            else if (nr) MTE_DEE_LAUNCH(true, false, false);
-            else if (nm && hy) MTE_DEE_LAUNCH(false, true, true);
-            else if (nm) MTE_DEE_LAUNCH(false, true, false);
-            else if (hy) MTE_DEE_LAUNCH(false, false, true);
-            else MTE_DEE_LAUNCH(false, false, false);
-#undef MTE_DEE_LAUNCH
+            const int v = (normals != nullptr) * 4 + (do_nms != 0) * 2 + (do_hyst && wantVal);
+            kFront[v]<<<xt, kXThreads, 0, st>>>(map, tab, N, H, W, lo, hi, normals, reinterpret_cast<float *>(nmsDst), cl,
+                                                E, stats);
             tma = true;
         }
     }
@@ -885,25 +848,25 @@ static int run(const T *prob, int N, int H, int W, int do_nms, int do_hyst, doub
         int rc = canny::run_level_hysteresis(cl, E, N, H, W, 1, ws + L.offActive, st);
         if (rc) return rc;
         // the reference computes in float64 once NMS has run (its output array is float64), else in the input type
-        const bool c64 = do_nms || sizeof(T) == 8;
-        // one image per blockIdx.y: batches beyond the grid's y limit go in slices
-        for (int n0 = 0; n0 < N; n0 += 65535) {
-            const int nn = N - n0 < 65535 ? N - n0 : 65535;
-            const size_t po = (size_t)n0 * H * W;
-            const dim3 fg((unsigned)ceil_div(H * W, kFinPx), (unsigned)nn);
-            if (out_dtype == MTE_F64) {
-                if (c64) dee_finish_kernel<T, double, double><<<fg, kFinThreads, 0, st>>>(val + po, E + po, nn, H, W, stats + n0, (double *)out + po);
-                else dee_finish_kernel<T, float, double><<<fg, kFinThreads, 0, st>>>(val + po, E + po, nn, H, W, stats + n0, (double *)out + po);
-            } else {
-                if (c64) dee_finish_kernel<T, double, float><<<fg, kFinThreads, 0, st>>>(val + po, E + po, nn, H, W, stats + n0, (float *)out + po);
-                else dee_finish_kernel<T, float, float><<<fg, kFinThreads, 0, st>>>(val + po, E + po, nn, H, W, stats + n0, (float *)out + po);
+        auto finish = [&](auto computeType) {
+            using C = decltype(computeType);
+            // one image per blockIdx.y: batches beyond the grid's y limit go in slices
+            for (int n0 = 0; n0 < N; n0 += 65535) {
+                const int nn = N - n0 < 65535 ? N - n0 : 65535;
+                const size_t po = (size_t)n0 * H * W;
+                const dim3 fg((unsigned)ceil_div(H * W, kFinPx), (unsigned)nn);
+                if (out_dtype == MTE_F64) dee_finish_kernel<T, C, double><<<fg, kFinThreads, 0, st>>>(val + po, E + po, nn, H, W, stats + n0, (double *)out + po);
+                else dee_finish_kernel<T, C, float><<<fg, kFinThreads, 0, st>>>(val + po, E + po, nn, H, W, stats + n0, (float *)out + po);
             }
-        }
+        };
+        if (do_nms) finish(0.0);
+        else finish(T(0));
         MTE_RETURN_IF_CUDA_ERROR();
     } else if (nmsDst == val) {
-        // NMS only: the reference returns float64 whatever the input type (tools.py:15 np.zeros((H, W)))
-        if (out_dtype == MTE_F64) dee_convert_kernel<T, double><<<grid, 256, 0, st>>>(val, (double *)out, n);
-        else dee_convert_kernel<T, float><<<grid, 256, 0, st>>>(val, (float *)out, n);
+        // NMS only: the reference returns float64 whatever the input type (tools.py:15 np.zeros((H, W))); an output in
+        // the input type was written in place above, so this converts into the other float type
+        using O = std::conditional_t<sizeof(T) == 4, double, float>;
+        dee_convert_kernel<T, O><<<grid, 256, 0, st>>>(val, static_cast<O *>(out), n);
         MTE_RETURN_IF_CUDA_ERROR();
     }
     return MTE_OK;
